@@ -4,6 +4,7 @@
 Contract (one JSON line on stdout from rank 0):
     python bench.py --gpus N --steps K --warmup W            (N > 1: launched under torchrun, one rank per GPU)
     python bench.py --impl reference ...                      (the CPU implementation of the same path, host cores)
+    python bench.py ... --dump-outputs DIR                    (also writes what the last timed step computed, DIR/*.npy)
 
 Workload (BASELINE.json configs[2], the configuration its metric and SURVEY 8(d)'s >= 50 % target are
 quoted on): 4096 independent sequences x T = 16384, p = 16 outputs, L = 8 latents, Matern-5/2 (state
@@ -322,6 +323,24 @@ def emit(line):
 
 _REAL_STDOUT = 1
 
+DUMP_BUDGET = 60 << 20     # bytes of array data --dump-outputs writes: with the .npy headers, under 64 MB
+
+
+def dump_outputs(torch, path, arrays, seed=0):
+    """Write each array (a tensor on any device) as path/<name>.npy in float64.  Together they stay within DUMP_BUDGET: an
+    array too large for its share is reduced to a fixed, seeded sample of its rows along the first two axes (the same rows
+    on every run of the same workload), in ascending order."""
+    os.makedirs(path, exist_ok=True)
+    share = DUMP_BUDGET // len(arrays)
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() * 8 > share:
+            rows = t.reshape(t.shape[0] * t.shape[1], -1) if t.dim() > 1 else t.reshape(-1, 1)
+            keep = max(1, share // (8 * rows.shape[1]))
+            idx = np.sort(np.random.default_rng(seed).choice(rows.shape[0], size=keep, replace=False))
+            t = rows[torch.from_numpy(idx).to(t.device)]
+        np.save(os.path.join(path, name + ".npy"), t.to(torch.float64).cpu().numpy())
+
 
 def run_ours(a, wl, torch, dist, rank, local_rank, world, steps, warmup, cores, with_e2e, with_cpu, nseq=0, tlen=0, shard="auto"):
     """One workload on this rank's GPU: device-resident timed region (+ e2e through the host-buffer C ABI, + CPU baseline).
@@ -422,6 +441,12 @@ def run_ours(a, wl, torch, dist, rank, local_rank, world, steps, warmup, cores, 
     units = float(N) * T_total * L if time_shard else float(N) * T * L * world
     value = units / (ms_per_step * 1e-3)
     result_scalar = float(out[0].item())
+    if a.dump_outputs and wl == a.workload and rank == 0:
+        # what the timed path returned in its last step (this rank's share of it)
+        if kind == "fsn":
+            dump_outputs(torch, a.dump_outputs, {"X": X, "Xs": Xs, "nll": nll}, seed)
+        else:
+            dump_outputs(torch, a.dump_outputs, {"loss": out[0:1], "grad": out[2:]}, seed)
 
     # per-kernel device times: the events recorded during the timed steps above.  Event-bracketed kernel times add up
     # to ~5-10 % more than the event-bracketed loop (an event between two kernels costs a drain the plain stream does
@@ -593,6 +618,9 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-also", action="store_true", help="skip the extra configs[3] / configs[4] device passes of the default run")
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last step computed as DIR/<name>.npy (float64, at most 64 MB in all: "
+                         "a fixed, seeded sample of the rows of a larger output); GPU path only, with N > 1 GPUs rank 0's share")
     a = ap.parse_args()
 
     rank = int(os.environ.get("RANK", "0"))
@@ -604,6 +632,8 @@ def main():
 
     # ------------------------------------------------------------------ reference arm (CPU)
     if a.impl == "reference":
+        if a.dump_outputs:
+            raise SystemExit("bench.py: --dump-outputs writes the GPU path's outputs; --impl reference has none to write")
         if rank != 0:
             return
         t0 = time.perf_counter()

@@ -1,9 +1,10 @@
-// The reference's learners driven by the reference's own vendored LBFGS++ (LBFGSpp::LBFGSBSolver::minimize, LBFGSB.h:116-241),
-// ONE source built twice:
-//   -DUSE_REFERENCE : against the UNMODIFIED reference headers under /root/reference/moihgp/include (CPU; Eigen-API shim) -
-//                     run in the build container by tests/cpp/gen_lbfgs_golden.sh, its log is the fixture tests/golden_lbfgs/
-//   (default)       : against include/moihgp_b200/dropin (same include paths, same class names) + libmoihgp.so - run on the
-//                     GPU box by tests/test_cpp_host_api.py, its log must follow the fixture evaluation by evaluation.
+// The reference's learners driven by LBFGS++ (LBFGSpp::LBFGSBSolver::minimize, LBFGSB.h:116-241), ONE source built
+//   -DUSE_REFERENCE : against the UNMODIFIED reference headers and the reference's vendored LBFGS++ (CPU; Eigen-API shim) -
+//                     its log is the fixture tests/golden_lbfgs/ (tests/cpp/Makefile: golden)
+//   (default)       : against include/moihgp_b200/dropin (same include paths, same class names) + libmoihgp.so, with the
+//                     reference's LBFGS++ where the reference tree is present (_build/lbfgs_dropin), or with
+//                     tests/cpp/replay/LBFGSpp, which replays the fixture's optimiser decisions (_build/lbfgs_replay, run on
+//                     the GPU by tests/test_cpp_host_api.py and compared with the fixture evaluation by evaluation).
 // Both print every objective evaluation the optimiser makes (parameters in, loss and gradient out), the iteration counts, the
 // final parameters, predictions and the streamed outputs of the online learner, as "tag v0 v1 ..." lines (%.17g).
 // TEST INFRASTRUCTURE: `private` is opened so that both builds can start from the same KNOWN parameters (the reference draws

@@ -39,6 +39,18 @@ static void expect(const char* what, double err, double tol = 1e-9) {
     if (!(err <= tol)) ++failures;
 }
 
+// A BFGS matrix holding corrections (get_m() > 0), H = I + w w^T with w_i = 0.1 cos(i): apply_Hv(v, a, res) = a H v, the
+// call the proximal term of OnlineObjective makes (moihgp_online.h:45-48)
+struct DenseBFGSMat {
+    int get_m() const { return 2; }
+    void apply_Hv(const Vec& v, const double& a, Vec& res) const {
+        double wv = 0.0;
+        for (size_t i = 0; i < v.size(); ++i) wv += 0.1 * std::cos(double(i)) * v[i];
+        res.assign(v.size(), 0.0);
+        for (size_t i = 0; i < v.size(); ++i) res[i] = a * (v[i] + 0.1 * std::cos(double(i)) * wv);
+    }
+};
+
 template <typename SS>
 static void run(int kernel, size_t p, size_t L, size_t T, bool threading, unsigned seed) {
     using namespace moihgp_b200;
@@ -110,7 +122,8 @@ static void run(int kernel, size_t p, size_t L, size_t T, bool threading, unsign
     expect("MOIHGP::negLogLikelihood(x,y,dx,grad) grad", e_g);
     expect("MOIHGP::negLogLikelihood(x,y)", e_l2);
 
-    // (3) OnlineObjective: window maintenance + objective == the same loop on the oracle (no BFGS corrections yet: identity proximal term)
+    // (3) OnlineObjective: window maintenance + objective == the same loop on the oracle, with the identity proximal term (no BFGS
+    //     corrections yet) and with a BFGS matrix holding corrections
     {
         const size_t W = 4;
         OnlineObjective<SS> fo(&gp, 0.9, W);
@@ -145,6 +158,23 @@ static void run(int kernel, size_t p, size_t L, size_t T, bool threading, unsign
         l2o += prox;
         expect("OnlineObjective loss (window 4, proximal identity)", std::fabs(l2 - l2o) / std::fabs(l2o));
         expect("OnlineObjective grad", rel_err(g2.data(), g2o.data(), np));
+        gp.update(params);
+        oracle_update(o, params.data());
+        // the same window with BFGS corrections: prepare() builds B column by column from apply_Hv and uploads it
+        OnlineObjective<SS, Vec, DenseBFGSMat> fb(&gp, 0.9, W);
+        for (size_t t = 0; t < 9 && t < T; ++t) fb.push_back(Y[t]);
+        fb.prepare();
+        Vec g3(np), g3o(np), dp(np), Bp(np);
+        const double l3 = fb(p2, g3);
+        oracle_update(o, p2.data());
+        cx = sx;
+        cdx = sdx;
+        double l3o = oracle_objective(o, wflat.data(), 1, win.size(), cx.data(), cdx.data(), g3o.data(), 0);
+        for (size_t i = 0; i < np; ++i) dp[i] = p2[i] - fb.oldparams[i];
+        fb.bfgs_mat.apply_Hv(dp, 0.9, Bp);
+        for (size_t i = 0; i < np; ++i) { l3o += 0.5 * dp[i] * Bp[i]; g3o[i] += Bp[i]; }
+        expect("OnlineObjective loss (window 4, BFGS corrections)", std::fabs(l3 - l3o) / std::fabs(l3o));
+        expect("OnlineObjective grad (BFGS corrections)", rel_err(g3.data(), g3o.data(), np));
         gp.update(params);
         oracle_update(o, params.data());
     }
