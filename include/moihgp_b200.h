@@ -149,6 +149,26 @@ int moihgp_cuda_filter_smoother_nll_dev(moihgp_handle* h, const double* Y, size_
 int moihgp_cuda_smooth(moihgp_handle* h, const double* X, size_t N, size_t T, int smoother_mode, double* Xs);
 int moihgp_cuda_smooth_dev(moihgp_handle* h, const double* X, size_t N, size_t T, int smoother_mode, double* Xs);
 
+/* Posterior sample paths of the latent processes (steady-state forward-filtering, backward-sampling in RTS form):
+ *   x~[T-1] = Xs[T-1] + e[T-1],  e[T-1] = LF z[T-1],   x~[t] = Xs[t] + e[t],  e[t] = G e[t+1] + LC z[t]
+ * with Xs the RTS-smoothed mean (MOIHGP_SMOOTH_RTS), G = its gain, LF LF' = PF and LC LC' = PF - G (A PF A' + Q) G'.
+ * z[t] is d standard normals from ONE Philox4x32-10 call with counter (t, n, l, s) and key (seed & 0xffffffff, seed >> 32):
+ * uniforms u_i = (w_i + 0.5) 2^-32, Box-Muller in fp64 (z_2k = r cos(2 pi u_2k+1), z_2k+1 = r sin(2 pi u_2k+1),
+ * r = sqrt(-2 ln u_2k)), the first d of z0..z3.  A draw depends on (seed, s, n, l, t) only; T, N and S must be < 2^32.
+ * The noise process is the steady-state one, the approximation the smoother itself makes.
+ *   _dev : DEVICE buffers, asynchronous on the handle's stream (capturable into a CUDA graph like the fused pass).  Runs the
+ *          fused pass with MOIHGP_SMOOTH_RTS into Xs_mean [N][T][L][d] (NULL = a workspace), then the sampler.
+ *   Xsamp [S][N][T][L][d], Fsamp [S][N][T][L] (x~(0)), Ysamp [S][N][T][p] (U sqrt(S) x~(0), noise-free outputs): any may be
+ *   NULL, not all three.  Missing observations (NaN) are handled as in the fused pass (moihgp_cuda_nan_status).
+ *   moihgp_cuda_set_path also selects the sampler: 1 = time-chunked, 2 = one pass per chain, 0 = by the number of chains.
+ * The host-buffer twin copies in, calls the _dev entry point and copies out. */
+int moihgp_cuda_sample_posterior_dev(moihgp_handle* h, const double* Y, size_t N, size_t T, const double* x0, size_t S,
+                                     unsigned long long seed, double* Xs_mean, double* Xsamp, double* Fsamp, double* Ysamp);
+int moihgp_cuda_sample_posterior(moihgp_handle* h, const double* Y, size_t N, size_t T, const double* x0, size_t S,
+                                 unsigned long long seed, double* Xs_mean, double* Xsamp, double* Fsamp, double* Ysamp);
+/* the sampler's factors LF, LC of latent l (lower-triangular, d x d row-major; either may be NULL) */
+int moihgp_cuda_sampler_consts(moihgp_handle* h, size_t l, double* LF, double* LC);
+
 /* RegressionObjective::operator() / OnlineObjective::operator() window loop over N sequences
  * (moihgp_regression.h:42-50, moihgp_online.h:61-70): loss = sum_n sum_t negLogLikelihood(x, y, dx, grad)
  * with MOIHGP::step v2 advancing (x, dx); grad[num_param] summed the same way.  x0 [N][L][d] and

@@ -13,7 +13,7 @@ CSRC = os.path.join(_HERE, "csrc")
 c_double_p = ctypes.POINTER(ctypes.c_double)
 c_int_p = ctypes.POINTER(ctypes.c_int)
 
-_SOURCES = ["ls_project.cuh", "polar.cu", "chain_kernels.cuh", "chain_inst_16x8.cu", "chain_inst_8x4.cu", "chain_inst_8x2.cu", "chain_inst_8x8.cu", "chain_inst_16x2.cu", "chain_inst_16x4.cu", "chain_inst_16x16.cu", "chain_inst_32x4.cu", "chain_inst_32x8.cu", "chain_inst_32x16.cu", "chain_inst_4x2.cu", "chain_inst_4x4.cu", "chain_inst_32x2.cu", "chain_inst_4x1.cu", "chain_inst_8x1.cu", "chain_inst_16x1.cu", "chain_inst_32x1.cu", "setup.cu", "project.cu", "scan.cu", "objective.cu", "chain.cu", "step.cu", "capi.cu", "moihgp_device.cuh", "tma.cuh", "small_mat.cuh", "launch.h", "Makefile"]
+_SOURCES = ["ls_project.cuh", "polar.cu", "chain_kernels.cuh", "chain_inst_16x8.cu", "chain_inst_8x4.cu", "chain_inst_8x2.cu", "chain_inst_8x8.cu", "chain_inst_16x2.cu", "chain_inst_16x4.cu", "chain_inst_16x16.cu", "chain_inst_32x4.cu", "chain_inst_32x8.cu", "chain_inst_32x16.cu", "chain_inst_4x2.cu", "chain_inst_4x4.cu", "chain_inst_32x2.cu", "chain_inst_4x1.cu", "chain_inst_8x1.cu", "chain_inst_16x1.cu", "chain_inst_32x1.cu", "setup.cu", "sample.cu", "project.cu", "scan.cu", "objective.cu", "chain.cu", "step.cu", "capi.cu", "moihgp_device.cuh", "tma.cuh", "small_mat.cuh", "launch.h", "Makefile"]
 
 
 def build(force=False, verbose=False):
@@ -141,6 +141,11 @@ def load():
     for name in ("moihgp_cuda_smooth", "moihgp_cuda_smooth_dev"):
         getattr(lib, name).restype = ctypes.c_int
         getattr(lib, name).argtypes = [vp, vp, sz, sz, ctypes.c_int, vp]
+    for name in ("moihgp_cuda_sample_posterior", "moihgp_cuda_sample_posterior_dev"):
+        getattr(lib, name).restype = ctypes.c_int
+        getattr(lib, name).argtypes = [vp, vp, sz, sz, vp, sz, ctypes.c_uint64, vp, vp, vp, vp]
+    lib.moihgp_cuda_sampler_consts.restype = ctypes.c_int
+    lib.moihgp_cuda_sampler_consts.argtypes = [vp, sz, vp, vp]
     lib.moihgp_cuda_bind_data.restype = ctypes.c_int
     lib.moihgp_cuda_bind_data.argtypes = [vp, vp, sz, sz]
     lib.moihgp_cuda_objective_bound.restype = ctypes.c_int
@@ -155,5 +160,5 @@ LEGACY_NAMES = ["new", "del", "step1", "step2", "step3", "step4", "update", "lik
 CUDA_NAMES = ["create", "destroy", "set_stream", "sync", "last_error", "launch_count", "profile", "profile_read", "set_path", "set_chain_seqs_per_warp", "igp_dim", "num_param",
               "num_igp_param", "update", "get_params", "get_U", "latent_consts", "latent_iters", "smoother_consts",
               "filter_smoother_nll", "filter_smoother_nll_values", "filter_smoother_nll_dev", "objective", "objective_dev", "bind_data", "objective_bound", "objective_begin_dev", "objective_finish_dev", "block_transition", "fsn_block_dev", "fsn_block_async", "fsn_carry_dev", "smoother_power", "smooth", "smooth_dev", "objective_begin_async", "carry_in_dev", "nan_status", "online_begin", "online_push", "online_set_proximal",
-              "online_objective", "online_get_state"]
+              "online_objective", "online_get_state", "sample_posterior", "sample_posterior_dev", "sampler_consts"]
 ALL_SYMBOLS = ["gp%s_%s" % (xx, n) for xx in ("32", "52") for n in LEGACY_NAMES] + ["moihgp_cuda_" + n for n in CUDA_NAMES]

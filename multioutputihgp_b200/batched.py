@@ -318,6 +318,51 @@ class MOIHGPSequences(object):
         self._check(self._lib.moihgp_cuda_smooth(self._h, _ptr(X), N, T, int(smoother_mode), _ptr(Xs)))
         return Xs[0] if squeeze else Xs
 
+    # ---- posterior sample paths (moihgp_cuda_sample_posterior*) ----------------------------------------------------
+    def sample_posterior(self, Y, num_samples, seed, x0=None, want_states=False, want_outputs=True):
+        """``num_samples`` draws of the latent trajectories from the posterior given Y [N,T,p] (or [T,p]) NumPy array, by
+        steady-state forward-filtering, backward-sampling around the RTS-smoothed mean.  Returns a dict of NumPy arrays:
+        Xs [N,T,L,d] (the RTS mean), X [S,N,T,L,d] (sampled states, if want_states), F [S,N,T,L] (sampled function values
+        x~(0)) and Y [S,N,T,p] (noise-free outputs U sqrt(S) x~(0), if want_outputs).  Draws depend only on (seed, sample,
+        sequence, latent, time): see include/moihgp_b200.h for the generator."""
+        Y = _np(Y)
+        if Y.ndim == 2:
+            Y = Y[None]
+        N, T, p = Y.shape
+        assert p == self.num_output
+        S, L, d = int(num_samples), self.num_latent, self.igp_dim
+        x0 = None if x0 is None else _np(x0).reshape(N, L, d)
+        Xs = np.empty((N, T, L, d))
+        X = np.empty((S, N, T, L, d)) if want_states else None
+        F = np.empty((S, N, T, L))
+        Ys = np.empty((S, N, T, p)) if want_outputs else None
+        self._check(self._lib.moihgp_cuda_sample_posterior(self._h, _ptr(Y), N, T, _ptr(x0), S, int(seed) & (2**64 - 1), _ptr(Xs),
+                                                           _ptr(X), _ptr(F), _ptr(Ys)))
+        return {"Xs": Xs, "X": X, "F": F, "Y": Ys}
+
+    def sample_posterior_device(self, Y, seed, x0=None, Xs=None, X=None, F=None, Ysamp=None):
+        """Device-resident variant: torch CUDA float64 tensors, outputs pre-allocated by the caller (Xs [N,T,L,d] the RTS mean
+        or None, X [S,N,T,L,d], F [S,N,T,L], Ysamp [S,N,T,p], at least one of the last three); the number of samples S is
+        their first dimension.  Asynchronous on torch's current stream."""
+        import torch
+        assert Y.is_cuda and Y.dtype == torch.float64 and Y.is_contiguous() and Y.dim() == 3
+        N, T, _ = Y.shape
+        outs = [o for o in (X, F, Ysamp) if o is not None]
+        S = int(outs[0].shape[0]) if outs else 1
+        for o in [Xs] + outs:
+            assert o is None or (o.is_cuda and o.dtype == torch.float64 and o.is_contiguous())
+        assert all(int(o.shape[0]) == S for o in outs), "X, F and Ysamp must hold the same number of samples"
+        self.set_stream(_torch_stream(Y.device))
+        self._check(self._lib.moihgp_cuda_sample_posterior_dev(self._h, _ptr(Y), N, T, _ptr(x0), S, int(seed) & (2**64 - 1), _ptr(Xs),
+                                                               _ptr(X), _ptr(F), _ptr(Ysamp)))
+
+    def sampler_consts(self, l):
+        """(LF, LC) of latent l, [d,d] lower-triangular: LF LF' = PF, LC LC' = PF - G PPc G' (the sampler's noise factors)."""
+        d = self.igp_dim
+        LF, LC = np.zeros((d, d)), np.zeros((d, d))
+        self._check(self._lib.moihgp_cuda_sampler_consts(self._h, l, _ptr(LF), _ptr(LC)))
+        return LF, LC
+
     # ---- device-resident streaming learner (moihgp_cuda_online_*) -----------------------------------------------
     def online_begin(self, windowsize):
         """Window, moving mean, carried state and proximal term in device memory; False if the shape does not qualify."""

@@ -869,6 +869,94 @@ int moihgp_cuda_smooth(moihgp_handle* h, const double* X, size_t N, size_t T, in
     return 0;
 }
 
+}  // extern "C"
+
+namespace {
+
+const char* sample_refusal(size_t N, size_t T, size_t S, bool any_output) {
+    if (N == 0 || T == 0) return "N and T must be positive";
+    if (S == 0) return "sample_posterior: the number of samples S must be positive";
+    const size_t lim = (size_t)1 << 32;                  // the Philox counter holds t, n and s in 32-bit words
+    if (T >= lim || N >= lim || S >= lim) return "sample_posterior: T, N and S must each be below 2^32";
+    if (!any_output) return "sample_posterior: no output requested (Xsamp, Fsamp and Ysamp are all NULL)";
+    return nullptr;
+}
+
+}  // namespace
+
+extern "C" {
+
+int moihgp_cuda_sampler_consts(moihgp_handle* h, size_t l, double* LF, double* LC) {
+    if (!h || l >= (size_t)h->L) return -2;
+    if (mirror(h)) return -1;
+    const int d = h->dim;
+    for (int i = 0; i < d; ++i) for (int j = 0; j < d; ++j) {
+        if (LF) LF[i * d + j] = h->consts[l].LF[i * 3 + j];
+        if (LC) LC[i * d + j] = h->consts[l].LC[i * 3 + j];
+    }
+    return 0;
+}
+
+int moihgp_cuda_sample_posterior_dev(moihgp_handle* h, const double* Y, size_t N, size_t T, const double* x0, size_t S,
+                                     unsigned long long seed, double* Xs_mean, double* Xsamp, double* Fsamp, double* Ysamp) {
+    if (!h || !Y) return -2;
+    if (const char* m = sample_refusal(N, T, S, Xsamp || Fsamp || Ysamp)) return fail(h, m);
+    DeviceGuard guard(h->device);
+    const int L = h->L, D = h->dim;
+    if (!Xs_mean && ws_get(h, "sXs", N * T * L * D, &Xs_mean)) return -1;
+    // set_path also selects the sampler's variant (1 time-chunked, 2 one pass); the mean pass then takes the many-chains
+    // kernels only where they serve the shape
+    const int path = h->path;
+    auto aligned16 = [](const void* q) { return (reinterpret_cast<size_t>(q) & 15) == 0; };
+    if (path == 2 && !(chain_supported(h->p, L, D, (long long)T) && aligned16(Y) && aligned16(Xs_mean))) h->path = 0;
+    const int rc = moihgp_cuda_filter_smoother_nll_dev(h, Y, N, T, x0, MOIHGP_SMOOTH_RTS, nullptr, Xs_mean, nullptr, nullptr, nullptr);
+    h->path = path;
+    if (rc) return rc;
+    const long long chains = (long long)(S * N * L);
+    const bool chunked = sample_chunked((long long)T, chains, path);
+    SampleArgs a;
+    a.consts = h->d_consts; a.S = (long long)S; a.N = (long long)N; a.T = (long long)T; a.L = L; a.seed = seed;
+    a.Xs = Xs_mean; a.Xsamp = Xsamp; a.F = Fsamp; a.carry = nullptr;
+    a.mk = h->profiling ? &h->marker : nullptr;
+    if (Ysamp && !Fsamp && ws_get(h, "sF", S * N * T * L, &a.F)) return -1;
+    if (chunked && ws_get(h, "scarry", sample_carry_doubles(D, (long long)T, chains), &a.carry)) return -1;
+    CK(launch_sample(D, a, chunked, h->stream));
+    h->launches += sample_launch_count(chunked);
+    if (Ysamp) {                                         // U sqrt(S) x~(0), the latent values as states of dimension 1
+        CK(launch_backproject(a.F, h->d_U, h->d_S, h->p, L, 1, (long long)(S * N), (long long)T, Ysamp, h->stream));
+        h->launches += 1;
+        mark(a.mk, "k_backproject");
+    }
+    return 0;
+}
+
+int moihgp_cuda_sample_posterior(moihgp_handle* h, const double* Y, size_t N, size_t T, const double* x0, size_t S,
+                                 unsigned long long seed, double* Xs_mean, double* Xsamp, double* Fsamp, double* Ysamp) {
+    if (!h || !Y) return -2;
+    if (const char* m = sample_refusal(N, T, S, Xsamp || Fsamp || Ysamp)) return fail(h, m);
+    DeviceGuard guard(h->device);
+    const size_t L = h->L, D = h->dim, p = h->p;
+    double *dY, *dx0 = nullptr, *dXs = nullptr, *dX = nullptr, *dF = nullptr, *dYs = nullptr;
+    if (ws_get(h, "spY", N * T * p, &dY)) return -1;
+    if (x0 && ws_get(h, "spx0", N * L * D, &dx0)) return -1;
+    if (Xs_mean && ws_get(h, "spXs", N * T * L * D, &dXs)) return -1;
+    if (Xsamp && ws_get(h, "spX", S * N * T * L * D, &dX)) return -1;
+    if (Fsamp && ws_get(h, "spF", S * N * T * L, &dF)) return -1;
+    if (Ysamp && ws_get(h, "spYs", S * N * T * p, &dYs)) return -1;
+    CK(cudaMemcpyAsync(dY, Y, sizeof(double) * N * T * p, cudaMemcpyHostToDevice, h->stream));
+    if (x0) CK(cudaMemcpyAsync(dx0, x0, sizeof(double) * N * L * D, cudaMemcpyHostToDevice, h->stream));
+    const int rc = moihgp_cuda_sample_posterior_dev(h, dY, N, T, dx0, S, seed, dXs, dX, dF, dYs);
+    if (rc) { cudaStreamSynchronize(h->stream); return rc; }
+    if (Xs_mean) CK(cudaMemcpyAsync(Xs_mean, dXs, sizeof(double) * N * T * L * D, cudaMemcpyDeviceToHost, h->stream));
+    if (Xsamp) CK(cudaMemcpyAsync(Xsamp, dX, sizeof(double) * S * N * T * L * D, cudaMemcpyDeviceToHost, h->stream));
+    if (Fsamp) CK(cudaMemcpyAsync(Fsamp, dF, sizeof(double) * S * N * T * L, cudaMemcpyDeviceToHost, h->stream));
+    if (Ysamp) CK(cudaMemcpyAsync(Ysamp, dYs, sizeof(double) * S * N * T * p, cudaMemcpyDeviceToHost, h->stream));
+    int status = 0;
+    if (moihgp_cuda_nan_status(h, &status)) return -1;   // waits for the stream
+    if (status == 2) return fail(h, "more than 2^22 observations with missing (NaN) outputs in one call: split the batch");
+    return 0;
+}
+
 // phase 0: whole evaluation; 1: begin (projection, summaries, block end from a zero carry-in -> zend, device);
 // 2: finish (from the true carry-in; reuses the workspace phase 1 filled)
 static int objective_phase(moihgp_handle* h, int phase, const double* Y, size_t N, size_t T, const double* x0, const double* dx0,

@@ -162,6 +162,23 @@ cudaError_t launch_online_push(const double* y_new, const double* ma_given /*or 
 cudaError_t launch_online_prox(const double* params, const double* oldparams, const double* B /*[np][np] or null*/, int np, int pL,
                                const double* U, double* out /*[loss, flag, grad[np], U[pL]]*/, cudaStream_t st);
 
+// sample.cu  (posterior sample paths: the RTS mean plus the data-independent backward noise process)
+struct SampleArgs {
+    const LatentConsts* consts;   // [L]
+    long long S, N, T, L;
+    unsigned long long seed;
+    const double* Xs;             // [N][T][L][D] RTS-smoothed mean
+    double* Xsamp;                // [S][N][T][L][D] or null
+    double* F;                    // [S][N][T][L] function values x~(0) or null (not both null)
+    double* carry;                // time-chunked variant: [chunks][S N L][D] workspace (sample_carry_doubles)
+    Marker* mk = nullptr;
+};
+bool sample_chunked(long long T, long long chains, int path);   // path: 0 automatic, 1 time-chunked, 2 one pass
+long long sample_chunk_len(long long T, long long chains);
+size_t sample_carry_doubles(int dim, long long T, long long chains);
+int sample_launch_count(bool chunked);
+cudaError_t launch_sample(int dim, const SampleArgs& a, bool chunked, cudaStream_t st);
+
 // step.cu  (one observation per call: the legacy gpXX_* entry points)
 struct StepArgs {
     const LatentConsts* consts;

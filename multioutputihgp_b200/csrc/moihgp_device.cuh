@@ -44,6 +44,9 @@ struct LatentConsts {
     int conv[4];          // their converged flags (ignored by the reference; diagnostics here)
     int smooth_iters;     // literal smoother DLyap iterations
     int dim;
+    // posterior sampling (sample.cu), lower-triangular factors of positive semi-definite matrices
+    double LF[9];         // LF LF' = PF                               (the end of a sequence)
+    double LC[9];         // LC LC' = PF - G[1] PPc G[1]'  (PPc = A PF A' + Q: x[t] given x[t+1])
 };
 
 // OILMM mixing parameters (moihgp.h:741-744) as the kernels see them

@@ -259,6 +259,77 @@ template <int D> __device__ __forceinline__ void store_mat(const double* m, doub
 template <int D> __device__ __forceinline__ void store_vec(const double* v, double* dst3) {
     for (int i = 0; i < 3; ++i) dst3[i] = i < D ? v[i] : 0.0;
 }
+// Lower-triangular Lo with Lo Lo' = M for a symmetric positive SEMI-definite M (its lower triangle is read).  A pivot at or
+// below 1e-13 x the largest diagonal entry leaves its column zero: the matrix is (numerically) rank-deficient there, and the
+// square root of a rounding-negative pivot is never taken.  Returns false if a pivot is below -1e-13 x that entry: M is
+// indefinite, Lo is not its factor.
+template <int D> __device__ bool chol_psd(const double* M, double* Lo) {
+    double dmax = 0.0;
+    for (int i = 0; i < D; ++i) dmax = fmax(dmax, M[i * D + i]);
+    const double tiny = 1e-13 * dmax;
+    bool psd = true;
+    zero<D * D>(Lo);
+    for (int j = 0; j < D; ++j) {
+        double s = M[j * D + j];
+        for (int k = 0; k < j; ++k) s -= Lo[j * D + k] * Lo[j * D + k];
+        if (!(s > tiny)) { psd = psd && s >= -tiny; continue; }
+        const double r = sqrt(s);
+        Lo[j * D + j] = r;
+        for (int i = j + 1; i < D; ++i) {
+            double t = M[i * D + j];
+            for (int k = 0; k < j; ++k) t -= Lo[i * D + k] * Lo[j * D + k];
+            Lo[i * D + j] = t / r;
+        }
+    }
+    return psd;
+}
+
+// The nearest positive semi-definite matrix (Frobenius norm) to a symmetric M: its negative eigenvalues set to zero.
+// Cyclic Jacobi rotations (Numerical Recipes' convention A <- P' A P).
+template <int D> __device__ void psd_part(const double* M, double* out) {
+    double A[D * D], V[D * D];
+    symmetrize<D>(M, A);
+    eye<D>(V);
+    for (int sweep = 0; sweep < 20; ++sweep) {
+        double off = 0.0, nrm = 0.0;
+        for (int i = 0; i < D; ++i) for (int j = 0; j < D; ++j) { nrm += A[i * D + j] * A[i * D + j]; if (i != j) off += A[i * D + j] * A[i * D + j]; }
+        if (off <= 1e-32 * nrm) break;
+        for (int p = 0; p < D - 1; ++p)
+            for (int q = p + 1; q < D; ++q) {
+                if (A[p * D + q] == 0.0) continue;
+                const double theta = (A[q * D + q] - A[p * D + p]) / (2.0 * A[p * D + q]);
+                const double t = (theta >= 0.0 ? 1.0 : -1.0) / (fabs(theta) + sqrt(theta * theta + 1.0));
+                const double c = 1.0 / sqrt(t * t + 1.0), s = t * c;
+                for (int k = 0; k < D; ++k) {
+                    const double kp = A[k * D + p], kq = A[k * D + q];
+                    A[k * D + p] = c * kp - s * kq; A[k * D + q] = s * kp + c * kq;
+                }
+                for (int k = 0; k < D; ++k) {
+                    const double pk = A[p * D + k], qk = A[q * D + k];
+                    A[p * D + k] = c * pk - s * qk; A[q * D + k] = s * pk + c * qk;
+                }
+                for (int k = 0; k < D; ++k) {
+                    const double kp = V[k * D + p], kq = V[k * D + q];
+                    V[k * D + p] = c * kp - s * kq; V[k * D + q] = s * kp + c * kq;
+                }
+            }
+    }
+    for (int i = 0; i < D; ++i)
+        for (int j = 0; j < D; ++j) {
+            double a = 0.0;
+            for (int k = 0; k < D; ++k) a += V[i * D + k] * fmax(A[k * D + k], 0.0) * V[j * D + k];
+            out[i * D + j] = a;
+        }
+}
+
+// the sampler's factor of a covariance: Cholesky where M is positive semi-definite, else of M's positive semi-definite part
+template <int D> __device__ void sampling_factor(const double* M, double* Lo) {
+    if (chol_psd<D>(M, Lo)) return;
+    double P[D * D];
+    psd_part<D>(M, P);
+    chol_psd<D>(P, Lo);
+}
+
 template <int D> __device__ void power_table(const double* M, double (*tab)[9]) {
     double P[D * D];
     cpy<D * D>(M, P);
@@ -448,6 +519,10 @@ __global__ void __launch_bounds__(192) k_setup(const double* __restrict__ igp_pa
         mm<D, D, D>(G, w.A, GA);
         for (int i = 0; i < D; ++i) for (int j = 0; j < D; ++j) Bs[i * D + j] = (i == j ? 1.0 : 0.0) - GA[i * D + j];
         store_mat<D>(G, o.G[1]); store_mat<D>(pv, o.Ps[1]); store_vec<D>(GK, o.GK); store_mat<D>(Bs, o.Bs);
+        double LF[DD], LC[DD];                      // posterior sampling: x[T-1] ~ N(., PF), x[t] | x[t+1] ~ N(., C)
+        sampling_factor<D>(w.PF, LF);
+        sampling_factor<D>(C, LC);
+        store_mat<D>(LF, o.LF); store_mat<D>(LC, o.LC);
         power_table<D>(G, o.powG[1]);
     } else if (warp == 5) {
         power_table<D>(w.AKHA, o.powM);             // AKHA^(2^k) for the chunked scans
