@@ -89,12 +89,19 @@ const char* moihgp_cuda_last_error(moihgp_handle* h);
  * (and clears the record).  Used by bench.py for the roofline figures; off by default. */
 int moihgp_cuda_profile(moihgp_handle* h, int enable);
 const char* moihgp_cuda_profile_read(moihgp_handle* h);
-/* which kernels serve the fused pass: 0 = automatic (many-chains kernels when there are enough independent
- * (sequence, latent) chains and the shape is instantiated, else the time-parallel chunked scan), 1 = chunked scan,
- * 2 = many-chains (fails if unavailable).  Results agree to rounding; used by the parity tests to cover both. */
+/* which kernels serve a call; 0 = automatic everywhere.  Results agree to rounding; used by the parity tests to cover
+ * every variant.  The setting has three effects:
+ *   - the fused pass (moihgp_cuda_filter_smoother_nll*): 0 = the many-chains kernels when there are enough independent
+ *     (sequence, latent) chains and the shape is instantiated, else the time-parallel chunked scan; 1 = chunked scan;
+ *     2 = many-chains (fails if unavailable);
+ *   - the posterior sampler (moihgp_cuda_sample_posterior*): 1 = time-chunked, 2 = one pass per chain, 0 = by the number
+ *     of chains.  Its mean pass follows the fused-pass choice, except that 2 takes the chunked scan where the many-chains
+ *     kernels are unavailable instead of failing;
+ *   - the host-buffer objective (moihgp_cuda_objective, moihgp_cuda_objective_bound): 1 sends a single short sequence
+ *     to the general kernels instead of the one-launch kernel; 0 and 2 leave the one-launch kernel in use. */
 int moihgp_cuda_set_path(moihgp_handle* h, int path);
 /* tuning knob of the many-chains kernels: sequences handled per warp (a power of two <= 32 / num_latent);
- * 0 = automatic (fewer sequences per warp when the batch alone does not fill the GPU with warps) */
+ * 0 = automatic (a full warp, 32 / num_latent sequences, whatever the batch size) */
 int moihgp_cuda_set_chain_seqs_per_warp(moihgp_handle* h, int n);
 /* kernels launched by this handle since creation (bench.py's gpu_launches) */
 long long moihgp_cuda_launch_count(moihgp_handle* h);
@@ -160,7 +167,7 @@ int moihgp_cuda_smooth_dev(moihgp_handle* h, const double* X, size_t N, size_t T
  *          fused pass with MOIHGP_SMOOTH_RTS into Xs_mean [N][T][L][d] (NULL = a workspace), then the sampler.
  *   Xsamp [S][N][T][L][d], Fsamp [S][N][T][L] (x~(0)), Ysamp [S][N][T][p] (U sqrt(S) x~(0), noise-free outputs): any may be
  *   NULL, not all three.  Missing observations (NaN) are handled as in the fused pass (moihgp_cuda_nan_status).
- *   moihgp_cuda_set_path also selects the sampler: 1 = time-chunked, 2 = one pass per chain, 0 = by the number of chains.
+ *   moihgp_cuda_set_path also selects the sampler's variant.
  * The host-buffer twin copies in, calls the _dev entry point and copies out. */
 int moihgp_cuda_sample_posterior_dev(moihgp_handle* h, const double* Y, size_t N, size_t T, const double* x0, size_t S,
                                      unsigned long long seed, double* Xs_mean, double* Xsamp, double* Fsamp, double* Ysamp);

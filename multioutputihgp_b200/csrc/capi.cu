@@ -118,6 +118,54 @@ int ws_get(moihgp_handle* h, const char* name, size_t count, T** out) {
     return 0;
 }
 
+// Workspace of the projection (k_project), shared by the scan and the objective passes: one handle alternating between
+// them reuses the same buffers.  Rows with a missing output are listed for re-projection, at most nan_cap of them.
+struct ProjectWs {
+    double *u, *rho;
+    int* nanf;                    // {status, count} (moihgp_cuda_nan_status)
+    long long* nanrows;
+    size_t nan_cap;
+};
+
+int project_ws(moihgp_handle* h, size_t N, size_t T, ProjectWs* w) {
+    w->nan_cap = std::min<size_t>(N * T, (size_t)1 << 22);
+    if (ws_get(h, "nanrows", w->nan_cap, &w->nanrows) || ws_get(h, "u", N * h->L * T, &w->u) ||
+        ws_get(h, "rho", N * project_tiles((long long)T), &w->rho) || ws_get(h, "nanf", 4, &w->nanf))
+        return -1;
+    return 0;
+}
+
+// A pass that meets more than 2^22 rows with missing outputs re-projects only the first 2^22 of them, so the host-buffer
+// entry points refuse such a call.  status: the status words of the call's passes, already on the host; null reads the
+// handle's own (that of the last pass), waiting for the stream.
+int refuse_nan_overflow(moihgp_handle* h, const int* status = nullptr, size_t n = 1) {
+    int last = 0;
+    if (!status) {
+        if (moihgp_cuda_nan_status(h, &last)) return -1;
+        status = &last;
+    }
+    for (size_t i = 0; i < n; ++i)
+        if (status[i] == 2) return fail(h, "more than 2^22 observations with missing (NaN) outputs in one call: split the batch");
+    return 0;
+}
+
+// Which kernels serve one fused pass over Y [N][T][p] into X / Xs (moihgp_cuda_set_path): 1 the many-chains kernels,
+// 0 the chunked scan.  The many-chains kernels need an instantiated shape and 16-byte aligned Y, X and Xs; the automatic
+// choice takes them where they are the faster path and the chains give every SM a warp.  A forced many-chains path that
+// cannot serve the pass fails (-2) when `strict`, else it takes the scan - as the automatic choice would, since
+// chain_preferred implies chain_supported.
+int chain_path(moihgp_handle* h, size_t N, size_t T, const void* Y, const void* X, const void* Xs, bool strict) {
+    auto aligned16 = [](const void* q) { return (reinterpret_cast<size_t>(q) & 15) == 0; };
+    const bool aligned = aligned16(Y) && aligned16(X) && aligned16(Xs);
+    if (h->path == 1) return 0;
+    if (h->path == 2) {
+        if (aligned && chain_supported(h->p, h->L, h->dim, (long long)T)) return 1;
+        return strict ? fail(h, "many-chains path not available for this shape/alignment") : 0;
+    }
+    const size_t chain_warps = (N * (size_t)h->L + 31) / 32;
+    return aligned && chain_preferred(h->p, h->L, h->dim, (long long)T) && chain_warps >= 148;
+}
+
 // Polar factor U = W V' of a (p x L, row-major, p >= L) via one-sided Jacobi: a V = W diag(s).
 // (MOIHGP::update forms svd.matrixU() * svd.matrixV().transpose(), moihgp.h:439,446.)
 void polar_factor(const double* a, int p, int L, double* out) {
@@ -555,27 +603,54 @@ int moihgp_cuda_smoother_consts(moihgp_handle* h, size_t l, int mode, double* G,
     return 0;
 }
 
-int moihgp_cuda_filter_smoother_nll_dev(moihgp_handle* h, const double* Y, size_t N, size_t T, const double* x0, int mode,
-                                        double* X, double* Xs, double* Yhat, double* nll, double* xT) {
+// The chunked-scan pass (project.cu + scan.cu) over Y [N][T][p] with N = a.N, T = a.T: a.phase 0 is the whole pass, 1 / 2 / 3
+// one block of a sequence sharded in time (ScanArgs).  The caller sets a's inputs, outputs, phase and marker; this takes the
+// workspace, projects Y (phases 0 and 1), scans, and reduces the NLL into nll (phases 0 and 3, when nll is set).  On return
+// a.u holds the projected observations.
+static int scan_pass(moihgp_handle* h, const double* Y, int mode, double* nll, ScanArgs& a) {
+    const size_t N = (size_t)a.N, T = (size_t)a.T, L = h->L, D = h->dim, nC = scan_chunks(a.T), nSB = scan_superblocks(a.T);
+    ProjectWs pw;
+    double *fsum, *bsum, *xin, *bin, *Bx, *vsq, *npart, *Wsum, *sbe, *sbi;
+    if (project_ws(h, N, T, &pw) || ws_get(h, "npart", nll_partials(a.N), &npart) || ws_get(h, "fsum", nC * N * L * D, &fsum) ||
+        ws_get(h, "bsum", nC * N * L * D, &bsum) || ws_get(h, "xin", nC * N * L * D, &xin) || ws_get(h, "bin", nC * N * L * D, &bin) ||
+        ws_get(h, "Bx", L * 2 * 9, &Bx) || ws_get(h, "Wsum", scan_weights_doubles((int)L), &Wsum) || ws_get(h, "sbe", N * L * nSB * D, &sbe) ||
+        ws_get(h, "sbi", N * L * nSB * D, &sbi) || ws_get(h, "vsq", nC * N * L, &vsq))
+        return -1;
+    if (a.phase <= 1) {
+        // the projection residuals rho feed only the NLL; a block keeps them from phase 1 for its phase 3
+        CK(cudaMemsetAsync(pw.nanf, 0, 2 * sizeof(int), h->stream));
+        CK(launch_project(Y, h->d_U, h->d_S, h->p, (int)L, a.N, a.T, pw.u, nullptr, nullptr, (nll || a.phase == 1) ? pw.rho : nullptr, pw.nanf,
+                          pw.nanrows, (long long)pw.nan_cap, h->stream));
+        h->launches += 2;
+        mark(a.mk, "k_project");
+    }
+    a.u = pw.u; a.consts = h->d_consts; a.L = (int)L;
+    a.fsum = fsum; a.bsum = bsum; a.xin = xin; a.bin = bin; a.Bx = Bx; a.Wsum = Wsum; a.sb_end = sbe; a.sb_in = sbi; a.vsq = vsq;
+    CK(launch_scan((int)D, mode, a, h->stream));
+    h->launches += scan_launch_count(a.T);
+    if ((a.phase == 0 || a.phase == 3) && nll) {
+        CK(launch_nll_reduce(pw.rho, vsq, h->d_consts, h->d_S, h->sigma, h->p, (int)L, a.N, a.T, npart, nll, h->stream));
+        h->launches += 2;
+        mark(a.mk, "k_nll_reduce");
+    }
+    return 0;
+}
+
+// strict_chain: a forced many-chains path that cannot serve the pass fails (the entry point) or takes the scan (the sampler)
+static int fused_pass(moihgp_handle* h, const double* Y, size_t N, size_t T, const double* x0, int mode, double* X, double* Xs,
+                      double* Yhat, double* nll, double* xT, bool strict_chain) {
     if (!h || !Y) return -2;
     if (N == 0 || T == 0) return fail(h, "N and T must be positive");
     if (mode < -1 || mode > 1) return fail(h, "smoother_mode must be -1, 0 or 1");
     if (mode < 0 && Xs) return fail(h, "Xs requested with smoother_mode = none");
     DeviceGuard guard(h->device);
     const int L = h->L, D = h->dim;
-    const size_t nC = scan_chunks((long long)T);
     double* Xtmp = nullptr;
     if ((Yhat || Xs) && !X) { if (ws_get(h, "Xtmp", N * T * L * D, &Xtmp)) return -1; X = Xtmp; }
     Marker* mk = h->profiling ? &h->marker : nullptr;
     if (mk) { mk->st = h->stream; mk->mark("begin"); }
-    auto aligned16 = [](const void* q) { return (reinterpret_cast<size_t>(q) & 15) == 0; };
-    const size_t chain_warps = (N * (size_t)L + 31) / 32;
-    bool use_chain = chain_preferred(h->p, L, D, (long long)T) && aligned16(Y) && aligned16(X) && aligned16(Xs) && chain_warps >= 148;
-    if (h->path == 1) use_chain = false;
-    if (h->path == 2) {
-        if (!(chain_supported(h->p, L, D, (long long)T) && aligned16(Y) && aligned16(X) && aligned16(Xs))) return fail(h, "many-chains path not available for this shape/alignment");
-        use_chain = true;
-    }
+    const int use_chain = chain_path(h, N, T, Y, X, Xs, strict_chain);
+    if (use_chain < 0) return use_chain;
     if (use_chain) {
         // one thread per (sequence, latent) chain, sequential in time: chain.cu
         int* nanf;
@@ -591,33 +666,18 @@ int moihgp_cuda_filter_smoother_nll_dev(moihgp_handle* h, const double* Y, size_
         CK(launch_chain(h->p, L, D, c, h->stream));
         h->launches += Xs ? 2 : 1;
     } else {
-        // time-parallel chunked scan: project.cu + scan.cu
-        const size_t nC = scan_chunks((long long)T);
-        double *u, *rho, *fsum, *bsum, *xin, *bin, *Bx, *vsq, *npart, *Wsum, *sbe, *sbi;
-        int* nanf;
-        long long* nanrows;
-        const size_t nan_cap = std::min<size_t>(N * T, (size_t)1 << 22);
-        if (ws_get(h, "nanrows", nan_cap, &nanrows)) return -1;
-        if (ws_get(h, "u", N * L * T, &u) || ws_get(h, "rho", N * project_tiles((long long)T), &rho) || ws_get(h, "npart", nll_partials((long long)N), &npart) ||
-            ws_get(h, "fsum", nC * N * L * D, &fsum) ||
-            ws_get(h, "bsum", nC * N * L * D, &bsum) || ws_get(h, "xin", nC * N * L * D, &xin) || ws_get(h, "bin", nC * N * L * D, &bin) ||
-            ws_get(h, "Bx", (size_t)L * 2 * 9, &Bx) || ws_get(h, "Wsum", scan_weights_doubles(L), &Wsum) ||
-            ws_get(h, "sbe", N * L * scan_superblocks((long long)T) * D, &sbe) || ws_get(h, "sbi", N * L * scan_superblocks((long long)T) * D, &sbi) || ws_get(h, "vsq", nC * N * L, &vsq) || ws_get(h, "nanf", 4, &nanf))
-            return -1;
-        CK(cudaMemsetAsync(nanf, 0, 2 * sizeof(int), h->stream));
-        CK(launch_project(Y, h->d_U, h->d_S, h->p, L, (long long)N, (long long)T, u, nullptr, nullptr, nll ? rho : nullptr, nanf, nanrows,
-                          (long long)nan_cap, h->stream));
-        mark(mk, "k_project");
-        ScanArgs a;
+        ScanArgs a{};
         a.mk = mk;
-        a.u = u; a.consts = h->d_consts; a.L = L; a.N = (long long)N; a.T = (long long)T; a.x0 = x0;
-        a.fsum = fsum; a.bsum = bsum; a.xin = xin; a.bin = bin; a.Bx = Bx; a.Wsum = Wsum; a.sb_end = sbe; a.sb_in = sbi; a.X = X; a.Xs = Xs; a.vsq = vsq; a.xT = xT;
-        CK(launch_scan(D, mode < 0 ? 1 : mode, a, h->stream));
-        h->launches += 2 + scan_launch_count((long long)T);
-        if (nll) { CK(launch_nll_reduce(rho, vsq, h->d_consts, h->d_S, h->sigma, h->p, L, (long long)N, (long long)T, npart, nll, h->stream)); h->launches += 2; mark(mk, "k_nll_reduce"); }
+        a.N = (long long)N; a.T = (long long)T; a.x0 = x0; a.X = X; a.Xs = Xs; a.xT = xT;
+        if (const int rc = scan_pass(h, Y, mode < 0 ? 1 : mode, nll, a)) return rc;
     }
     if (Yhat) { CK(launch_backproject(X, h->d_U, h->d_S, h->p, L, D, (long long)N, (long long)T, Yhat, h->stream)); h->launches += 1; mark(mk, "k_backproject"); }
     return 0;
+}
+
+int moihgp_cuda_filter_smoother_nll_dev(moihgp_handle* h, const double* Y, size_t N, size_t T, const double* x0, int mode,
+                                        double* X, double* Xs, double* Yhat, double* nll, double* xT) {
+    return fused_pass(h, Y, N, T, x0, mode, X, Xs, Yhat, nll, xT, /*strict_chain=*/true);
 }
 
 // One contiguous block of a longer sequence sharded in TIME over several devices (chunked-scan path), in three phases
@@ -634,31 +694,15 @@ static int fsn_block_impl(moihgp_handle* h, int phase, const double* Y, size_t N
     if (phase == 3 && Xs && !X) return fail(h, "Xs needs X");
     DeviceGuard guard(h->device);
     const int L = h->L, D = h->dim;
-    const size_t nC = scan_chunks((long long)T);
-    double *u, *rho, *fsum, *bsum, *xin, *bin, *Bx, *vsq, *npart, *Wsum, *sbe, *sbi, *xe, *bo;
-    int* nanf;
-    long long* nanrows;
-    const size_t nan_cap = std::min<size_t>(N * T, (size_t)1 << 22);
-    if (ws_get(h, "nanrows", nan_cap, &nanrows)) return -1;
-    if (ws_get(h, "u", N * L * T, &u) || ws_get(h, "rho", N * project_tiles((long long)T), &rho) || ws_get(h, "npart", nll_partials((long long)N), &npart) ||
-        ws_get(h, "fsum", nC * N * L * D, &fsum) || ws_get(h, "bsum", nC * N * L * D, &bsum) || ws_get(h, "xin", nC * N * L * D, &xin) ||
-        ws_get(h, "bin", nC * N * L * D, &bin) || ws_get(h, "Bx", (size_t)L * 2 * 9, &Bx) || ws_get(h, "Wsum", scan_weights_doubles(L), &Wsum) ||
-        ws_get(h, "sbe", N * L * scan_superblocks((long long)T) * D, &sbe) || ws_get(h, "sbi", N * L * scan_superblocks((long long)T) * D, &sbi) ||
-        ws_get(h, "vsq", nC * N * L, &vsq) || ws_get(h, "nanf", 4, &nanf) || ws_get(h, "blk_xe", N * L * D, &xe) || ws_get(h, "blk_bo", N * L * D, &bo))
-        return -1;
-    if (phase == 1) {
-        CK(cudaMemsetAsync(nanf, 0, 2 * sizeof(int), h->stream));
-        CK(launch_project(Y, h->d_U, h->d_S, h->p, L, (long long)N, (long long)T, u, nullptr, nullptr, rho, nanf, nanrows, (long long)nan_cap, h->stream));
-        h->launches += 2;
-    }
-    ScanArgs a;
-    a.u = u; a.consts = h->d_consts; a.L = L; a.N = (long long)N; a.T = (long long)T; a.x0 = x0;
-    a.fsum = fsum; a.bsum = bsum; a.xin = xin; a.bin = bin; a.Bx = Bx; a.Wsum = Wsum; a.sb_end = sbe; a.sb_in = sbi; a.vsq = vsq;
+    double *xe, *bo;
+    if (ws_get(h, "blk_xe", N * L * D, &xe) || ws_get(h, "blk_bo", N * L * D, &bo)) return -1;
+    ScanArgs a{};
+    a.N = (long long)N; a.T = (long long)T; a.x0 = x0;
     a.X = phase == 3 ? X : nullptr; a.Xs = phase == 3 ? Xs : nullptr; a.xT = phase == 3 ? xT : nullptr;
     a.phase = phase; a.seq_end = seq_end ? 1 : 0; a.u_after = seq_end ? nullptr : u_after; a.b_end = phase == 3 ? b_end : nullptr;
     a.x_end = phase == 1 ? xe : nullptr; a.b_out = phase == 2 ? bo : nullptr;
-    CK(launch_scan(D, mode, a, h->stream));
-    h->launches += scan_launch_count((long long)T);
+    if (const int rc = scan_pass(h, Y, mode, nll, a)) return rc;
+    const double* u = a.u;
     if (phase == 1 && host_out) {
         // [N][L][D + 1]: the block's end state from x0, then its first projected observation (the previous block's u_after)
         std::vector<double> hx(N * L * D), hu(N * L);
@@ -681,10 +725,6 @@ static int fsn_block_impl(moihgp_handle* h, int phase, const double* Y, size_t N
         CK(cudaMemcpy2DAsync(dev_out + D, sizeof(double) * (D + 1), u, sizeof(double) * T, sizeof(double), N * L, cudaMemcpyDeviceToDevice, h->stream));
     }
     if (phase == 2 && dev_out) CK(cudaMemcpyAsync(dev_out, bo, sizeof(double) * N * L * D, cudaMemcpyDeviceToDevice, h->stream));
-    if (phase == 3 && nll) {
-        CK(launch_nll_reduce(rho, vsq, h->d_consts, h->d_S, h->sigma, h->p, L, (long long)N, (long long)T, npart, nll, h->stream));
-        h->launches += 2;
-    }
     return 0;
 }
 
@@ -829,9 +869,7 @@ static int fsn_host(moihgp_handle* h, const double* Y, size_t N, size_t T, const
     }
     CK(cudaStreamSynchronize(h->s_out));
     CK(cudaStreamSynchronize(h->stream));
-    for (size_t i = 0; i < nsl; ++i)
-        if (flags[i] == 2) return fail(h, "more than 2^22 observations with missing (NaN) outputs in one call: split the batch");
-    return 0;
+    return refuse_nan_overflow(h, flags, nsl);
 }
 
 int moihgp_cuda_filter_smoother_nll(moihgp_handle* h, const double* Y, size_t N, size_t T, const double* x0, int mode, double* X,
@@ -906,14 +944,10 @@ int moihgp_cuda_sample_posterior_dev(moihgp_handle* h, const double* Y, size_t N
     if (!Xs_mean && ws_get(h, "sXs", N * T * L * D, &Xs_mean)) return -1;
     // set_path also selects the sampler's variant (1 time-chunked, 2 one pass); the mean pass then takes the many-chains
     // kernels only where they serve the shape
-    const int path = h->path;
-    auto aligned16 = [](const void* q) { return (reinterpret_cast<size_t>(q) & 15) == 0; };
-    if (path == 2 && !(chain_supported(h->p, L, D, (long long)T) && aligned16(Y) && aligned16(Xs_mean))) h->path = 0;
-    const int rc = moihgp_cuda_filter_smoother_nll_dev(h, Y, N, T, x0, MOIHGP_SMOOTH_RTS, nullptr, Xs_mean, nullptr, nullptr, nullptr);
-    h->path = path;
+    const int rc = fused_pass(h, Y, N, T, x0, MOIHGP_SMOOTH_RTS, nullptr, Xs_mean, nullptr, nullptr, nullptr, /*strict_chain=*/false);
     if (rc) return rc;
     const long long chains = (long long)(S * N * L);
-    const bool chunked = sample_chunked((long long)T, chains, path);
+    const bool chunked = sample_chunked((long long)T, chains, h->path);
     SampleArgs a;
     a.consts = h->d_consts; a.S = (long long)S; a.N = (long long)N; a.T = (long long)T; a.L = L; a.seed = seed;
     a.Xs = Xs_mean; a.Xsamp = Xsamp; a.F = Fsamp; a.carry = nullptr;
@@ -951,10 +985,7 @@ int moihgp_cuda_sample_posterior(moihgp_handle* h, const double* Y, size_t N, si
     if (Xsamp) CK(cudaMemcpyAsync(Xsamp, dX, sizeof(double) * S * N * T * L * D, cudaMemcpyDeviceToHost, h->stream));
     if (Fsamp) CK(cudaMemcpyAsync(Fsamp, dF, sizeof(double) * S * N * T * L, cudaMemcpyDeviceToHost, h->stream));
     if (Ysamp) CK(cudaMemcpyAsync(Ysamp, dYs, sizeof(double) * S * N * T * p, cudaMemcpyDeviceToHost, h->stream));
-    int status = 0;
-    if (moihgp_cuda_nan_status(h, &status)) return -1;   // waits for the stream
-    if (status == 2) return fail(h, "more than 2^22 observations with missing (NaN) outputs in one call: split the batch");
-    return 0;
+    return refuse_nan_overflow(h);                       // waits for the copies
 }
 
 // phase 0: whole evaluation; 1: begin (projection, summaries, block end from a zero carry-in -> zend, device);
@@ -966,22 +997,18 @@ static int objective_phase(moihgp_handle* h, int phase, const double* Y, size_t 
     DeviceGuard guard(h->device);
     const int L = h->L, D = h->dim, p = h->p;
     const size_t nC = obj_chunks((long long)T), nsplit = obj_gu_splits((long long)N, (long long)T);
-    double *u, *w, *yl, *rho, *zsum, *zin, *zsub, *part, *gU, *Ek, *lat;
-    int* nanf;
-    long long* nanrows;
-    const size_t nan_cap = std::min<size_t>(N * T, (size_t)1 << 22);
-    if (ws_get(h, "nanrows", nan_cap, &nanrows)) return -1;
-    if (ws_get(h, "u", N * L * T, &u) || ws_get(h, "w", N * L * T, &w) || ws_get(h, "yl", N * L * T, &yl) || ws_get(h, "rho", N * project_tiles((long long)T), &rho) ||
+    ProjectWs pw;
+    double *w, *yl, *zsum, *zin, *zsub, *part, *gU, *Ek, *lat;
+    if (project_ws(h, N, T, &pw) || ws_get(h, "w", N * L * T, &w) || ws_get(h, "yl", N * L * T, &yl) ||
         ws_get(h, "zsum", nC * N * L * 4 * D, &zsum) || ws_get(h, "zin", nC * N * L * 4 * D, &zin) || ws_get(h, "zsub", nC * 8 * N * L * 4 * D, &zsub) ||
         ws_get(h, "part", nC * N * L * 8, &part) ||
-        ws_get(h, "gU", nsplit * p * L, &gU) || ws_get(h, "Ek", (size_t)L * 27 * 16, &Ek) || ws_get(h, "lat", ((size_t)L + 1) * 8 * 16, &lat) ||
-        ws_get(h, "nanf", 4, &nanf))
+        ws_get(h, "gU", nsplit * p * L, &gU) || ws_get(h, "Ek", (size_t)L * 27 * 16, &Ek) || ws_get(h, "lat", ((size_t)L + 1) * 8 * 16, &lat))
         return -1;
     Marker* mk = h->profiling ? &h->marker : nullptr;
     if (mk) { mk->st = h->stream; mk->mark("begin"); }
     if (phase != 2) {
-        CK(cudaMemsetAsync(nanf, 0, 2 * sizeof(int), h->stream));
-        CK(launch_project(Y, h->d_U, h->d_S, p, L, (long long)N, (long long)T, u, w, yl, rho, nanf, nanrows, (long long)nan_cap, h->stream));
+        CK(cudaMemsetAsync(pw.nanf, 0, 2 * sizeof(int), h->stream));
+        CK(launch_project(Y, h->d_U, h->d_S, p, L, (long long)N, (long long)T, pw.u, w, yl, pw.rho, pw.nanf, pw.nanrows, (long long)pw.nan_cap, h->stream));
         mark(mk, "k_project");
         h->launches += 2;
     }
@@ -989,7 +1016,7 @@ static int objective_phase(moihgp_handle* h, int phase, const double* Y, size_t 
     a.mk = mk;
     a.phase = phase;
     a.zend = zend;
-    a.Y = Y; a.u = u; a.w = w; a.yl = yl; a.rho = rho; a.wgt = w;   // the weights overwrite w in place (same thread, same index)
+    a.Y = Y; a.u = pw.u; a.w = w; a.yl = yl; a.rho = pw.rho; a.wgt = w;   // the weights overwrite w in place (same thread, same index)
     a.consts = h->d_consts; a.U = h->d_U; a.S = h->d_S; a.sigma = h->sigma; a.p = p; a.L = L; a.threading = h->threading;
     a.N = (long long)N; a.T = (long long)T; a.x0 = x0; a.dx0 = dx0; a.zsum = zsum; a.zin = zin; a.zsub = zsub; a.part = part; a.gU_part = gU;
     a.Ek = Ek; a.lat_sums = lat; a.loss = loss; a.grad = grad; a.xT = xT; a.dxT = dxT;
@@ -1079,40 +1106,42 @@ static int objective_small(moihgp_handle* h, const double* Y, const double* Y_re
     return 0;
 }
 
-int moihgp_cuda_objective(moihgp_handle* h, const double* Y, size_t N, size_t T, const double* x0, const double* dx0, double* loss,
-                          double* grad, double* xT, double* dxT) {
-    if (!h || !Y || !loss || !grad) return -2;
-    if (N == 0 || T == 0) return fail(h, "N and T must be positive");
+// The objective on host buffers, over host Y (copied in) or over Y_resident, observations already on the device.
+static int objective_host(moihgp_handle* h, const double* Y, const double* Y_resident, size_t N, size_t T, const double* x0,
+                          const double* dx0, double* loss, double* grad, double* xT, double* dxT) {
     DeviceGuard guard(h->device);
     if (N == 1 && h->path != 1 && obj_small_smem(h->p, h->L, (long long)T)) {
-        const int rs = objective_small(h, Y, nullptr, T, x0, dx0, loss, grad, xT, dxT);
+        const int rs = objective_small(h, Y, Y_resident, T, x0, dx0, loss, grad, xT, dxT);
         if (rs <= 0) return rs;                  // 1: missing observations -> the general path below
     }
     const size_t L = h->L, D = h->dim, p = h->p, np = h->num_param;
-    double *dY, *dx = nullptr, *ddx = nullptr, *dout, *dxT_ = nullptr, *ddxT = nullptr;
-    if (ws_get(h, "hY", N * T * p, &dY) || ws_get(h, "hout", np + 2, &dout)) return -1;
+    double *dY = nullptr, *dx = nullptr, *ddx = nullptr, *dout, *dxT_ = nullptr, *ddxT = nullptr;
+    if (!Y_resident && ws_get(h, "hY", N * T * p, &dY)) return -1;
+    if (ws_get(h, "hout", np + 2, &dout)) return -1;
     if (x0 && ws_get(h, "hx0", N * L * D, &dx)) return -1;
     if (dx0 && ws_get(h, "hdx0", N * L * 3 * D, &ddx)) return -1;
     if (xT && ws_get(h, "hxT", N * L * D, &dxT_)) return -1;
     if (dxT && ws_get(h, "hdxT", N * L * 3 * D, &ddxT)) return -1;
-    CK(cudaMemcpyAsync(dY, Y, sizeof(double) * N * T * p, cudaMemcpyHostToDevice, h->stream));
+    if (!Y_resident) CK(cudaMemcpyAsync(dY, Y, sizeof(double) * N * T * p, cudaMemcpyHostToDevice, h->stream));
     if (x0) CK(cudaMemcpyAsync(dx, x0, sizeof(double) * N * L * D, cudaMemcpyHostToDevice, h->stream));
     if (dx0) CK(cudaMemcpyAsync(ddx, dx0, sizeof(double) * N * L * 3 * D, cudaMemcpyHostToDevice, h->stream));
-    const int rc = moihgp_cuda_objective_dev(h, dY, N, T, dx, ddx, dout, dout + 2, dxT_, ddxT);
+    const int rc = moihgp_cuda_objective_dev(h, Y_resident ? Y_resident : dY, N, T, dx, ddx, dout, dout + 2, dxT_, ddxT);
     if (rc) return rc;
     std::vector<double> host(np + 2);
     CK(cudaMemcpyAsync(host.data(), dout, sizeof(double) * (np + 2), cudaMemcpyDeviceToHost, h->stream));
     if (xT) CK(cudaMemcpyAsync(xT, dxT_, sizeof(double) * N * L * D, cudaMemcpyDeviceToHost, h->stream));
     if (dxT) CK(cudaMemcpyAsync(dxT, ddxT, sizeof(double) * N * L * 3 * D, cudaMemcpyDeviceToHost, h->stream));
-    int flag = 0;
-    int* nanf;
-    if (ws_get(h, "nanf", 4, &nanf)) return -1;
-    CK(cudaMemcpyAsync(&flag, nanf, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaStreamSynchronize(h->stream));
+    if (const int refused = refuse_nan_overflow(h)) return refused;   // waits for the copies
     *loss = host[0];
     std::copy(host.begin() + 2, host.end(), grad);
-    if (flag == 2) return fail(h, "more than 2^22 observations with missing (NaN) outputs in one call: split the batch");
     return 0;   // with NaN observations the loss is NaN, exactly as the reference's (moihgp.h:501 uses the full y)
+}
+
+int moihgp_cuda_objective(moihgp_handle* h, const double* Y, size_t N, size_t T, const double* x0, const double* dx0, double* loss,
+                          double* grad, double* xT, double* dxT) {
+    if (!h || !Y || !loss || !grad) return -2;
+    if (N == 0 || T == 0) return fail(h, "N and T must be positive");
+    return objective_host(h, Y, nullptr, N, T, x0, dx0, loss, grad, xT, dxT);
 }
 
 // Resident data set: the L-BFGS loop evaluates the objective tens of times on the SAME observations (LBFGSB.h:137,
@@ -1135,30 +1164,7 @@ int moihgp_cuda_bind_data(moihgp_handle* h, const double* Y, size_t N, size_t T)
 int moihgp_cuda_objective_bound(moihgp_handle* h, const double* x0, const double* dx0, double* loss, double* grad, double* xT, double* dxT) {
     if (!h || !loss || !grad) return -2;
     if (!h->d_bound) return fail(h, "no data bound: call moihgp_cuda_bind_data first");
-    DeviceGuard guard(h->device);
-    const size_t N = h->bound_N, T = h->bound_T, L = h->L, D = h->dim, np = h->num_param;
-    if (N == 1 && h->path != 1 && obj_small_smem(h->p, h->L, (long long)T)) {
-        const int rs = objective_small(h, nullptr, h->d_bound, T, x0, dx0, loss, grad, xT, dxT);
-        if (rs <= 0) return rs;
-    }
-    double *dx = nullptr, *ddx = nullptr, *dout, *dxT_ = nullptr, *ddxT = nullptr;
-    if (ws_get(h, "hout", np + 2, &dout)) return -1;
-    if (x0 && ws_get(h, "hx0", N * L * D, &dx)) return -1;
-    if (dx0 && ws_get(h, "hdx0", N * L * 3 * D, &ddx)) return -1;
-    if (xT && ws_get(h, "hxT", N * L * D, &dxT_)) return -1;
-    if (dxT && ws_get(h, "hdxT", N * L * 3 * D, &ddxT)) return -1;
-    if (x0) CK(cudaMemcpyAsync(dx, x0, sizeof(double) * N * L * D, cudaMemcpyHostToDevice, h->stream));
-    if (dx0) CK(cudaMemcpyAsync(ddx, dx0, sizeof(double) * N * L * 3 * D, cudaMemcpyHostToDevice, h->stream));
-    const int rc = moihgp_cuda_objective_dev(h, h->d_bound, N, T, dx, ddx, dout, dout + 2, dxT_, ddxT);
-    if (rc) return rc;
-    std::vector<double> host(np + 2);
-    CK(cudaMemcpyAsync(host.data(), dout, sizeof(double) * (np + 2), cudaMemcpyDeviceToHost, h->stream));
-    if (xT) CK(cudaMemcpyAsync(xT, dxT_, sizeof(double) * N * L * D, cudaMemcpyDeviceToHost, h->stream));
-    if (dxT) CK(cudaMemcpyAsync(dxT, ddxT, sizeof(double) * N * L * 3 * D, cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaStreamSynchronize(h->stream));
-    *loss = host[0];
-    std::copy(host.begin() + 2, host.end(), grad);
-    return 0;
+    return objective_host(h, nullptr, h->d_bound, h->bound_N, h->bound_T, x0, dx0, loss, grad, xT, dxT);
 }
 
 }  // extern "C"

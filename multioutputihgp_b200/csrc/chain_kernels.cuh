@@ -30,7 +30,6 @@
 #include <cuda_runtime.h>
 #include <math.h>
 #include <cmath>
-#include <cstdlib>
 #include "moihgp_device.cuh"
 #include "tma.cuh"
 #include "launch.h"
@@ -674,24 +673,18 @@ cudaError_t run_chain_ns(const ChainArgs& a, cudaStream_t st) {
         cudaFuncSetAttribute(k_smooth_chain<L, D, 1, SNS, SRM, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SS::BYTES);
         cudaFuncSetAttribute(k_smooth_chain<L, D, 0, SNS, SRM, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SS::BYTES);
         cudaFuncSetAttribute(k_smooth_chain<L, D, 1, SNS, SRM, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SS::BYTES);
-        cudaFuncSetAttribute(k_smooth_chain<L, D, 0, NS, 1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SmoothCfg<L, D, NS, 1>::BYTES);
-        cudaFuncSetAttribute(k_smooth_chain<L, D, 1, NS, 1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SmoothCfg<L, D, NS, 1>::BYTES);
     }
     if (!padded) k_filter_chain<P, L, D, NS, false><<<grid, 32, FS::BYTES, st>>>(a.Y, pc, a.consts, a.sigma, a.nll_const, a.N, a.T, a.x0, a.X, a.nll, a.xT, a.nan_flag, P, L);
     else k_filter_chain<P, L, D, NS, true><<<grid, 32, FS::BYTES, st>>>(a.Y, pc, a.consts, a.sigma, a.nll_const, a.N, a.T, a.x0, a.X, a.nll, a.xT, a.nan_flag, p_real, L_real);
     mark(a.mk, "k_filter_chain");
     if (a.Xs) {
-        static const bool long_rounds = []() { const char* e = std::getenv("MOIHGP_SMOOTH_LONG_ROUNDS"); return !(e && e[0] == '0'); }();
         const unsigned sgrid = (unsigned)((a.N + SNS - 1) / SNS);
         if (padL) {
             if (a.mode == 0) k_smooth_chain<L, D, 0, SNS, SRM, true><<<sgrid, 32, SS::BYTES, st>>>(a.X, a.consts, a.N, a.T, a.Xs, L_real);
             else k_smooth_chain<L, D, 1, SNS, SRM, true><<<sgrid, 32, SS::BYTES, st>>>(a.X, a.consts, a.N, a.T, a.Xs, L_real);
-        } else if (long_rounds) {
+        } else {
             if (a.mode == 0) k_smooth_chain<L, D, 0, SNS, SRM, false><<<sgrid, 32, SS::BYTES, st>>>(a.X, a.consts, a.N, a.T, a.Xs, L);
             else k_smooth_chain<L, D, 1, SNS, SRM, false><<<sgrid, 32, SS::BYTES, st>>>(a.X, a.consts, a.N, a.T, a.Xs, L);
-        } else {
-            if (a.mode == 0) k_smooth_chain<L, D, 0, NS, 1, false><<<grid, 32, SmoothCfg<L, D, NS, 1>::BYTES, st>>>(a.X, a.consts, a.N, a.T, a.Xs, L);
-            else k_smooth_chain<L, D, 1, NS, 1, false><<<grid, 32, SmoothCfg<L, D, NS, 1>::BYTES, st>>>(a.X, a.consts, a.N, a.T, a.Xs, L);
         }
         mark(a.mk, "k_smooth_chain");
     }

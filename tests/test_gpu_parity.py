@@ -855,6 +855,22 @@ def test_bound_data_objective_equals_host_buffer_objective(cuda_lib):
 
 
 @pytest.mark.gpu
+@pytest.mark.parametrize("entry", ["objective", "objective_bound"])
+def test_host_objective_refuses_more_than_2_22_missing_rows(cuda_lib, entry):
+    """Both host-buffer objective entry points refuse a call with more than 2^22 rows with missing outputs (the rows beyond
+    that are not re-projected), whether the observations come with the call or were bound to the device before."""
+    from multioutputihgp_b200 import MOIHGPSequences
+    p, L, T = 2, 1, (1 << 22) + 64
+    m = MOIHGPSequences(0.1, p, L, "Matern32", True)
+    Y = np.full((1, T, p), np.nan)
+    if entry == "objective_bound":
+        m.bind(Y)
+    with pytest.raises(RuntimeError, match=r"more than 2\^22 observations with missing \(NaN\) outputs"):
+        m.objective(Y) if entry == "objective" else m.objective_bound()
+    assert m.nan_status == 2
+
+
+@pytest.mark.gpu
 @pytest.mark.parametrize("path,kernel,p,L,N,T", [("chain", "Matern52", 16, 8, 5, 203), ("chain", "Matern32", 8, 4, 9, 37),
                                                  ("chain", "Matern52", 4, 2, 37, 45), ("chain", "Matern52", 10, 4, 11, 57), ("chain", "Matern32", 22, 8, 5, 43), ("chain", "Matern52", 7, 2, 19, 41), ("chain", "Matern32", 2, 1, 45, 50), ("chain", "Matern32", 9, 5, 9, 47), ("chain", "Matern52", 12, 6, 7, 39), ("chain", "Matern52", 9, 3, 13, 46), ("chain", "Matern32", 32, 2, 19, 70), ("chain", "Matern52", 4, 4, 9, 66),
                                                  ("scan", "Matern52", 16, 8, 3, 515), ("scan", "Matern32", 5, 3, 2, 257)])
