@@ -70,7 +70,7 @@ struct moihgp_handle {
         double *d_params = nullptr, *d_old = nullptr, *d_B = nullptr, *d_out = nullptr;
         double *h_params = nullptr, *h_out = nullptr, *h_y = nullptr;                  // pinned
         int *d_count = nullptr, *d_pst = nullptr;
-        bool has_B = false, has_prox = true, use_graph = true;
+        bool has_B = false, has_prox = true;
         std::map<long long, int> seen;                    // evaluations per (window length, proximal kind)
         std::map<long long, cudaGraphExec_t> graphs;
     } on;
@@ -1225,8 +1225,6 @@ int moihgp_cuda_online_begin(moihgp_handle* h, size_t windowsize) {
     CK(cudaMemcpyAsync(o.d_old, cur.data(), sizeof(double) * np, cudaMemcpyHostToDevice, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     o.W = windowsize; o.count = 0; o.has_B = false; o.has_prox = true;
-    const char* e = std::getenv("MOIHGP_ONLINE_GRAPH");
-    o.use_graph = !(e && e[0] == '0');
     return 0;
 }
 
@@ -1303,7 +1301,7 @@ int moihgp_cuda_online_objective(moihgp_handle* h, const double* params, double*
     const long long key = (long long)o.count * 4 + (o.has_prox ? 2 : 0) + (o.has_B ? 1 : 0);
     const int seen = o.seen[key]++;
     auto it = o.graphs.find(key);
-    if (o.use_graph && it == o.graphs.end() && seen >= 1) {
+    if (it == o.graphs.end() && seen >= 1) {
         // second evaluation with this window length: record the sequence once (the first one ran eagerly and set every
         // function attribute / workspace), replay it from now on
         cudaGraph_t g = nullptr;

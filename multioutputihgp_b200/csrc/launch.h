@@ -30,7 +30,7 @@ cudaError_t launch_setup(int dim, const double* d_igp_params, double dt, int L, 
 
 // polar.cu  (MOIHGP::update's polar factor on the device, for large p * L)
 size_t polar_smem_bytes(int p, int L);
-cudaError_t launch_polar(const double* A /*[p][L]*/, int p, int L, double* U, int* status /*device int or null*/, cudaStream_t st);
+cudaError_t launch_polar(const double* A /*[p][L]*/, int p, int L, double* U, int* status /*device int*/, cudaStream_t st);
 
 // project.cu
 size_t project_tiles(long long T);     // tiles of 128 time steps per sequence: rho_part is [N][project_tiles(T)]

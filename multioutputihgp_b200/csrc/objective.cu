@@ -20,7 +20,6 @@
 // Q8 (pv uses the RAW y(l)), Q9 (norm not squared; 1/2 log(sum S)), Q20 (dv_k uses HdA_k(0) x(0)).
 #include <cuda_runtime.h>
 #include <math.h>
-#include <stdlib.h>
 #include "moihgp_device.cuh"
 #include "small_mat.cuh"
 #include "tma.cuh"
@@ -1185,7 +1184,7 @@ cudaError_t run_objective(const ObjArgs& a, cudaStream_t st) {
     // phase 0: the whole evaluation; phase 1 ("begin"): summaries + the block's end state from a zero carry-in;
     // phase 2 ("finish"): from the true carry-in, reusing the projected series and the summaries of phase 1
     // thread-per-sub-chunk kernels when the latents come in whole groups of 8, else the warp-scan kernel
-    const bool lanes = a.L % 8 == 0 && getenv("MOIHGP_OBJ_WARP") == nullptr;        // A/B switch, read per call
+    const bool lanes = a.L % 8 == 0;
     if (a.phase != 2 && (nC > 1 || a.phase == 1)) {
         if (lanes) {
             // interior chunks (whole) by k_obj_lanes; the last chunk of the sequence (possibly ragged) by the warp-scan kernel

@@ -8,7 +8,6 @@
 // k_polar_ns (below) gets the same factor by the Newton-Schulz iteration and runs first; the Jacobi kernel is its fallback.
 #include <cuda_runtime.h>
 #include <math.h>
-#include <stdlib.h>
 #include "launch.h"
 
 namespace moihgp {
@@ -256,7 +255,8 @@ size_t polar_ns_smem_bytes(int p, int L) {
     return sizeof(double) * ((size_t)p * PX + Lp * PX + 1024);
 }
 
-// status: one device int (workspace) or null.  With it, Newton-Schulz runs first and the Jacobi kernel only if it asks.
+// status: one device int (workspace).  Where its shared memory fits, Newton-Schulz runs first and the Jacobi kernel only if
+// it asks; elsewhere the Jacobi kernel alone.
 cudaError_t launch_polar(const double* A, int p, int L, double* U, int* status, cudaStream_t st) {
     const size_t smem = polar_smem_bytes(p, L);
     if (smem > 200 * 1024) return cudaErrorInvalidValue;
@@ -266,7 +266,7 @@ cudaError_t launch_polar(const double* A, int p, int L, double* U, int* status, 
         cudaFuncSetAttribute(k_polar_ns, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
     }
     const size_t ns = polar_ns_smem_bytes(p, L);
-    const bool use_ns = status != nullptr && L <= 64 && ns <= 200 * 1024 && getenv("MOIHGP_POLAR_JACOBI") == nullptr;
+    const bool use_ns = ns <= 200 * 1024;
     if (use_ns) k_polar_ns<<<1, 1024, ns, st>>>(A, p, L, U, status);
     const int Lp = (L + 1) & ~1;
     int warps = Lp / 2;

@@ -19,13 +19,13 @@
 // k_project_rows<NB, NW, NST>: the same contraction as a PERSISTENT kernel without CTA-wide barriers in its loop.  U is
 //   staged into shared memory once per CTA; every warp owns units of 16 consecutive rows of Y and its own ring of NST
 //   stages, filled by TMA tensor copies (cp.async.bulk.tensor, 128-byte swizzle, mbarrier completion) NST - 1 items
-//   ahead of the tensor-pipe loop.  Used whenever U (padded) and the rings fit into shared memory and p is even.
+//   ahead of the tensor-pipe loop.  Used for even p >= 8 and a 16-byte aligned Y whenever U (padded) and the rings of one
+//   of the four configurations of try_project_rows fit into shared memory; k_project_mma serves the other such shapes.
 // The residual norms are written as one partial sum per 16 rows: rho_part[n][ceil(T / 16)] (project_tiles).
 #include <cuda.h>
 #include <cuda_runtime.h>
 #include <math.h>
 #include <algorithm>
-#include <cstdlib>
 #include "moihgp_device.cuh"
 #include "launch.h"
 #include "ls_project.cuh"
@@ -707,17 +707,18 @@ cudaError_t run_project_rows(const CUtensorMap& tm, const double* Y, const doubl
     return cudaGetLastError();
 }
 
-// picks (warps, stages, panel width) so that U and the rings fit into 227 KB; false = shape not served by k_project_rows
+// the first configuration (warps, stages, boxes per stage), in order of falling ring size, whose rings fit into 227 KB
+// beside U: 1 = (16, 2, up to 2), 2 = (16, 3, 1), 5 = (8, 2, up to 2), 8 = (8, 2, 1); false = shape not served by
+// k_project_rows
 template <int NB>
 bool try_project_rows(cudaError_t& e, const double* Y, const double* U, const double* S, int p, int L, long long N, long long T, double* u,
                       double* w, double* yl, double* rho_part, int* nan_info, long long* nan_rows, long long nan_cap, cudaStream_t stream) {
     using SMC = RowsSmem<NB>;
     const size_t cap = 227 * 1024;
-    static const int force = std::getenv("MOIHGP_PROJECT_ROWS_CFG") ? std::atoi(std::getenv("MOIHGP_PROJECT_ROWS_CFG")) : 0;   // A/B runs only
     const long long rows = N * T, ups = (T + RU - 1) / RU;
     if (rows >= (1LL << 31) || ups * N >= (1LL << 31) || !encode_tiled_fn()) return false;
     const int nb_all = (p + 15) / 16;
-    const int nb_wide = nb_all < 4 ? nb_all : 4, nb_narrow = nb_all < 2 ? nb_all : 2;
+    const int nb_narrow = nb_all < 2 ? nb_all : 2;
     alignas(64) CUtensorMap tm;
     const cuuint64_t gdim[2] = {(cuuint64_t)p, (cuuint64_t)rows};
     const cuuint64_t gstr[1] = {(cuuint64_t)p * 8};
@@ -725,16 +726,15 @@ bool try_project_rows(cudaError_t& e, const double* Y, const double* U, const do
     if (encode_tiled_fn()(&tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 2, const_cast<double*>(Y), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                           CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
         return false;
-#define MOIHGP_TRY_ROWS(ID, NW_, NST_, NBOX_)                                                                                       \
-    if ((force == 0 || force == ID) && SMC::bytes(p, NBOX_, NW_, NST_) <= cap) {                                                    \
+#define MOIHGP_TRY_ROWS(NW_, NST_, NBOX_)                                                                                           \
+    if (SMC::bytes(p, NBOX_, NW_, NST_) <= cap) {                                                                                   \
         e = run_project_rows<NB, NW_, NST_>(tm, Y, U, S, p, L, N, T, NBOX_, u, w, yl, rho_part, nan_info, nan_rows, nan_cap, stream); \
         return true;                                                                                                                \
     }
-    MOIHGP_TRY_ROWS(1, 16, 2, nb_narrow)
-    MOIHGP_TRY_ROWS(2, 16, 3, 1)
-    MOIHGP_TRY_ROWS(3, 12, 2, nb_wide)
-    MOIHGP_TRY_ROWS(5, 8, 2, nb_narrow)
-    MOIHGP_TRY_ROWS(8, 8, 2, 1)
+    MOIHGP_TRY_ROWS(16, 2, nb_narrow)   // 1
+    MOIHGP_TRY_ROWS(16, 3, 1)           // 2
+    MOIHGP_TRY_ROWS(8, 2, nb_narrow)    // 5
+    MOIHGP_TRY_ROWS(8, 2, 1)            // 8
 #undef MOIHGP_TRY_ROWS
     return false;
 }
@@ -748,9 +748,8 @@ cudaError_t launch_project(const double* Y, const double* U, const double* S, in
                            cudaStream_t stream) {
     const bool aligned = (reinterpret_cast<size_t>(Y) & 15) == 0;
     cudaError_t e = cudaSuccess;
-    static const bool no_rows = std::getenv("MOIHGP_PROJECT_ROWS_OFF") != nullptr;      // A/B runs only
     bool done = false;
-    if (p % 2 == 0 && aligned && L <= 64 && p >= 8 && !no_rows) {
+    if (p % 2 == 0 && aligned && L <= 64 && p >= 8) {
         if (L <= 8) done = try_project_rows<1>(e, Y, U, S, p, L, N, T, u, w, yl, rho_part, nan_info, nan_rows, nan_cap, stream);
         else if (L <= 16) done = try_project_rows<2>(e, Y, U, S, p, L, N, T, u, w, yl, rho_part, nan_info, nan_rows, nan_cap, stream);
         else if (L <= 32) done = try_project_rows<4>(e, Y, U, S, p, L, N, T, u, w, yl, rho_part, nan_info, nan_rows, nan_cap, stream);

@@ -27,9 +27,7 @@
 // A block of a longer sequence sharded in time over several devices runs the same kernels in three
 // phases (run_scan; ScanArgs::phase, seq_end, u_after, b_end): SURVEY.md section 8(e).
 #include <cuda_runtime.h>
-#include <cstdlib>
 #include <math.h>
-#include <stdlib.h>
 #include "moihgp_device.cuh"
 #include "small_mat.cuh"
 #include "tma.cuh"
@@ -1152,8 +1150,7 @@ cudaError_t run_scan(const ScanArgs& a, cudaStream_t st) {
     mark(a.mk, "k_carry");
     if (ph == 2) return cudaGetLastError();
     // final pass: thread-per-sub-chunk kernel when the latents come in whole groups of 16 or 8, else the warp-per-chunk one
-    const bool force_warp = getenv("MOIHGP_SCAN_FINAL_WARP") != nullptr;   // A/B switch, read per call
-    if (!force_warp && a.L % 8 == 0) {
+    if (a.L % 8 == 0) {
         const cudaError_t e = a.L % 16 == 0 ? launch_scan_lanes<D, MODE, 16>(a, nC, st) : launch_scan_lanes<D, MODE, 8>(a, nC, st);
         mark(a.mk, "k_scan_final");
         return e;

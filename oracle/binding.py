@@ -4,7 +4,7 @@
 * ``RefMOIHGP``     - oracle/_ref/libmoihgp_ref*.so, the UNMODIFIED reference sources compiled against
                       the Eigen-API shim (only exists where /root/reference was present at build time).
 
-Only tests/, ``__graft_entry__.smoke()`` and bench.py's CPU-baseline legs may import this module.
+Only tests/, ``__graft_entry__.smoke()``, bench.py's CPU-baseline legs and scripts/gpu_fuzz.py may import this module.
 """
 import ctypes
 import os

@@ -1,6 +1,7 @@
-"""Differential fuzz on the GPU: random shapes through the alternative implementations of the same pass -
-thread-per-sub-chunk vs warp-per-chunk kernels (scan final pass, objective scan), many-chains vs chunked-scan path,
-one-launch vs general objective, time-sharded blocks vs the whole sequence.  Prints a summary; exits non-zero on a mismatch."""
+"""Differential fuzz on the GPU: random shapes through the chunked-scan pass and the general objective against the CPU
+oracle (L drawn on both sides of the multiple-of-8 rule, so both the thread-per-sub-chunk and the warp-per-chunk kernels
+run), and through the alternative implementations of the same pass - many-chains vs chunked-scan path, one-launch vs
+general objective, time-sharded blocks vs the whole sequence.  Prints a summary; exits non-zero on a mismatch."""
 import os
 import sys
 
@@ -10,8 +11,10 @@ import torch
 
 from multioutputihgp_b200 import MOIHGPSequences
 from multioutputihgp_b200.parallel import backward_carry_in, forward_carry_in
+from oracle.binding import OracleMOIHGP
 from oracle.gen_golden import make_data, make_params
 
+TOL = 1e-9          # fp64 agreement with the oracle, norm-wise relative (tests/conftest.py)
 CASES = int(os.environ.get("FUZZ_CASES", 120))
 rng = np.random.default_rng(int(os.environ.get("FUZZ_SEED", 2024)))
 dev = torch.device("cuda:0")
@@ -40,20 +43,20 @@ for case in range(CASES):
     ctx = (kernel, p, L, N, T)
     params = make_params(rng, p, L, kernel)
     Y = np.stack([make_data(rng, p, L, T) for _ in range(N)])
-    m = MOIHGPSequences(0.1, p, L, kernel, bool(rng.integers(2)))
+    threading = bool(rng.integers(2))
+    m = MOIHGPSequences(0.1, p, L, kernel, threading)
+    o = OracleMOIHGP(0.1, p, L, kernel, threading)
     m.update(params)
+    o.update(params)
     d = m.igp_dim
     x0 = 0.3 * rng.standard_normal((N, L, d))
     dx0 = 0.1 * rng.standard_normal((N, L, 3, d))
-    # --- scan path: the two final-pass kernels
+    # --- scan path (final pass: k_scan_lanes when L % 8 == 0, else k_scan) against the oracle
     m.set_path("scan")
-    os.environ.pop("MOIHGP_SCAN_FINAL_WARP", None)
     a = m.filter_smoother_nll(Y, x0=x0, smoother_mode=1)
-    os.environ["MOIHGP_SCAN_FINAL_WARP"] = "1"
-    b = m.filter_smoother_nll(Y, x0=x0, smoother_mode=1)
-    os.environ.pop("MOIHGP_SCAN_FINAL_WARP", None)
+    ao = o.filter_smoother_nll(Y, x0=x0, smoother_mode=1, nthreads=8)
     for k in ("X", "Xs", "nll", "xT"):
-        note("scan lanes vs warp " + k, rel(a[k], b[k]), 1e-11, ctx)
+        note("scan vs oracle " + k, rel(a[k], ao[k]), TOL, ctx)
     # --- many-chains path where instantiated
     try:
         m.set_path("chain")
@@ -63,17 +66,14 @@ for case in range(CASES):
     except RuntimeError:
         pass
     m.set_path("auto")
-    # --- objective: lanes vs warp kernels, one-launch vs general
-    os.environ.pop("MOIHGP_OBJ_WARP", None)
+    # --- objective: general path (k_obj_lanes when L % 8 == 0, else k_obj_scan) against the oracle, one-launch vs general
     m.set_path("scan")                                   # general path (no one-launch kernel)
     la, ga, xa, dxa = m.objective(Y, x0=x0, dx0=dx0, want_state=True)
-    os.environ["MOIHGP_OBJ_WARP"] = "1"
-    lb, gb, xb, dxb = m.objective(Y, x0=x0, dx0=dx0, want_state=True)
-    os.environ.pop("MOIHGP_OBJ_WARP", None)
     m.set_path("auto")
-    note("objective lanes vs warp loss", abs(la - lb) / abs(lb), 1e-11, ctx)
-    note("objective lanes vs warp grad", rel(ga, gb), 1e-10, ctx)
-    note("objective lanes vs warp state", max(rel(xa, xb), rel(dxa, dxb)), 1e-10, ctx)
+    lo, go, xo, dxo = o.objective(Y, x0=x0, dx0=dx0)
+    note("objective vs oracle loss", abs(la - lo) / abs(lo), TOL, ctx)
+    note("objective vs oracle grad", rel(ga, go), TOL, ctx)
+    note("objective vs oracle state", max(rel(xa, xo), rel(dxa, dxo)), TOL, ctx)
     if N == 1:
         lc, gc, xc, dxc = m.objective(Y, x0=x0, dx0=dx0, want_state=True)
         note("objective one-launch vs general loss", abs(lc - la) / abs(la), 1e-11, ctx)

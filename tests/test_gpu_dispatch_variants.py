@@ -5,17 +5,13 @@ oracle at conftest.TOL and, where the same call on default inputs exists, agains
   B. host-buffer calls that span several pipeline slices (double-buffered device buffers, per-slice NaN flags, slices of
      one call on different paths);
   C. the many-chains kernels with fewer sequences per warp (moihgp_cuda_set_chain_seqs_per_warp);
-  D. every k_project_rows configuration and k_project_mma, forced through their environment switches in a child process.
-Every test checks that its variant was reached (profile records, pointer alignment, slice counts, shared-memory fit), so
-that a later dispatch change fails it instead of leaving it passing without testing anything."""
-import os
-import subprocess
-import sys
-
+  D. every k_project_rows configuration and k_project_mma, each on shapes that select it.
+Every test checks that its variant was reached (profile records, pointer alignment, slice counts, the shape rule of the
+projection), so that a later dispatch change fails it instead of leaving it passing without testing anything."""
 import numpy as np
 import pytest
 
-from conftest import ROOT, TOL, literal_smoother_err, rel_err
+from conftest import TOL, literal_smoother_err, rel_err
 
 pytestmark = pytest.mark.gpu
 
@@ -163,29 +159,26 @@ def test_forced_many_chains_path_refuses_offset_operands(cuda_lib, which):
         assert rel_err(r[k], ro[k]) < TOL, k
 
 
-@pytest.mark.parametrize("kernel,p,L,N,T", [("Matern32", 64, 32, 1, 3000), ("Matern52", 16, 8, 2, 1300), ("Matern32", 12, 5, 2, 700)])
-def test_scan_path_with_offset_states(cuda_lib, kernel, p, L, N, T, monkeypatch):
+@pytest.mark.parametrize("kernel,p,L,N,T", [("Matern32", 64, 32, 1, 3000), ("Matern52", 16, 8, 2, 1300), ("Matern32", 12, 5, 2, 700),
+                                            ("Matern32", 64, 30, 1, 3000)])
+def test_scan_path_with_offset_states(cuda_lib, kernel, p, L, N, T):
     """The chunked scan writing X / Xs / xT at an 8-byte offset: the final-pass kernels then store element by element
-    instead of in 16-byte pieces - k_scan_lanes (L a multiple of 8) and the warp-per-chunk k_scan (other L, or forced with
-    MOIHGP_SCAN_FINAL_WARP).  Oracle and aligned call agree."""
+    instead of in 16-byte pieces - k_scan_lanes (L a multiple of 8) and the warp-per-chunk k_scan (other L).  Oracle and
+    aligned call agree."""
     m, o, rng = _model(kernel, p, L, 63 + p)
     Y = _data(rng, p, L, N, T)
     x0 = 0.3 * rng.standard_normal((N, L, m.igp_dim))
     m.set_path("scan")
-    for warp in ((False, True) if L % 8 == 0 else (False,)):
-        if warp:
-            monkeypatch.setenv("MOIHGP_SCAN_FINAL_WARP", "1")
-        for mode in (1, 0):
-            ro = o.filter_smoother_nll(Y, x0=x0, smoother_mode=mode, want_yhat=True, nthreads=8)
-            r, prof = _fused_device(m, Guarded(), Y, x0, mode, ["X", "Xs", "xT"], N, T)
-            assert "k_scan_final" in prof and "k_filter_chain" not in prof
-            a, _ = _fused_device(m, Guarded(), Y, x0, mode, [], N, T)
-            for k in ("X", "Yhat", "xT", "nll"):
-                assert rel_err(r[k], ro[k]) < TOL, (warp, mode, k)
-                assert rel_err(r[k], a[k]) < 1e-13, (warp, mode, k)
-            _states_close(r["Xs"], ro["Xs"], mode, TOL, (warp, mode))
-            _states_close(r["Xs"], a["Xs"], mode, 1e-13, (warp, mode))
-        monkeypatch.delenv("MOIHGP_SCAN_FINAL_WARP", raising=False)
+    for mode in (1, 0):
+        ro = o.filter_smoother_nll(Y, x0=x0, smoother_mode=mode, want_yhat=True, nthreads=8)
+        r, prof = _fused_device(m, Guarded(), Y, x0, mode, ["X", "Xs", "xT"], N, T)
+        assert "k_scan_final" in prof and "k_filter_chain" not in prof
+        a, _ = _fused_device(m, Guarded(), Y, x0, mode, [], N, T)
+        for k in ("X", "Yhat", "xT", "nll"):
+            assert rel_err(r[k], ro[k]) < TOL, (mode, k)
+            assert rel_err(r[k], a[k]) < 1e-13, (mode, k)
+        _states_close(r["Xs"], ro["Xs"], mode, TOL, mode)
+        _states_close(r["Xs"], a["Xs"], mode, 1e-13, mode)
 
 
 def _with_missing(Y, L, rng):
@@ -504,9 +497,9 @@ def test_sequences_per_warp_knob_is_inert_on_full_warp_only_shapes(cuda_lib):
 
 
 # ======================================================================================== D. projection variants
-# k_project_rows<NB> config -> (warps NW, stages NST, boxes per stage NBOX) as project.cu's try_project_rows; nb_all = ceil(p / 16)
-ROWS_CFGS = {1: lambda nb: (16, 2, min(nb, 2)), 2: lambda nb: (16, 3, 1), 3: lambda nb: (12, 2, min(nb, 4)), 5: lambda nb: (8, 2, min(nb, 2)),
-             8: lambda nb: (8, 2, 1)}
+# k_project_rows<NB> configurations in the order of project.cu's try_project_rows -> (warps NW, stages NST, boxes per stage
+# NBOX); nb_all = ceil(p / 16)
+ROWS_CFGS = {1: lambda nb: (16, 2, min(nb, 2)), 2: lambda nb: (16, 3, 1), 5: lambda nb: (8, 2, min(nb, 2)), 8: lambda nb: (8, 2, 1)}
 
 
 def _rows_smem(NB, p, nw, nst, nbox):
@@ -515,75 +508,52 @@ def _rows_smem(NB, p, nw, nst, nbox):
     return 1024 + nw * nst * nbox * 2048 + ((p + 15) & ~15) * (8 * NB + 4) * 8 + 8 * NB * 8 + nw * 386 * 8 + nw * nst * 8
 
 
-# one shape per panel width NB (L <= 8, 16, 32, 64); N > 1 and T not a multiple of 16 (the unit walk wraps into the next
-# sequence inside a CTA's stride).  With the largest of them, config 3 at NB = 8: 1024 + 12*2*3*2048 + 48*68*8 + 512 +
-# 12*3088 + 192 = 212 352 B <= 227 KB = 232 448 B; _rows_smem checks every pair below.
-PROJ_SHAPES = [(1, "Matern52", 40, 6, 3, 203), (2, "Matern32", 24, 12, 2, 301), (4, "Matern52", 48, 20, 2, 150), (8, "Matern32", 48, 40, 2, 130)]
-
-_PROJ_CHILD = r"""
-import sys
-import numpy as np
-sys.path.insert(0, sys.argv[1])
-sys.path.insert(0, sys.argv[1] + "/tests")
-from conftest import TOL, literal_smoother_err, rel_err
-from multioutputihgp_b200 import MOIHGPSequences
-from oracle.binding import OracleMOIHGP
-from oracle.gen_golden import make_data, make_params
-for NB, kernel, p, L, N, T in %r:
-    rng = np.random.default_rng(NB)
-    params = make_params(rng, p, L, kernel)
-    m = MOIHGPSequences(0.1, p, L, kernel, True)
-    o = OracleMOIHGP(0.1, p, L, kernel, True)
-    m.update(params)
-    o.update(params)
-    Y = np.stack([make_data(rng, p, L, T) for _ in range(N)])
-    Yn = Y.copy()
-    Yn[0, 7, :p - L - 2] = np.nan
-    Yn[0, 9, :] = np.nan
-    Yn[N - 1, T - 1, 1] = np.nan
-    x0 = 0.2 * rng.standard_normal((N, L, m.igp_dim))
-    dx0 = 0.1 * rng.standard_normal((N, L, 3, m.igp_dim))
-    m.set_path("scan")
-    for mode in (1, 0):
-        r = m.filter_smoother_nll(Yn, x0=x0, smoother_mode=mode, want_yhat=True)
-        ro = o.filter_smoother_nll(Yn, x0=x0, smoother_mode=mode, want_yhat=True)
-        for k in ("X", "Yhat", "xT"):
-            assert rel_err(r[k], ro[k]) < TOL, (NB, mode, k)
-        if mode == 1:
-            assert rel_err(r["Xs"], ro["Xs"]) < TOL, (NB, mode)
-        else:
-            err, steps = literal_smoother_err(r["Xs"], ro["Xs"])
-            assert err < TOL and steps >= 100, (NB, mode, err, steps)
-        assert np.array_equal(np.isnan(r["nll"]), np.isnan(ro["nll"])) and np.isnan(r["nll"][0]), NB
-        ok = ~np.isnan(ro["nll"])
-        assert rel_err(r["nll"][ok], ro["nll"][ok]) < TOL, NB
-    l, g, xT, dxT = m.objective(Y, x0=x0, dx0=dx0, want_state=True)
-    lo, go, xo, dxo = o.objective(Y, x0=x0, dx0=dx0)
-    assert abs(l - lo) <= TOL * abs(lo) and rel_err(g, go) < TOL, NB
-    assert rel_err(xT, xo) < TOL and rel_err(dxT, dxo) < TOL, NB
-    l, g, xT, dxT = m.objective(Yn, x0=x0, dx0=dx0, want_state=True)
-    lo, go, xo, dxo = o.objective(Yn, x0=x0, dx0=dx0)
-    assert np.isnan(l) and rel_err(xT, xo) < TOL and rel_err(dxT, dxo) < TOL, NB
-    print("projection variant ok", NB, p, L, N, T, flush=True)
-"""
+def _projection_variant(NB, p):
+    """the kernel launch_project picks for a 16-byte aligned Y with even p >= 8 at panel width NB: the first k_project_rows
+    configuration whose shared memory fits into 227 KB, else k_project_mma"""
+    for cfg, shape in ROWS_CFGS.items():
+        if _rows_smem(NB, p, *shape((p + 15) // 16)) <= 227 * 1024:
+            return "rows%d" % cfg
+    return "mma"
 
 
-@pytest.mark.parametrize("variant", ["rows1", "rows2", "rows3", "rows5", "rows8", "mma"])
+# one shape per panel width NB (L <= 8, 16, 32, 64): (NB, kernel, L, N, T), N > 1 and T not a multiple of 16 (the unit walk
+# wraps into the next sequence inside a CTA's stride); per variant the p of each NB that selects it
+PROJ_SHAPES = [(1, "Matern52", 6, 3, 203), (2, "Matern32", 12, 2, 301), (4, "Matern52", 20, 2, 150), (8, "Matern32", 40, 2, 130)]
+PROJ_P = {"rows1": (40, 24, 48, 48), "rows2": (600, 400, 200, 120), "rows5": (1000, 700, 400, 200), "rows8": (1600, 1000, 540, 280),
+          "mma": (1900, 1100, 600, 320)}
+
+
+@pytest.mark.parametrize("variant", list(PROJ_P))
 def test_projection_variant_matches_oracle(cuda_lib, variant):
-    """Each k_project_rows configuration (MOIHGP_PROJECT_ROWS_CFG) and k_project_mma (MOIHGP_PROJECT_ROWS_OFF) on one
-    shape per panel width, through the chunked-scan fused pass (both smoother modes, missing outputs) and the objective,
-    against the oracle.  The switches are read once per process, so each variant runs in a child process of its own.  A
-    forced configuration that does not fit into shared memory would fall back to k_project_mma without a word: the fit of
-    every (configuration, shape) pair is checked here first."""
-    env = {k: v for k, v in os.environ.items() if not k.startswith("MOIHGP_PROJECT_ROWS")}
-    if variant == "mma":
-        env["MOIHGP_PROJECT_ROWS_OFF"] = "1"
-    else:
-        cfg = int(variant[4:])
-        env["MOIHGP_PROJECT_ROWS_CFG"] = str(cfg)
-        for NB, _, p, L, _, _ in PROJ_SHAPES:
-            assert 8 * NB >= L > 8 * NB // 2 and p % 2 == 0 and p >= 8
-            assert _rows_smem(NB, p, *ROWS_CFGS[cfg]((p + 15) // 16)) <= 227 * 1024, (cfg, NB, p)
-    r = subprocess.run([sys.executable, "-c", _PROJ_CHILD % (PROJ_SHAPES,), ROOT], capture_output=True, text=True, env=env, timeout=600)
-    print(r.stdout[-2000:], r.stderr[-4000:])
-    assert r.returncode == 0 and r.stdout.count("projection variant ok") == len(PROJ_SHAPES)
+    """Each k_project_rows configuration and k_project_mma on one shape per panel width that selects it, through the
+    chunked-scan fused pass (both smoother modes, missing outputs) and the objective, against the oracle.  Each shape is
+    first checked to select its variant under the rule of launch_project, so that a change of that rule fails here."""
+    for (NB, kernel, L, N, T), p in zip(PROJ_SHAPES, PROJ_P[variant]):
+        assert 8 * NB >= L > 8 * NB // 2 and p % 2 == 0 and p >= 8
+        assert _projection_variant(NB, p) == variant, (NB, p)
+        m, o, rng = _model(kernel, p, L, NB)
+        Y = _data(rng, p, L, N, T)
+        Yn = Y.copy()
+        Yn[0, 7, :p - L - 2] = np.nan
+        Yn[0, 9, :] = np.nan
+        Yn[N - 1, T - 1, 1] = np.nan
+        x0 = 0.2 * rng.standard_normal((N, L, m.igp_dim))
+        dx0 = 0.1 * rng.standard_normal((N, L, 3, m.igp_dim))
+        what = (variant, NB, p)
+        m.set_path("scan")
+        for mode in (1, 0):
+            r = m.filter_smoother_nll(Yn, x0=x0, smoother_mode=mode, want_yhat=True)
+            ro = o.filter_smoother_nll(Yn, x0=x0, smoother_mode=mode, want_yhat=True, nthreads=8)
+            for k in ("X", "Yhat", "xT"):
+                assert rel_err(r[k], ro[k]) < TOL, (what, mode, k)
+            _states_close(r["Xs"], ro["Xs"], mode, TOL, (what, mode))
+            _nll_close(r["nll"], ro["nll"], TOL, (what, mode))
+            assert np.isnan(r["nll"][0]), what
+        l, g, xT, dxT = m.objective(Y, x0=x0, dx0=dx0, want_state=True)
+        lo, go, xo, dxo = o.objective(Y, x0=x0, dx0=dx0)
+        assert abs(l - lo) <= TOL * abs(lo) and rel_err(g, go) < TOL, what
+        assert rel_err(xT, xo) < TOL and rel_err(dxT, dxo) < TOL, what
+        l, g, xT, dxT = m.objective(Yn, x0=x0, dx0=dx0, want_state=True)
+        lo, go, xo, dxo = o.objective(Yn, x0=x0, dx0=dx0)
+        assert np.isnan(l) and rel_err(xT, xo) < TOL and rel_err(dxT, dxo) < TOL, what

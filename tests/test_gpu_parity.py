@@ -951,53 +951,63 @@ def test_objective_begin_finish_blocks_equal_the_whole_sequence(cuda_lib, kernel
     assert _close(h0[0] + h1[0], lo) and rel_err(h0[2:] + h1[2:], go) < TOL
 
 
+# chunked-scan shapes with several chunks and latent groups: L a multiple of 8 (the thread-per-sub-chunk kernels) and not
+# (the warp-per-chunk kernels)
+SCAN_LANES_SHAPES = [("Matern32", 64, 32, 1, 5000), ("Matern52", 16, 8, 2, 1300), ("Matern32", 32, 16, 2, 256), ("Matern52", 24, 24, 1, 777)]
+OBJ_LANES_SHAPES = [("Matern32", 64, 32, 1, 5000), ("Matern52", 16, 8, 3, 1300), ("Matern32", 32, 16, 2, 256), ("Matern52", 24, 8, 2, 33),
+                    ("Matern32", 48, 24, 1, 4097)]
+WARP_SHAPES = [("Matern32", 64, 30, 1, 5000), ("Matern52", 16, 5, 2, 1300), ("Matern32", 48, 21, 1, 4097), ("Matern52", 24, 11, 2, 33)]
+
+
 @pytest.mark.gpu
-@pytest.mark.parametrize("kernel,p,L,N,T", [("Matern32", 64, 32, 1, 5000), ("Matern52", 16, 8, 2, 1300), ("Matern32", 32, 16, 2, 256),
-                                            ("Matern52", 24, 24, 1, 777)])
-def test_scan_final_kernels_agree(cuda_lib, kernel, p, L, N, T, monkeypatch):
-    """The two final-pass kernels of the chunked-scan path (thread per sub-chunk, warp per chunk) evaluate the same
-    recurrence from the same carries: outputs agree to rounding, in both smoother modes."""
+@pytest.mark.parametrize("kernel,p,L,N,T", SCAN_LANES_SHAPES + WARP_SHAPES)
+def test_scan_final_kernels_agree(cuda_lib, kernel, p, L, N, T):
+    """Both final-pass kernels of the chunked-scan path - thread per sub-chunk (k_scan_lanes, L a multiple of 8) and warp
+    per chunk (k_scan, other L) - against the oracle from a carried-in state, in both smoother modes."""
     from multioutputihgp_b200 import MOIHGPSequences
+    from oracle.binding import OracleMOIHGP
     from oracle.gen_golden import make_data, make_params
+    assert (L % 8 == 0) == ((kernel, p, L, N, T) in SCAN_LANES_SHAPES)
     rng = np.random.default_rng(T)
+    params = make_params(rng, p, L, kernel)
     m = MOIHGPSequences(0.1, p, L, kernel, True)
-    m.update(make_params(rng, p, L, kernel))
+    o = OracleMOIHGP(0.1, p, L, kernel, True)
+    m.update(params)
+    o.update(params)
     m.set_path("scan")
     Y = np.stack([make_data(rng, p, L, T) for _ in range(N)])
     x0 = 0.3 * rng.standard_normal((N, L, m.igp_dim))
     for mode in (1, 0):
-        monkeypatch.delenv("MOIHGP_SCAN_FINAL_WARP", raising=False)
-        a = m.filter_smoother_nll(Y, x0=x0, smoother_mode=mode)
-        monkeypatch.setenv("MOIHGP_SCAN_FINAL_WARP", "1")
-        b = m.filter_smoother_nll(Y, x0=x0, smoother_mode=mode)
-        monkeypatch.delenv("MOIHGP_SCAN_FINAL_WARP", raising=False)
+        r = m.filter_smoother_nll(Y, x0=x0, smoother_mode=mode)
+        ro = o.filter_smoother_nll(Y, x0=x0, smoother_mode=mode, nthreads=8)
         for k in ("X", "nll", "xT"):
-            assert rel_err(a[k], b[k]) < 1e-12, (k, mode)
-        assert (rel_err(a["Xs"], b["Xs"]) if mode == 1 else literal_smoother_err(a["Xs"], b["Xs"])[0]) < 1e-11, mode
+            assert rel_err(r[k], ro[k]) < TOL, (k, mode)
+        _assert_smoothed(r, ro, mode, mode)
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("kernel,p,L,N,T", [("Matern32", 64, 32, 1, 5000), ("Matern52", 16, 8, 3, 1300), ("Matern32", 32, 16, 2, 256),
-                                            ("Matern52", 24, 8, 2, 33), ("Matern32", 48, 24, 1, 4097)])
-def test_objective_kernels_agree(cuda_lib, kernel, p, L, N, T, monkeypatch):
-    """The two implementations of the objective's scan (thread per sub-chunk, warp per chunk) give the same loss,
-    gradient and final state to rounding."""
+@pytest.mark.parametrize("kernel,p,L,N,T", OBJ_LANES_SHAPES + WARP_SHAPES)
+def test_objective_kernels_agree(cuda_lib, kernel, p, L, N, T):
+    """Both implementations of the objective's scan - thread per sub-chunk (k_obj_lanes, L a multiple of 8) and warp per
+    chunk (k_obj_scan, other L) - against the oracle: loss, gradient and final state from a carried-in state."""
     from multioutputihgp_b200 import MOIHGPSequences
+    from oracle.binding import OracleMOIHGP
     from oracle.gen_golden import make_data, make_params
+    assert (L % 8 == 0) == ((kernel, p, L, N, T) in OBJ_LANES_SHAPES)
     rng = np.random.default_rng(T + L)
+    params = make_params(rng, p, L, kernel)
     m = MOIHGPSequences(0.1, p, L, kernel, True)
-    m.update(make_params(rng, p, L, kernel))
+    o = OracleMOIHGP(0.1, p, L, kernel, True)
+    m.update(params)
+    o.update(params)
     Y = np.stack([make_data(rng, p, L, T) for _ in range(N)])
     x0 = 0.3 * rng.standard_normal((N, L, m.igp_dim))
     dx0 = 0.1 * rng.standard_normal((N, L, 3, m.igp_dim))
-    monkeypatch.delenv("MOIHGP_OBJ_WARP", raising=False)
-    la, ga, xa, dxa = m.objective(Y, x0=x0, dx0=dx0, want_state=True)
-    monkeypatch.setenv("MOIHGP_OBJ_WARP", "1")
-    lb, gb, xb, dxb = m.objective(Y, x0=x0, dx0=dx0, want_state=True)
-    monkeypatch.delenv("MOIHGP_OBJ_WARP", raising=False)
-    assert abs(la - lb) <= 1e-12 * abs(lb)
-    assert rel_err(ga, gb) < 1e-11
-    assert rel_err(xa, xb) < 1e-12 and rel_err(dxa, dxb) < 1e-11
+    loss, grad, xT, dxT = m.objective(Y, x0=x0, dx0=dx0, want_state=True)
+    lo, go, xo, dxo = o.objective(Y, x0=x0, dx0=dx0)
+    assert _close(loss, lo)
+    assert rel_err(grad, go) < TOL
+    assert rel_err(xT, xo) < TOL and rel_err(dxT, dxo) < TOL
 
 
 @pytest.mark.gpu
@@ -1229,10 +1239,10 @@ def test_function_values_only_output(cuda_lib, kernel, p, L, N, T, path):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("p,L", [(256, 64), (128, 33), (100, 21), (512, 16)])
-def test_newton_schulz_polar_factor_agrees_with_jacobi(cuda_lib, p, L, monkeypatch):
+def test_device_polar_factor_matches_svd_and_falls_back_on_rank_deficiency(cuda_lib, p, L):
     """update() on the device: k_polar_ns (Newton-Schulz, the fast way for a block that is nearly orthonormal, as inside a
-    line search) against k_polar (one-sided Jacobi) on nearly orthonormal, generic, badly scaled and ill-conditioned
-    blocks; a rank-deficient block falls back to Jacobi."""
+    line search) against the SVD polar factor on nearly orthonormal, generic, badly scaled and ill-conditioned blocks; a
+    rank-deficient block falls back to k_polar (one-sided Jacobi), whose answer must still be a polar factor."""
     from multioutputihgp_b200 import MOIHGPSequences
     from oracle.gen_golden import make_params
     rng = np.random.default_rng(p + L)
@@ -1249,26 +1259,22 @@ def test_newton_schulz_polar_factor_agrees_with_jacobi(cuda_lib, p, L, monkeypat
     for name, B in blocks.items():
         params = base.copy()
         params[:p * L] = B.ravel()
-        monkeypatch.delenv("MOIHGP_POLAR_JACOBI", raising=False)
         m.update(params)
-        U_ns = m.U.copy()
-        monkeypatch.setenv("MOIHGP_POLAR_JACOBI", "1")
-        m.update(params)
-        U_j = m.U.copy()
-        monkeypatch.delenv("MOIHGP_POLAR_JACOBI", raising=False)
+        U = m.U.copy()
         Wm, _, Vt = np.linalg.svd(B, full_matrices=False)
         tol = 1e-9 if name != "ill-conditioned" else 1e-7           # the polar factor's conditioning is 1 / sigma_min
-        assert rel_err(U_ns, Wm @ Vt) < tol, name
-        assert rel_err(U_ns, U_j) < tol, name
-        assert np.max(np.abs(U_ns.T @ U_ns - np.eye(L))) < 1e-12, name
-    # rank-deficient: no unique polar factor; the iteration gives up and the Jacobi kernel's answer is the result
+        assert rel_err(U, Wm @ Vt) < tol, name
+        assert np.max(np.abs(U.T @ U - np.eye(L))) < 1e-12, name
+    # rank-deficient: no unique polar factor; the iteration gives up and the Jacobi kernel's answer is the result.  Any
+    # polar factor B = U H has orthonormal columns, H = U'B symmetric positive semi-definite, and U U'B = B.
     B = rng.standard_normal((p, L))
     B[:, -1] = B[:, 0]
     params = base.copy()
     params[:p * L] = B.ravel()
     m.update(params)
-    U_a = m.U.copy()
-    monkeypatch.setenv("MOIHGP_POLAR_JACOBI", "1")
-    m.update(params)
-    monkeypatch.delenv("MOIHGP_POLAR_JACOBI", raising=False)
-    assert np.array_equal(U_a, m.U)
+    U = m.U.copy()
+    H = U.T @ B
+    assert np.max(np.abs(U.T @ U - np.eye(L))) < 1e-12
+    assert rel_err(H, H.T) < 1e-12
+    assert np.min(np.linalg.eigvalsh(0.5 * (H + H.T))) > -1e-12 * np.max(np.abs(H))
+    assert rel_err(U @ H, B) < 1e-9
