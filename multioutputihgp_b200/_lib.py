@@ -13,7 +13,7 @@ CSRC = os.path.join(_HERE, "csrc")
 c_double_p = ctypes.POINTER(ctypes.c_double)
 c_int_p = ctypes.POINTER(ctypes.c_int)
 
-_SOURCES = ["ls_project.cuh", "polar.cu", "chain_kernels.cuh", "chain_inst_16x8.cu", "chain_inst_8x4.cu", "chain_inst_8x2.cu", "chain_inst_8x8.cu", "chain_inst_16x2.cu", "chain_inst_16x4.cu", "chain_inst_16x16.cu", "chain_inst_32x4.cu", "chain_inst_32x8.cu", "chain_inst_32x16.cu", "chain_inst_4x2.cu", "chain_inst_4x4.cu", "chain_inst_32x2.cu", "chain_inst_4x1.cu", "chain_inst_8x1.cu", "chain_inst_16x1.cu", "chain_inst_32x1.cu", "setup.cu", "sample.cu", "project.cu", "scan.cu", "objective.cu", "chain.cu", "step.cu", "capi.cu", "moihgp_device.cuh", "tma.cuh", "small_mat.cuh", "launch.h", "Makefile"]
+_SOURCES = ["ls_project.cuh", "polar.cu", "chain_kernels.cuh", "chain_inst_16x8.cu", "chain_inst_8x4.cu", "chain_inst_8x2.cu", "chain_inst_8x8.cu", "chain_inst_16x2.cu", "chain_inst_16x4.cu", "chain_inst_16x16.cu", "chain_inst_32x4.cu", "chain_inst_32x8.cu", "chain_inst_32x16.cu", "chain_inst_4x2.cu", "chain_inst_4x4.cu", "chain_inst_32x2.cu", "chain_inst_4x1.cu", "chain_inst_8x1.cu", "chain_inst_16x1.cu", "chain_inst_32x1.cu", "setup.cu", "sample.cu", "project.cu", "scan.cu", "objective.cu", "chain.cu", "step.cu", "capi.cu", "moihgp_device.cuh", "ptx.cuh", "small_mat.cuh", "launch.h", "Makefile"]
 
 
 def build(force=False, verbose=False):

@@ -20,6 +20,7 @@
 #include <vector>
 #include "../../include/moihgp_b200.h"
 #include "launch.h"
+#include "small_mat.cuh"
 
 using namespace moihgp;
 
@@ -307,7 +308,6 @@ int step_call(moihgp_handle* h, const double* x, const double* y, const double* 
     a.consts = h->d_consts; a.U = h->d_U; a.S = h->d_S; a.sigma = h->sigma; a.p = h->p; a.L = h->L; a.dim = h->dim; a.threading = h->threading;
     a.x = h->d_stage + s.x; a.y = y ? h->d_stage + s.y : nullptr; a.dx = dx ? h->d_stage + s.dx : nullptr;
     a.xnew = h->d_stage + s.xnew; a.yhat = yhat ? h->d_stage + s.yhat : nullptr; a.dxnew = (dx && dxnew) ? h->d_stage + s.dxnew : nullptr;
-    a.scratch = nullptr;
     CK(launch_step(a, h->stream));
     h->launches += 1;
     CK(cudaMemcpyAsync(h->h_stage + s.xnew, h->d_stage + s.xnew, sizeof(double) * (s.loss - s.xnew), cudaMemcpyDeviceToHost, h->stream));
@@ -329,7 +329,7 @@ int lik_call(moihgp_handle* h, const double* x, const double* y, const double* d
     LikArgs a;
     a.consts = h->d_consts; a.U = h->d_U; a.S = h->d_S; a.sigma = h->sigma; a.p = h->p; a.L = h->L; a.dim = h->dim; a.threading = h->threading;
     a.x = h->d_stage + s.x; a.y = h->d_stage + s.y; a.dx = dx ? h->d_stage + s.dx : nullptr;
-    a.loss = h->d_stage + s.loss; a.grad = (dx && grad) ? h->d_stage + s.grad : nullptr; a.scratch = nullptr;
+    a.loss = h->d_stage + s.loss; a.grad = (dx && grad) ? h->d_stage + s.grad : nullptr;
     CK(launch_lik(a, h->stream));
     h->launches += 1;
     const size_t nout = 2 + ((dx && grad) ? (size_t)h->num_param : 0);
@@ -547,40 +547,10 @@ long long moihgp_cuda_latent_consts(moihgp_handle* h, size_t l, double* out, siz
 int moihgp_cuda_block_transition(moihgp_handle* h, size_t n, double* out) {
     if (!h || !out) return -2;
     if (mirror(h)) return -1;
-    const int d = h->dim, dd = d * d;
-    auto mul = [&](const double* A, const double* B, double* C) {            // C = A B   (d x d, row-major, C distinct)
-        for (int i = 0; i < d; ++i) for (int j = 0; j < d; ++j) {
-            double s = 0.0;
-            for (int q = 0; q < d; ++q) s += A[i * d + q] * B[q * d + j];
-            C[i * d + j] = s;
-        }
-    };
-    for (int l = 0; l < h->L; ++l) {
-        const LatentConsts& c = h->consts[l];
-        double P[9] = {0}, E[3][9] = {{0}}, Pb[9], Eb[3][9], t1[9], t2[9];
-        for (int i = 0; i < d; ++i) P[i * d + i] = 1.0;
-        for (int k = 0; k < 3; ++k) for (int i = 0; i < d; ++i) for (int j = 0; j < d; ++j) Eb[k][i * d + j] = c.dAKHA[k][i * 3 + j];
-        // bits of n from the least significant: (Pb, Eb) = T(2^j) by doubling, (P, E) = T(bits seen so far);
-        // appending a span b after a span a:  P <- Pb P,  E_k <- Pb E_k + Eb_k P
-        for (int j = 0; (n >> j) != 0 && j < NPOW; ++j) {
-            for (int i = 0; i < d; ++i) for (int q = 0; q < d; ++q) Pb[i * d + q] = c.powM[j][i * 3 + q];
-            if ((n >> j) & 1) {
-                for (int k = 0; k < 3; ++k) {
-                    mul(Pb, E[k], t1);
-                    mul(Eb[k], P, t2);
-                    for (int i = 0; i < dd; ++i) E[k][i] = t1[i] + t2[i];
-                }
-                mul(Pb, P, t1);
-                for (int i = 0; i < dd; ++i) P[i] = t1[i];
-            }
-            for (int k = 0; k < 3; ++k) {                                   // E(2b) = E(b) M^b + M^b E(b)
-                mul(Eb[k], Pb, t1);
-                mul(Pb, Eb[k], t2);
-                for (int i = 0; i < dd; ++i) Eb[k][i] = t1[i] + t2[i];
-            }
-        }
-        double* o = out + (size_t)l * 4 * dd;
-        for (int i = 0; i < dd; ++i) { o[i] = P[i]; for (int k = 0; k < 3; ++k) o[(1 + k) * dd + i] = E[k][i]; }
+    for (int l = 0; l < h->L; ++l) {                                      // out[l] = [P | E_0 | E_1 | E_2]
+        double* o = out + (size_t)l * 4 * h->dim * h->dim;
+        if (h->dim == 2) block_transition<2>(h->consts[l], n, o, reinterpret_cast<double(*)[4]>(o + 4));
+        else block_transition<3>(h->consts[l], n, o, reinterpret_cast<double(*)[9]>(o + 9));
     }
     return 0;
 }
@@ -656,12 +626,9 @@ static int fused_pass(moihgp_handle* h, const double* Y, size_t N, size_t T, con
         int* nanf;
         if (ws_get(h, "nanf", 4, &nanf)) return -1;
         CK(cudaMemsetAsync(nanf, 0, 2 * sizeof(int), h->stream));
-        double Ssum = 0.0;                         // no mirror(h): nothing here waits for K-setup (asynchronous, capturable)
-        for (int l = 0; l < L; ++l) Ssum += h->S[l];
-        const double m_n = std::max((double)(h->p - L), 0.0);
-        ChainArgs c;
+        ChainArgs c;                               // no mirror(h): nothing here waits for K-setup (asynchronous, capturable)
         c.Y = Y; c.U_host = h->U.data(); c.S_host = h->S.data(); c.consts = h->d_consts; c.sigma = h->sigma;
-        c.nll_const = 0.5 * std::log(Ssum) + 0.5 * m_n * std::log(h->sigma);
+        c.nll_const = nll_step_const(h->S.data(), h->p, L, h->sigma);
         c.N = (long long)N; c.T = (long long)T; c.mode = mode < 0 ? 1 : mode; c.x0 = x0; c.X = X; c.Xs = Xs; c.nll = nll; c.xT = xT; c.mk = mk; c.nan_flag = nanf; c.seqs_per_warp = h->chain_spw;
         CK(launch_chain(h->p, L, D, c, h->stream));
         h->launches += Xs ? 2 : 1;
@@ -756,21 +723,9 @@ int moihgp_cuda_fsn_carry_dev(moihgp_handle* h, int direction, int mode, const d
 int moihgp_cuda_smoother_power(moihgp_handle* h, int mode, size_t n, double* out) {
     if (!h || !out || mode < 0 || mode > 1) return -2;
     if (mirror(h)) return -1;
-    const int d = h->dim, dd = d * d;
     for (int l = 0; l < h->L; ++l) {
-        const LatentConsts& c = h->consts[l];
-        double P[9] = {0}, t1[9];
-        for (int i = 0; i < d; ++i) P[i * d + i] = 1.0;
-        for (int j = 0; (n >> j) != 0 && j < NPOW; ++j) {
-            if (!((n >> j) & 1)) continue;
-            for (int i = 0; i < d; ++i) for (int q = 0; q < d; ++q) {
-                double s_ = 0.0;
-                for (int r = 0; r < d; ++r) s_ += c.powG[mode][j][i * 3 + r] * P[r * d + q];
-                t1[i * d + q] = s_;
-            }
-            for (int i = 0; i < dd; ++i) P[i] = t1[i];
-        }
-        for (int i = 0; i < dd; ++i) out[(size_t)l * dd + i] = P[i];
+        if (h->dim == 2) mat_pow<2>(h->consts[l].powG[mode], n, out + (size_t)l * 4);
+        else mat_pow<3>(h->consts[l].powG[mode], n, out + (size_t)l * 9);
     }
     return 0;
 }
@@ -1247,7 +1202,7 @@ int moihgp_cuda_online_push(moihgp_handle* h, const double* y, const double* ma_
         // the window slid: the carried state advances with the NEW front element (Q12), step v2 (moihgp_online.h:89)
         StepArgs a;
         a.consts = h->d_consts; a.U = h->d_U; a.S = h->d_S; a.sigma = h->sigma; a.p = h->p; a.L = h->L; a.dim = h->dim; a.threading = h->threading;
-        a.x = o.d_x; a.y = o.d_front; a.dx = o.d_dx; a.xnew = o.d_x2; a.yhat = nullptr; a.dxnew = o.d_dx2; a.scratch = nullptr;
+        a.x = o.d_x; a.y = o.d_front; a.dx = o.d_dx; a.xnew = o.d_x2; a.yhat = nullptr; a.dxnew = o.d_dx2;
         CK(launch_step(a, h->stream));
         h->launches += 1;
         CK(cudaMemcpyAsync(o.d_x, o.d_x2, sizeof(double) * L * D, cudaMemcpyDeviceToDevice, h->stream));

@@ -31,7 +31,7 @@
 #include <math.h>
 #include <cmath>
 #include "moihgp_device.cuh"
-#include "tma.cuh"
+#include "ptx.cuh"
 #include "launch.h"
 #include "ls_project.cuh"
 
@@ -53,23 +53,6 @@ struct ProjConsts {          // passed by value: lives in the constant bank
     double U[P][L];
     double rs[L];            // S^-1/2
 };
-
-__device__ __forceinline__ void cp_async16(void* smem, const void* gmem) {
-    const unsigned s = (unsigned)__cvta_generic_to_shared(smem);
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;\n" ::"r"(s), "l"(gmem) : "memory");
-}
-__device__ __forceinline__ void cp_async8(void* smem, const void* gmem) {
-    const unsigned s = (unsigned)__cvta_generic_to_shared(smem);
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 8;\n" ::"r"(s), "l"(gmem) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;\n" ::: "memory"); }
-template <int N> __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;\n" ::"n"(N) : "memory"); }
-
-// D(8x8) += A(8x4) * B(4x8), fp64 tensor pipe.  Fragments: A[lane/4][lane%4], B[lane%4][lane/4],
-// C[lane/4][2*(lane%4) + {0,1}].
-__device__ __forceinline__ void dmma884(double& c0, double& c1, double a, double b) {
-    asm("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};\n" : "+d"(c0), "+d"(c1) : "d"(a), "d"(b));
-}
 
 // one latent's state in the staging tile: a single 16-byte access when D = 2
 template <int D> __device__ __forceinline__ void store_state(double* p, const double (&v)[D]) {

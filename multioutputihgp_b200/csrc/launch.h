@@ -25,6 +25,15 @@ struct Marker {
 };
 inline void mark(Marker* m, const char* name) { if (m) m->mark(name); }
 
+// Chunks per CTA / warp of a chunked pass over `units` independent units: about `target` CTAs / warps, enough to fill
+// the machine several times over, with as few chunk prologues as that allows.
+inline long long chunks_per_group(long long units, long long chunks, long long target) {
+    long long groups = (target + units - 1) / units;
+    if (groups < 1) groups = 1;
+    if (groups > chunks) groups = chunks;
+    return (chunks + groups - 1) / groups;
+}
+
 // setup.cu
 cudaError_t launch_setup(int dim, const double* d_igp_params, double dt, int L, LatentConsts* d_out, cudaStream_t stream);
 
@@ -187,7 +196,6 @@ struct StepArgs {
     int p, L, dim, threading;
     const double *x, *y, *dx;     // device staging: [L][D], [p] (null = predict only), [L][3][D] (may be null)
     double *xnew, *yhat, *dxnew;  // outputs (yhat/dxnew may be null)
-    double* scratch;              // >= L*L + 3*L doubles
 };
 cudaError_t launch_step(const StepArgs& a, cudaStream_t st);
 struct LikArgs {
@@ -198,7 +206,6 @@ struct LikArgs {
     const double *x, *y, *dx;     // dx null => lik2 (no gradient)
     double* loss;                 // [1]
     double* grad;                 // [num_param] or null
-    double* scratch;
 };
 cudaError_t launch_lik(const LikArgs& a, cudaStream_t st);
 cudaError_t launch_extract_values(const double* X, double* F, long long n, int d, cudaStream_t st);

@@ -8,6 +8,7 @@
 #pragma once
 #include <cstddef>
 #include <cstdint>
+#include <math.h>
 
 namespace moihgp {
 
@@ -56,5 +57,13 @@ struct MixView {
     double sigma;
     int p, L;
 };
+
+// The NLL's constant per time step, 1/2 log(sum_l S_l) + 1/2 m_n log(sigma) with m_n = max(p - L, 0)   moihgp.h:502-503
+__host__ __device__ inline double nll_step_const(const double* S, int p, int L, double sigma) {
+    const double m_n = fmax((double)(p - L), 0.0);
+    double Ssum = 0.0;
+    for (int l = 0; l < L; ++l) Ssum += S[l];
+    return 0.5 * log(Ssum) + 0.5 * m_n * log(sigma);
+}
 
 }  // namespace moihgp

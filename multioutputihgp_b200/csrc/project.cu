@@ -29,7 +29,7 @@
 #include "moihgp_device.cuh"
 #include "launch.h"
 #include "ls_project.cuh"
-#include "tma.cuh"
+#include "ptx.cuh"
 
 namespace moihgp {
 
@@ -159,17 +159,6 @@ __global__ void __launch_bounds__(PT) k_project(const double* __restrict__ Y, co
 }
 
 // -------------------------------------------------------------------------------------------------
-__device__ __forceinline__ void dmma884(double& c0, double& c1, double a, double b) {
-    asm("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};\n" : "+d"(c0), "+d"(c1) : "d"(a), "d"(b));
-}
-// 16-byte cp.async with zero fill: `bytes` (0, 8 or 16) are read from gmem, the rest of the 16 bytes are zeros
-__device__ __forceinline__ void cp_async16_zfill(void* smem, const void* gmem, int bytes) {
-    const unsigned s = (unsigned)__cvta_generic_to_shared(smem);
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;\n" ::"r"(s), "l"(gmem), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;\n" ::: "memory"); }
-template <int N> __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;\n" ::"n"(N) : "memory"); }
-
 constexpr int MW = 8;                 // warps per CTA, 16 rows each
 constexpr int MT = 32 * MW;           // threads
 constexpr int KP = 16;                // columns of Y per K panel (4 k blocks)

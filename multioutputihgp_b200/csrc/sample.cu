@@ -19,6 +19,7 @@
 #include <cuda_runtime.h>
 #include <curand_philox4x32_x.h>
 #include "launch.h"
+#include "small_mat.cuh"
 
 namespace moihgp {
 
@@ -135,23 +136,7 @@ __global__ void __launch_bounds__(kThreads) k_sample_carry(const SampleArgs a, l
     if (chain >= chains) return;
     const LatentConsts& k = a.consts[chain % a.L];
     double P[D * D];
-#pragma unroll
-    for (int i = 0; i < D * D; ++i) P[i] = (i / D == i % D) ? 1.0 : 0.0;
-    for (int j = 0; (chunk_len >> j) != 0 && j < NPOW; ++j) {   // P = G^chunk_len
-        if (!((chunk_len >> j) & 1)) continue;
-        double t[D * D];
-#pragma unroll
-        for (int i = 0; i < D; ++i)
-#pragma unroll
-            for (int m = 0; m < D; ++m) {
-                double s = 0.0;
-#pragma unroll
-                for (int q = 0; q < D; ++q) s += k.powG[1][j][i * 3 + q] * P[q * D + m];
-                t[i * D + m] = s;
-            }
-#pragma unroll
-        for (int i = 0; i < D * D; ++i) P[i] = t[i];
-    }
+    mat_pow<D>(k.powG[1], chunk_len, P);                         // P = G^chunk_len
     double* cv = a.carry + (size_t)chain * D;
     const size_t cs = (size_t)chains * D;                        // one chunk of the carry array
     double e[D];
