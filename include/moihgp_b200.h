@@ -150,6 +150,21 @@ int moihgp_cuda_filter_smoother_nll_values(moihgp_handle* h, const double* Y, si
 int moihgp_cuda_filter_smoother_nll_dev(moihgp_handle* h, const double* Y, size_t N, size_t T, const double* x0,
                                         int smoother_mode, double* X, double* Xs, double* Yhat, double* nll, double* xT);
 
+/* Per-step NLL terms of the filter pass (no smoother, no states written):
+ *   nll_steps[n][t] = MOIHGP::negLogLikelihood(x_{t-1}, y_t)  (moihgp.h:614-688), the term the fused pass sums into nll[n]:
+ *                     1/2 ||y_t - U U' y_t|| / sigma + sum_l 1/2 v_{l,t}^2 / S_l + the per-step constant + 1/2 sum_l log S_l
+ * A row with a missing output (NaN) gives a NaN term, as in the reference, and the least-squares projection carries the
+ * filter on (moihgp_cuda_nan_status); the other terms stay finite.  Summed over t the terms give nll[n] up to rounding.
+ * nll_steps [N][T] is required; nll [N] and xT [N][L][d] may be NULL; x0 as for the fused pass.  moihgp_cuda_set_path 1 / 2
+ * forces the chunked scan / the many-chains kernels as for the fused pass (the many-chains kernels then take a full warp of
+ * sequences whatever moihgp_cuda_set_chain_seqs_per_warp says).
+ *   _dev : DEVICE buffers, asynchronous on the handle's stream (capturable into a CUDA graph like the fused pass).
+ * The host-buffer twin copies in, calls the _dev entry point and copies out. */
+int moihgp_cuda_nll_steps_dev(moihgp_handle* h, const double* Y, size_t N, size_t T, const double* x0, double* nll_steps,
+                              double* nll, double* xT);
+int moihgp_cuda_nll_steps(moihgp_handle* h, const double* Y, size_t N, size_t T, const double* x0, double* nll_steps,
+                          double* nll, double* xT);
+
 /* IHGP::backwardSmoother(X, Xprev, P, G) (ihgp.h:103-114) for every latent, over CALLER-SUPPLIED filtered states
  * X[N][T][L][d] (not necessarily produced by this library): Xs[N][T][L][d] per `smoother_mode` (0 = the reference's
  * recursion as written, 1 = RTS).  G and P of each latent come from moihgp_cuda_smoother_consts.  HOST / DEVICE buffers. */

@@ -346,6 +346,13 @@ public:
         detail::check(_h, moihgp_cuda_filter_smoother_nll(_h, Y, 1, T, &_xb[0], smoother_mode, X, Xs, Yhat, nll, &_xb[nx()]), "MOIHGP::predict");
         unpack_x(&_xb[nx()], x);
     }
+    // negLogLikelihood(x, y) of every step of the same filter loop (moihgp.h:614-688) over packed Y[T][p] into nll_steps[T]
+    // (NaN for a row with a missing output); x is the carried-in state and receives the final state.
+    void nllSteps(const double* Y, size_t T, State& x, double* nll_steps) {
+        pack_x(x, &_xb[0]);
+        detail::check(_h, moihgp_cuda_nll_steps(_h, Y, 1, T, &_xb[0], nll_steps, NULL, &_xb[nx()]), "MOIHGP::nllSteps");
+        unpack_x(&_xb[nx()], x);
+    }
 
     // Keep the data set resident on the device across objective evaluations (the optimiser calls the functor tens of times
     // on the same observations); the caller re-binds after changing them.  Y = NULL releases it.

@@ -207,6 +207,33 @@ class MOIHGPSequences(object):
         self._check(self._lib.moihgp_cuda_filter_smoother_nll_dev(self._h, _ptr(Y), N, T, _ptr(x0), smoother_mode, _ptr(X), _ptr(Xs),
                                                                   _ptr(Yhat), _ptr(nll), _ptr(xT)))
 
+    # ---- per-step NLL terms (moihgp_cuda_nll_steps*) -----------------------------------------------------------
+    def nll_steps(self, Y, x0=None):
+        """Y: [N,T,p] (or [T,p]) NumPy array -> dict of NumPy arrays: nll_steps [N,T], the term MOIHGP::negLogLikelihood(x_{t-1},
+        y_t) of every step (NaN for a row with a missing output), nll [N] (their sum, as filter_smoother_nll returns it) and xT
+        [N,L,d].  Filter only: no smoother, no states."""
+        Y = _np(Y)
+        if Y.ndim == 2:
+            Y = Y[None]
+        N, T, p = Y.shape
+        assert p == self.num_output
+        L, d = self.num_latent, self.igp_dim
+        x0 = None if x0 is None else _np(x0).reshape(N, L, d)
+        steps, nll, xT = np.empty((N, T)), np.empty(N), np.empty((N, L, d))
+        self._check(self._lib.moihgp_cuda_nll_steps(self._h, _ptr(Y), N, T, _ptr(x0), _ptr(steps), _ptr(nll), _ptr(xT)))
+        return {"nll_steps": steps, "nll": nll, "xT": xT}
+
+    def nll_steps_device(self, Y, nll_steps, x0=None, nll=None, xT=None):
+        """Device-resident variant: torch CUDA float64 tensors, outputs pre-allocated by the caller (nll_steps [N,T] required,
+        nll [N] and xT [N,L,d] may be None); runs asynchronously on torch's current stream."""
+        import torch
+        assert Y.is_cuda and Y.dtype == torch.float64 and Y.is_contiguous() and Y.dim() == 3
+        N, T, _ = Y.shape
+        for o in (nll_steps, x0, nll, xT):
+            assert o is None or (o.is_cuda and o.dtype == torch.float64 and o.is_contiguous())
+        self.set_stream(_torch_stream(Y.device))
+        self._check(self._lib.moihgp_cuda_nll_steps_dev(self._h, _ptr(Y), N, T, _ptr(x0), _ptr(nll_steps), _ptr(nll), _ptr(xT)))
+
     # ---- objective: NLL + gradient ----------------------------------------------------------------
     def objective(self, Y, x0=None, dx0=None, want_state=False):
         """sum over sequences and time of negLogLikelihood(x, y, dx, grad) with step v2 advancing the state

@@ -575,8 +575,8 @@ int moihgp_cuda_smoother_consts(moihgp_handle* h, size_t l, int mode, double* G,
 
 // The chunked-scan pass (project.cu + scan.cu) over Y [N][T][p] with N = a.N, T = a.T: a.phase 0 is the whole pass, 1 / 2 / 3
 // one block of a sequence sharded in time (ScanArgs).  The caller sets a's inputs, outputs, phase and marker; this takes the
-// workspace, projects Y (phases 0 and 1), scans, and reduces the NLL into nll (phases 0 and 3, when nll is set).  On return
-// a.u holds the projected observations.
+// workspace, projects Y (phases 0 and 1), scans, and reduces the NLL into nll (phases 0 and 3, when nll is set) and, when
+// a.nll_steps is set (phase 0), into per-step terms.  On return a.u holds the projected observations.
 static int scan_pass(moihgp_handle* h, const double* Y, int mode, double* nll, ScanArgs& a) {
     const size_t N = (size_t)a.N, T = (size_t)a.T, L = h->L, D = h->dim, nC = scan_chunks(a.T), nSB = scan_superblocks(a.T);
     ProjectWs pw;
@@ -586,11 +586,13 @@ static int scan_pass(moihgp_handle* h, const double* Y, int mode, double* nll, S
         ws_get(h, "Bx", L * 2 * 9, &Bx) || ws_get(h, "Wsum", scan_weights_doubles((int)L), &Wsum) || ws_get(h, "sbe", N * L * nSB * D, &sbe) ||
         ws_get(h, "sbi", N * L * nSB * D, &sbi) || ws_get(h, "vsq", nC * N * L, &vsq))
         return -1;
+    if (a.nll_steps && ws_get(h, "vstep", N * L * T, &a.vstep)) return -1;
     if (a.phase <= 1) {
         // the projection residuals rho feed only the NLL; a block keeps them from phase 1 for its phase 3
         CK(cudaMemsetAsync(pw.nanf, 0, 2 * sizeof(int), h->stream));
-        CK(launch_project(Y, h->d_U, h->d_S, h->p, (int)L, a.N, a.T, pw.u, nullptr, nullptr, (nll || a.phase == 1) ? pw.rho : nullptr, pw.nanf,
-                          pw.nanrows, (long long)pw.nan_cap, h->stream));
+        // per-step terms: the projection leaves each row's residual norm in nll_steps, k_nll_steps completes them in place
+        CK(launch_project(Y, h->d_U, h->d_S, h->p, (int)L, a.N, a.T, pw.u, nullptr, nullptr, (nll || a.phase == 1 || a.nll_steps) ? pw.rho : nullptr,
+                          a.nll_steps, pw.nanf, pw.nanrows, (long long)pw.nan_cap, h->stream));
         h->launches += 2;
         mark(a.mk, "k_project");
     }
@@ -603,12 +605,18 @@ static int scan_pass(moihgp_handle* h, const double* Y, int mode, double* nll, S
         h->launches += 2;
         mark(a.mk, "k_nll_reduce");
     }
+    if (a.phase == 0 && a.nll_steps) {
+        CK(launch_nll_steps(a.vstep, h->d_consts, h->d_S, h->sigma, h->p, (int)L, a.N, a.T, a.nll_steps, h->stream));
+        h->launches += 1;
+        mark(a.mk, "k_nll_steps");
+    }
     return 0;
 }
 
-// strict_chain: a forced many-chains path that cannot serve the pass fails (the entry point) or takes the scan (the sampler)
+// strict_chain: a forced many-chains path that cannot serve the pass fails (the entry point) or takes the scan (the sampler).
+// nll_steps ([N][T] per-step NLL terms) is the filter-only pass of moihgp_cuda_nll_steps_dev: mode -1, X, Xs and Yhat null.
 static int fused_pass(moihgp_handle* h, const double* Y, size_t N, size_t T, const double* x0, int mode, double* X, double* Xs,
-                      double* Yhat, double* nll, double* xT, bool strict_chain) {
+                      double* Yhat, double* nll, double* xT, bool strict_chain, double* nll_steps = nullptr) {
     if (!h || !Y) return -2;
     if (N == 0 || T == 0) return fail(h, "N and T must be positive");
     if (mode < -1 || mode > 1) return fail(h, "smoother_mode must be -1, 0 or 1");
@@ -630,12 +638,13 @@ static int fused_pass(moihgp_handle* h, const double* Y, size_t N, size_t T, con
         c.Y = Y; c.U_host = h->U.data(); c.S_host = h->S.data(); c.consts = h->d_consts; c.sigma = h->sigma;
         c.nll_const = nll_step_const(h->S.data(), h->p, L, h->sigma);
         c.N = (long long)N; c.T = (long long)T; c.mode = mode < 0 ? 1 : mode; c.x0 = x0; c.X = X; c.Xs = Xs; c.nll = nll; c.xT = xT; c.mk = mk; c.nan_flag = nanf; c.seqs_per_warp = h->chain_spw;
+        c.nll_steps = nll_steps;
         CK(launch_chain(h->p, L, D, c, h->stream));
         h->launches += Xs ? 2 : 1;
     } else {
         ScanArgs a{};
         a.mk = mk;
-        a.N = (long long)N; a.T = (long long)T; a.x0 = x0; a.X = X; a.Xs = Xs; a.xT = xT;
+        a.N = (long long)N; a.T = (long long)T; a.x0 = x0; a.X = X; a.Xs = Xs; a.xT = xT; a.nll_steps = nll_steps;
         if (const int rc = scan_pass(h, Y, mode < 0 ? 1 : mode, nll, a)) return rc;
     }
     if (Yhat) { CK(launch_backproject(X, h->d_U, h->d_S, h->p, L, D, (long long)N, (long long)T, Yhat, h->stream)); h->launches += 1; mark(mk, "k_backproject"); }
@@ -645,6 +654,38 @@ static int fused_pass(moihgp_handle* h, const double* Y, size_t N, size_t T, con
 int moihgp_cuda_filter_smoother_nll_dev(moihgp_handle* h, const double* Y, size_t N, size_t T, const double* x0, int mode,
                                         double* X, double* Xs, double* Yhat, double* nll, double* xT) {
     return fused_pass(h, Y, N, T, x0, mode, X, Xs, Yhat, nll, xT, /*strict_chain=*/true);
+}
+
+int moihgp_cuda_nll_steps_dev(moihgp_handle* h, const double* Y, size_t N, size_t T, const double* x0, double* nll_steps, double* nll,
+                              double* xT) {
+    if (!h) return -2;
+    if (!nll_steps) return fail(h, "nll_steps: the output nll_steps [N][T] is required");
+    if (N == 0 || T == 0) return fail(h, "N and T must be positive");
+    return fused_pass(h, Y, N, T, x0, MOIHGP_SMOOTH_NONE, nullptr, nullptr, nullptr, nll, xT, /*strict_chain=*/true, nll_steps);
+}
+
+// Host buffers: copy in, the device pass, copy out (the input dominates the traffic: no slice pipeline).
+int moihgp_cuda_nll_steps(moihgp_handle* h, const double* Y, size_t N, size_t T, const double* x0, double* nll_steps, double* nll,
+                          double* xT) {
+    if (!h) return -2;
+    if (!nll_steps) return fail(h, "nll_steps: the output nll_steps [N][T] is required");
+    if (!Y) return -2;
+    if (N == 0 || T == 0) return fail(h, "N and T must be positive");
+    DeviceGuard guard(h->device);
+    const size_t L = h->L, D = h->dim, p = h->p;
+    double *dY, *dx0 = nullptr, *dsteps, *dnll = nullptr, *dxT = nullptr;
+    if (ws_get(h, "nsY", N * T * p, &dY) || ws_get(h, "nsSteps", N * T, &dsteps)) return -1;
+    if (x0 && ws_get(h, "nsx0", N * L * D, &dx0)) return -1;
+    if (nll && ws_get(h, "nsNll", N, &dnll)) return -1;
+    if (xT && ws_get(h, "nsxT", N * L * D, &dxT)) return -1;
+    CK(cudaMemcpyAsync(dY, Y, sizeof(double) * N * T * p, cudaMemcpyHostToDevice, h->stream));
+    if (x0) CK(cudaMemcpyAsync(dx0, x0, sizeof(double) * N * L * D, cudaMemcpyHostToDevice, h->stream));
+    const int rc = moihgp_cuda_nll_steps_dev(h, dY, N, T, dx0, dsteps, dnll, dxT);
+    if (rc) { cudaStreamSynchronize(h->stream); return rc; }
+    CK(cudaMemcpyAsync(nll_steps, dsteps, sizeof(double) * N * T, cudaMemcpyDeviceToHost, h->stream));
+    if (nll) CK(cudaMemcpyAsync(nll, dnll, sizeof(double) * N, cudaMemcpyDeviceToHost, h->stream));
+    if (xT) CK(cudaMemcpyAsync(xT, dxT, sizeof(double) * N * L * D, cudaMemcpyDeviceToHost, h->stream));
+    return refuse_nan_overflow(h);                       // waits for the copies
 }
 
 // One contiguous block of a longer sequence sharded in TIME over several devices (chunked-scan path), in three phases
@@ -963,7 +1004,7 @@ static int objective_phase(moihgp_handle* h, int phase, const double* Y, size_t 
     if (mk) { mk->st = h->stream; mk->mark("begin"); }
     if (phase != 2) {
         CK(cudaMemsetAsync(pw.nanf, 0, 2 * sizeof(int), h->stream));
-        CK(launch_project(Y, h->d_U, h->d_S, p, L, (long long)N, (long long)T, pw.u, w, yl, pw.rho, pw.nanf, pw.nanrows, (long long)pw.nan_cap, h->stream));
+        CK(launch_project(Y, h->d_U, h->d_S, p, L, (long long)N, (long long)T, pw.u, w, yl, pw.rho, nullptr, pw.nanf, pw.nanrows, (long long)pw.nan_cap, h->stream));
         mark(mk, "k_project");
         h->launches += 2;
     }

@@ -138,12 +138,18 @@ struct FilterCfg {
 // The same variant serves L_real < L latents (L_real * D even, or T even: 16-byte aligned runs of X either way): U has zero columns there, lanes (s, j >= L_real) own no
 // chain, and X keeps the CALLER'S layout [t][L_real][D] - a sequence-round is L steps of L_real * D doubles, staged and
 // copied out with run-time lengths.
-template <int P, int L, int D, int NS_, bool PADP>
+// STEPS: the filter-only variant that also writes every step's NLL term, nll_steps[n][t] (MOIHGP::negLogLikelihood(x_{t-1}, y_t),
+// moihgp.h:614-688); X must be null.  The owner lane of each row leaves sqrt(q) in the padding of its sequence's exchange tile,
+// lane (s, j) overwrites the u it consumed with v^2, and after phase 2 lane (s, i) sums v^2 / (2 S_l) of its row over the
+// L_real latents in a fixed order that starts at latent i mod L_real (a row read from column 0 would put 16 lanes on one bank
+// pair): the stores leave as NS contiguous runs of L steps.  1 / (2 S_l), 1 / (2 sigma) and the per-step constant sit in
+// 8 (L + 2) extra bytes of dynamic shared memory, not in registers.
+template <int P, int L, int D, int NS_, bool PADP, bool STEPS>
 __global__ void __launch_bounds__(32, 14) k_filter_chain(const double* __restrict__ Y, const __grid_constant__ ProjConsts<P, L> pc,
                                                     const LatentConsts* __restrict__ consts, double sigma, double nll_const,
                                                     long long N, long long T, const double* __restrict__ x0,
                                                     double* __restrict__ X, double* __restrict__ nll, double* __restrict__ xT,
-                                                    int* __restrict__ nan_flag, int p_real, int L_real) {
+                                                    int* __restrict__ nan_flag, int p_real, int L_real, double* __restrict__ nll_steps) {
     using C = FilterCfg<P, L, D, NS_>;
     constexpr int NS = C::NS, CH = C::CH, KB = C::KB, NB = C::NB, LD = C::LD, R = C::R, RB = C::RB;
     static_assert(P % 4 == 0 && (CH & (CH - 1)) == 0 && CH <= 32, "P must be 4, 8, 16, 32 or 64");
@@ -154,6 +160,7 @@ __global__ void __launch_bounds__(32, 14) k_filter_chain(const double* __restric
     unsigned char* ytile = smem_raw;                                           // [STAGES][32 rows][P] swizzled
     double* xch = reinterpret_cast<double*>(smem_raw + STAGES * C::TILE);      // [NS][L][XROW]
     double* ost = xch + C::XCH;                                                // [NS][L][L*D]
+    double* kst = ost + C::OSTD;                                               // STEPS: [L] 1 / (2 S_l), the per-step constant, 1 / (2 sigma)
     const int lane = threadIdx.x;
     const int s = lane / L, j = lane % L;                                      // phase 2: (sequence, latent)
     const long long n0 = (long long)blockIdx.x * NS;
@@ -196,6 +203,15 @@ __global__ void __launch_bounds__(32, 14) k_filter_chain(const double* __restric
     const double rs_j = pc.rs[j];                                              // S_j^-1/2  (moihgp.h:181)
     double rho_acc = 0.0, vsq_acc = 0.0;
     bool saw_nan = false;
+    if (STEPS) {
+        if (lane < L) kst[lane] = lane < Lr ? 0.5 / __ldg(&consts[lane].S) : 0.0;   // read by phase 2 after the first round's __syncwarp
+        if (lane == 0) {
+            double logs = 0.0;
+            for (int l = 0; l < Lr; ++l) logs += __ldg(&consts[l].logS);
+            kst[L] = nll_const + 0.5 * logs;                                   // moihgp.h:652, ihgp.h:207
+            kst[L + 1] = 0.5 / sigma;
+        }
+    }
 
     // ---- cp.async producer: tile of round r into stage r % STAGES ----------------------------------
     // pass k of a round covers rows lr + RPP * k (lr = lane / CH), chunk lc16 = lane % CH of each
@@ -249,9 +265,9 @@ __global__ void __launch_bounds__(32, 14) k_filter_chain(const double* __restric
     for (int r = 0; r < STAGES - 1; ++r) issue(r);
 
     double* const xw = xch + (g4 / L) * C::XSEQ + (g4 % L) * C::XROW + 2 * q4;   // + row-block offset below
-    const double* const xc = xch + s * C::XSEQ + j;
+    double* const xc = xch + s * C::XSEQ + j;
     double* const oc = ost + s * C::OSEQ + j * D;
-    double* const Xcta = X ? X + (size_t)n0 * T * LDr : nullptr;
+    double* const Xcta = !STEPS && X ? X + (size_t)n0 * T * LDr : nullptr;     // STEPS writes no X: its copy-out is dead code
 
     for (long long r = 0; r < rounds; ++r) {
         issue(r + STAGES - 1);
@@ -330,6 +346,8 @@ __global__ void __launch_bounds__(32, 14) k_filter_chain(const double* __restric
                 saw_nan = saw_nan || (q != q);
                 rho_acc += sqrt(q);                                               // norm, not squared (Q9); NaN row => NaN NLL, as the reference
             }
+            // the row's residual norm into the padding after its sequence's L exchange rows (nothing else writes there)
+            if (STEPS && owner) xch[own_s * C::XSEQ + L * C::XROW + own_i] = sqrt(q);
             // missing observations (NaN): least-squares projection on the observed outputs, moihgp.h:167-178.  Rare: the
             // whole warp solves one such row at a time, scratch in the (idle) staging tile.
             unsigned nanrows = __ballot_sync(FULL, own_ok && (ysq != ysq));
@@ -376,7 +394,8 @@ __global__ void __launch_bounds__(32, 14) k_filter_chain(const double* __restric
                 vsq_acc = fma(v, v, vsq_acc);
 #pragma unroll
                 for (int a = 0; a < D; ++a) x[a] = xn[a];
-                store_state<D>(oc + i * LDr, xn);
+                if (STEPS) xc[i * C::XROW] = v * v * kst[j];                      // ihgp.h:207, into this lane's own u slot (already read)
+                else store_state<D>(oc + i * LDr, xn);
             }
         } else {
 #pragma unroll
@@ -399,10 +418,28 @@ __global__ void __launch_bounds__(32, 14) k_filter_chain(const double* __restric
 #pragma unroll
                     for (int a = 0; a < D; ++a) x[a] = xn[a];
                 }
-                store_state<D>(oc + i * LDr, x);
+                if (STEPS) xc[i * C::XROW] = v * v * kst[j];
+                else store_state<D>(oc + i * LDr, x);
             }
         }
         __syncwarp();
+        // ---- per-step NLL terms: lane (s, i) sums row i of sequence s over the latents, in order ------------
+        if (STEPS && lane < R) {
+            const double* xr = xch + s * C::XSEQ + j * C::XROW;                   // lane (s, j) serves step i = j
+            double vs = 0.0;
+            if (!PADP) {
+#pragma unroll
+                for (int k = 0; k < L; ++k) vs += xr[(j + k) & (L - 1)];
+            } else {
+                int l = j % Lr;
+                for (int k = 0; k < Lr; ++k) {
+                    vs += xr[l];
+                    if (++l == Lr) l = 0;
+                }
+            }
+            const double rho = xch[s * C::XSEQ + L * C::XROW + j];
+            if (seq_ok && t0 + j < T) nll_steps[(size_t)n * T + t0 + j] = rho * kst[L + 1] + vs + kst[L];   // moihgp.h:652-653
+        }
         // ---- store: NS contiguous runs of L rows ------------------------------------------------------
         if (Xcta && PADP && Lr != L) {
             // padded latents: a sequence-round is L steps of LDr doubles (even), copied out in 16-byte pieces with run-time lengths
@@ -634,9 +671,11 @@ __global__ void __launch_bounds__(32, 14) k_smooth_chain(const double* __restric
     if (lane == 0) bulk_wait_read<0>();            // shared memory must outlive the last bulk store's reads
 }
 
-template <int P, int L, int D, int NS>
+// STEPS: the filter-only pass with per-step NLL terms (a.nll_steps; a.X and a.Xs null)
+template <int P, int L, int D, int NS, bool STEPS>
 cudaError_t run_chain_ns(const ChainArgs& a, cudaStream_t st) {
     using FS = FilterCfg<P, L, D, NS>;
+    constexpr int FBYTES = FS::BYTES + (STEPS ? 8 * (L + 2) : 0);     // STEPS: the table of k_filter_chain's kst
     constexpr int SNS = (NS >= 2 && NS == 32 / L) ? NS / 2 : NS;     // smoother: half the sequences per warp ...
     constexpr int SRM = (NS >= 2 && NS == 32 / L) ? 2 : 1;           // ... rounds twice as long: 2x longer contiguous runs per bulk copy
     using SS = SmoothCfg<L, D, SNS, SRM>;
@@ -650,16 +689,19 @@ cudaError_t run_chain_ns(const ChainArgs& a, cudaStream_t st) {
     const unsigned grid = (unsigned)((a.N + NS - 1) / NS);
     static std::atomic<int> attr_done[64];          // per device: function attributes belong to the device's context
     if (AttrOnce once(attr_done); once) {
-        cudaFuncSetAttribute(k_filter_chain<P, L, D, NS, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, FS::BYTES);
-        cudaFuncSetAttribute(k_filter_chain<P, L, D, NS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, FS::BYTES);
-        cudaFuncSetAttribute(k_smooth_chain<L, D, 0, SNS, SRM, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SS::BYTES);
-        cudaFuncSetAttribute(k_smooth_chain<L, D, 1, SNS, SRM, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SS::BYTES);
-        cudaFuncSetAttribute(k_smooth_chain<L, D, 0, SNS, SRM, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SS::BYTES);
-        cudaFuncSetAttribute(k_smooth_chain<L, D, 1, SNS, SRM, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SS::BYTES);
+        cudaFuncSetAttribute(k_filter_chain<P, L, D, NS, false, STEPS>, cudaFuncAttributeMaxDynamicSharedMemorySize, FBYTES);
+        cudaFuncSetAttribute(k_filter_chain<P, L, D, NS, true, STEPS>, cudaFuncAttributeMaxDynamicSharedMemorySize, FBYTES);
+        if constexpr (!STEPS) {
+            cudaFuncSetAttribute(k_smooth_chain<L, D, 0, SNS, SRM, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SS::BYTES);
+            cudaFuncSetAttribute(k_smooth_chain<L, D, 1, SNS, SRM, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SS::BYTES);
+            cudaFuncSetAttribute(k_smooth_chain<L, D, 0, SNS, SRM, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SS::BYTES);
+            cudaFuncSetAttribute(k_smooth_chain<L, D, 1, SNS, SRM, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SS::BYTES);
+        }
     }
-    if (!padded) k_filter_chain<P, L, D, NS, false><<<grid, 32, FS::BYTES, st>>>(a.Y, pc, a.consts, a.sigma, a.nll_const, a.N, a.T, a.x0, a.X, a.nll, a.xT, a.nan_flag, P, L);
-    else k_filter_chain<P, L, D, NS, true><<<grid, 32, FS::BYTES, st>>>(a.Y, pc, a.consts, a.sigma, a.nll_const, a.N, a.T, a.x0, a.X, a.nll, a.xT, a.nan_flag, p_real, L_real);
+    if (!padded) k_filter_chain<P, L, D, NS, false, STEPS><<<grid, 32, FBYTES, st>>>(a.Y, pc, a.consts, a.sigma, a.nll_const, a.N, a.T, a.x0, a.X, a.nll, a.xT, a.nan_flag, P, L, a.nll_steps);
+    else k_filter_chain<P, L, D, NS, true, STEPS><<<grid, 32, FBYTES, st>>>(a.Y, pc, a.consts, a.sigma, a.nll_const, a.N, a.T, a.x0, a.X, a.nll, a.xT, a.nan_flag, p_real, L_real, a.nll_steps);
     mark(a.mk, "k_filter_chain");
+    if constexpr (STEPS) return cudaGetLastError();
     if (a.Xs) {
         const unsigned sgrid = (unsigned)((a.N + SNS - 1) / SNS);
         if (padL) {
@@ -677,16 +719,21 @@ cudaError_t run_chain_ns(const ChainArgs& a, cudaStream_t st) {
 // Sequences per warp.  Measured on B200 (BASELINE config 3, profiles/r01): a full warp (32 / L sequences) is fastest
 // even when that leaves < 2 warps per SM sub-partition - the pass is bound by HBM, not by latency - so that is the
 // automatic choice; fewer sequences per warp (idle lanes in the recurrence phase, more warps) stay selectable.
+// The per-step NLL pass always takes the full warp: its variant is instantiated for that choice only.
 template <int P, int L, int D, bool ALLNS>
 cudaError_t run_chain(const ChainArgs& a, cudaStream_t st) {
     constexpr int NSMAX = 32 / L, NSMIN = L >= 8 ? 1 : 8 / L;
+    if (a.nll_steps) {
+        if constexpr (L == 1 && D == 3) return cudaErrorInvalidValue;     // not served (chain.cu: find_shape)
+        else return run_chain_ns<P, L, D, NSMAX, true>(a, st);
+    }
     if constexpr (!ALLNS) {
-        return run_chain_ns<P, L, D, NSMAX>(a, st);
+        return run_chain_ns<P, L, D, NSMAX, false>(a, st);
     } else {
         const int ns = a.seqs_per_warp <= 0 ? NSMAX : a.seqs_per_warp;
-        if (ns >= NSMAX) return run_chain_ns<P, L, D, NSMAX>(a, st);
-        if (NSMAX / 2 >= NSMIN && ns >= NSMAX / 2) return run_chain_ns<P, L, D, (NSMAX / 2 >= NSMIN ? NSMAX / 2 : NSMAX)>(a, st);
-        return run_chain_ns<P, L, D, (NSMAX / 4 >= NSMIN ? NSMAX / 4 : NSMIN)>(a, st);
+        if (ns >= NSMAX) return run_chain_ns<P, L, D, NSMAX, false>(a, st);
+        if (NSMAX / 2 >= NSMIN && ns >= NSMAX / 2) return run_chain_ns<P, L, D, (NSMAX / 2 >= NSMIN ? NSMAX / 2 : NSMAX), false>(a, st);
+        return run_chain_ns<P, L, D, (NSMAX / 4 >= NSMIN ? NSMAX / 4 : NSMIN), false>(a, st);
     }
 }
 

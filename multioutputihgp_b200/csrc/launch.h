@@ -44,7 +44,7 @@ cudaError_t launch_polar(const double* A /*[p][L]*/, int p, int L, double* U, in
 // project.cu
 size_t project_tiles(long long T);     // tiles of 128 time steps per sequence: rho_part is [N][project_tiles(T)]
 cudaError_t launch_project(const double* Y, const double* U, const double* S, int p, int L, long long N, long long T,
-                           double* u, double* w, double* yl, double* rho_part, int* nan_info /*{flag, count}*/, long long* nan_rows,
+                           double* u, double* w, double* yl, double* rho_part, double* rho_row /*[N][T] or null*/, int* nan_info /*{flag, count}*/, long long* nan_rows,
                            long long nan_cap, cudaStream_t stream);
 cudaError_t launch_backproject(const double* X, const double* U, const double* S, int p, int L, int d, long long N,
                                long long T, double* Yhat, cudaStream_t stream);
@@ -96,6 +96,8 @@ struct ScanArgs {
     double* x_end = nullptr;      // phase 1: [N][L][D] filtered state after the block's last step, from x0
     int phase = 0;                // 0: whole pass; 1: summaries + forward chain -> x_end; 2: forward chain from the true
                                   // x0, backward chain from b_end = 0 -> b_out; 3: backward chain from b_end + final pass
+    double* nll_steps = nullptr;  // [N][T] per-step NLL terms or null (phase 0; scan_pass in capi.cu)
+    double* vstep = nullptr;      // [N][L][T] squared innovations of the final pass (workspace of nll_steps) or null
     Marker* mk = nullptr;
 };
 size_t scan_chunks(long long T);
@@ -104,6 +106,9 @@ size_t scan_superblocks(long long T);
 int scan_launch_count(long long T);
 cudaError_t launch_scan(int dim, int mode, const ScanArgs& a, cudaStream_t st);
 size_t nll_partials(long long N);
+// per-step NLL terms: nll_steps holds the per-row residual norms on entry (launch_project's rho_row) and the terms on return
+cudaError_t launch_nll_steps(const double* vstep, const LatentConsts* consts, const double* S, double sigma, int p, int L, long long N,
+                             long long T, double* nll_steps, cudaStream_t st);
 cudaError_t launch_nll_reduce(const double* rho_part, const double* vsq, const LatentConsts* consts, const double* S, double sigma,
                               int p, int L, long long N, long long T, double* part, double* nll, cudaStream_t st);
 
@@ -120,6 +125,7 @@ struct ChainArgs {
     double *X, *Xs, *nll, *xT;    // X must be non-null when Xs is requested
     int* nan_flag;                // set to 1 if a NaN observation was seen
     int seqs_per_warp = 0;        // 0 = automatic
+    double* nll_steps = nullptr;  // [N][T] per-step NLL terms (filter-only pass: X and Xs null) or null
     Marker* mk = nullptr;
 };
 bool chain_supported(int p, int L, int dim, long long T);     // a many-chains instantiation serves the shape (exactly, or padded to the next widths)

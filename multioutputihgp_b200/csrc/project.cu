@@ -60,6 +60,7 @@ __device__ __forceinline__ double block_sum(double v, double* red) {
 //   w[n][l][t]    = sum_r U[r][l] y[r]                      (optional, objective path)
 //   yl[n][l][t]   = y[l]  (raw output l, for pv: moihgp.h:510, Q8)   (optional, objective path)
 //   rho_part[n][tile] = sum over the tile of || y - U U' y ||_2      (optional)
+//   rho_row[n][t] = || y_t - U U' y_t ||_2 of every row               (optional; only together with rho_part)
 //   nan_info      = {flag, count}: flag set to 1 if any y is NaN; rows with a NaN are appended to nan_rows (global row
 //                   index n*T + t, at most nan_cap entries) and re-projected by k_nan_fix (missing-data LS projection)
 __device__ __forceinline__ void note_nan_row(int* nan_info, long long* nan_rows, long long nan_cap, long long row) {
@@ -72,7 +73,7 @@ __device__ __forceinline__ void note_nan_row(int* nan_info, long long* nan_rows,
 __global__ void __launch_bounds__(PT) k_project(const double* __restrict__ Y, const double* __restrict__ U,
                                                const double* __restrict__ S, int p, int L, long long T,
                                                double* __restrict__ u, double* __restrict__ w, double* __restrict__ yl,
-                                               double* __restrict__ rho_part, int* __restrict__ nan_info,
+                                               double* __restrict__ rho_part, double* __restrict__ rho_row, int* __restrict__ nan_info,
                                                long long* __restrict__ nan_rows, long long nan_cap) {
     extern __shared__ double sm[];
     __shared__ double red[PT / 32];
@@ -152,6 +153,7 @@ __global__ void __launch_bounds__(PT) k_project(const double* __restrict__ Y, co
             }
         }
         if (rho_part) {
+            if (rho_row && live) rho_row[n * T + t] = sqrt(q);
             const double s = block_sum<PT>(live ? sqrt(q) : 0.0, red);
             if (tid == 0) rho_part[n * rho_tiles + tile * (PT / RU)] = s;
         }
@@ -178,7 +180,7 @@ template <int NB>
 __global__ void __launch_bounds__(MT, NB <= 4 ? 3 : 2) k_project_mma(const double* __restrict__ Y, const double* __restrict__ U,
                                                    const double* __restrict__ S, int p, int L, long long T,
                                                    double* __restrict__ u, double* __restrict__ w, double* __restrict__ yl,
-                                                   double* __restrict__ rho_part, int* __restrict__ nan_info,
+                                                   double* __restrict__ rho_part, double* __restrict__ rho_row, int* __restrict__ nan_info,
                                                    long long* __restrict__ nan_rows, long long nan_cap) {
     using SMC = MmaSmem<NB>;
     extern __shared__ __align__(16) unsigned char smraw[];
@@ -312,6 +314,7 @@ __global__ void __launch_bounds__(MT, NB <= 4 ? 3 : 2) k_project_mma(const doubl
         const bool square_ok = p == L && ysq == ysq;
         bad_row[rb] = t < T && !(q >= 1e-4 * ysq) && !square_ok;
         if (q4 == 0 && t < T && !bad_row[rb] && q >= 1e-4 * ysq) rho_sum += sqrt(q);
+        if (rho_row && q4 == 0 && t < T && !bad_row[rb]) rho_row[n * T + t] = q >= 1e-4 * ysq ? sqrt(q) : 0.0;
     }
     if (bad_row[0] || bad_row[1]) any_bad = 1;
     __syncthreads();
@@ -338,6 +341,7 @@ __global__ void __launch_bounds__(MT, NB <= 4 ? 3 : 2) k_project_mma(const doubl
                 }
                 if (isn) note_nan_row(nan_info, nan_rows, nan_cap, n * T + t0 + row0 + 8 * rb);
                 rho_sum += sqrt(q);
+                if (rho_row) rho_row[n * T + t0 + row0 + 8 * rb] = sqrt(q);
             }
         }
     }
@@ -390,7 +394,7 @@ __global__ void __launch_bounds__(32 * NW, 1) k_project_rows(const __grid_consta
                                                             const double* __restrict__ U, const double* __restrict__ S, int p, int L,
                                                             long long T, unsigned units_per_seq, unsigned total_units, int nbox,
                                                             double* __restrict__ u, double* __restrict__ w, double* __restrict__ yl,
-                                                            double* __restrict__ rho_part, int* __restrict__ nan_info,
+                                                            double* __restrict__ rho_part, double* __restrict__ rho_row, int* __restrict__ nan_info,
                                                             long long* __restrict__ nan_rows, long long nan_cap) {
     using SMC = RowsSmem<NB>;
     extern __shared__ unsigned char smraw_unaligned[];
@@ -507,6 +511,7 @@ __global__ void __launch_bounds__(32 * NW, 1) k_project_rows(const __grid_consta
                 }
             }
         }
+        if (rho_row && k < nk && (long long)unit_k * RU + tau < T) rho_row[(size_t)n_k * T + (size_t)unit_k * RU + tau] = rho;
         __syncwarp();
 #pragma unroll
         for (int o = 8; o >= 1; o >>= 1) rho += __shfl_xor_sync(FULL, rho, o);       // fixed-order sum over the unit's 16 rows
@@ -656,13 +661,13 @@ __global__ void __launch_bounds__(PT) k_backproject(const double* __restrict__ X
 
 template <int NB>
 cudaError_t run_project_mma(const double* Y, const double* U, const double* S, int p, int L, long long N, long long T, double* u,
-                            double* w, double* yl, double* rho_part, int* nan_info, long long* nan_rows, long long nan_cap,
+                            double* w, double* yl, double* rho_part, double* rho_row, int* nan_info, long long* nan_rows, long long nan_cap,
                             cudaStream_t stream) {
     using SMC = MmaSmem<NB>;
     static std::atomic<int> attr_done[64];          // per device: function attributes belong to the device's context
     if (AttrOnce once(attr_done); once) cudaFuncSetAttribute(k_project_mma<NB>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMC::BYTES);
     const unsigned grid = (unsigned)(((T + PT - 1) / PT) * N);
-    k_project_mma<NB><<<grid, MT, SMC::BYTES, stream>>>(Y, U, S, p, L, T, u, w, yl, rho_part, nan_info, nan_rows, nan_cap);
+    k_project_mma<NB><<<grid, MT, SMC::BYTES, stream>>>(Y, U, S, p, L, T, u, w, yl, rho_part, rho_row, nan_info, nan_rows, nan_cap);
     return cudaGetLastError();
 }
 
@@ -682,7 +687,7 @@ EncodeTiledFn encode_tiled_fn() {
 
 template <int NB, int NW, int NST>
 cudaError_t run_project_rows(const CUtensorMap& tm, const double* Y, const double* U, const double* S, int p, int L, long long N, long long T,
-                             int nbox, double* u, double* w, double* yl, double* rho_part, int* nan_info, long long* nan_rows,
+                             int nbox, double* u, double* w, double* yl, double* rho_part, double* rho_row, int* nan_info, long long* nan_rows,
                              long long nan_cap, cudaStream_t stream) {
     using SMC = RowsSmem<NB>;
     const size_t smem = SMC::bytes(p, nbox, NW, NST);
@@ -692,7 +697,7 @@ cudaError_t run_project_rows(const CUtensorMap& tm, const double* Y, const doubl
     const int per_sm = (int)std::max<size_t>(1, std::min<size_t>(4, (size_t)(227 * 1024) / (smem + 1024)));
     const long long grid = std::min<long long>((total + NW - 1) / NW, 148LL * per_sm);
     k_project_rows<NB, NW, NST><<<(unsigned)grid, 32 * NW, smem, stream>>>(tm, Y, U, S, p, L, T, (unsigned)ups, (unsigned)total, nbox, u, w, yl,
-                                                                           rho_part, nan_info, nan_rows, nan_cap);
+                                                                           rho_part, rho_row, nan_info, nan_rows, nan_cap);
     return cudaGetLastError();
 }
 
@@ -701,7 +706,7 @@ cudaError_t run_project_rows(const CUtensorMap& tm, const double* Y, const doubl
 // k_project_rows
 template <int NB>
 bool try_project_rows(cudaError_t& e, const double* Y, const double* U, const double* S, int p, int L, long long N, long long T, double* u,
-                      double* w, double* yl, double* rho_part, int* nan_info, long long* nan_rows, long long nan_cap, cudaStream_t stream) {
+                      double* w, double* yl, double* rho_part, double* rho_row, int* nan_info, long long* nan_rows, long long nan_cap, cudaStream_t stream) {
     using SMC = RowsSmem<NB>;
     const size_t cap = 227 * 1024;
     const long long rows = N * T, ups = (T + RU - 1) / RU;
@@ -717,7 +722,7 @@ bool try_project_rows(cudaError_t& e, const double* Y, const double* U, const do
         return false;
 #define MOIHGP_TRY_ROWS(NW_, NST_, NBOX_)                                                                                           \
     if (SMC::bytes(p, NBOX_, NW_, NST_) <= cap) {                                                                                   \
-        e = run_project_rows<NB, NW_, NST_>(tm, Y, U, S, p, L, N, T, NBOX_, u, w, yl, rho_part, nan_info, nan_rows, nan_cap, stream); \
+        e = run_project_rows<NB, NW_, NST_>(tm, Y, U, S, p, L, N, T, NBOX_, u, w, yl, rho_part, rho_row, nan_info, nan_rows, nan_cap, stream); \
         return true;                                                                                                                \
     }
     MOIHGP_TRY_ROWS(16, 2, nb_narrow)   // 1
@@ -733,30 +738,30 @@ bool try_project_rows(cudaError_t& e, const double* Y, const double* U, const do
 size_t project_tiles(long long T) { return (size_t)((T + RU - 1) / RU); }
 
 cudaError_t launch_project(const double* Y, const double* U, const double* S, int p, int L, long long N, long long T,
-                           double* u, double* w, double* yl, double* rho_part, int* nan_info, long long* nan_rows, long long nan_cap,
+                           double* u, double* w, double* yl, double* rho_part, double* rho_row, int* nan_info, long long* nan_rows, long long nan_cap,
                            cudaStream_t stream) {
     const bool aligned = (reinterpret_cast<size_t>(Y) & 15) == 0;
     cudaError_t e = cudaSuccess;
     bool done = false;
     if (p % 2 == 0 && aligned && L <= 64 && p >= 8) {
-        if (L <= 8) done = try_project_rows<1>(e, Y, U, S, p, L, N, T, u, w, yl, rho_part, nan_info, nan_rows, nan_cap, stream);
-        else if (L <= 16) done = try_project_rows<2>(e, Y, U, S, p, L, N, T, u, w, yl, rho_part, nan_info, nan_rows, nan_cap, stream);
-        else if (L <= 32) done = try_project_rows<4>(e, Y, U, S, p, L, N, T, u, w, yl, rho_part, nan_info, nan_rows, nan_cap, stream);
-        else done = try_project_rows<8>(e, Y, U, S, p, L, N, T, u, w, yl, rho_part, nan_info, nan_rows, nan_cap, stream);
+        if (L <= 8) done = try_project_rows<1>(e, Y, U, S, p, L, N, T, u, w, yl, rho_part, rho_row, nan_info, nan_rows, nan_cap, stream);
+        else if (L <= 16) done = try_project_rows<2>(e, Y, U, S, p, L, N, T, u, w, yl, rho_part, rho_row, nan_info, nan_rows, nan_cap, stream);
+        else if (L <= 32) done = try_project_rows<4>(e, Y, U, S, p, L, N, T, u, w, yl, rho_part, rho_row, nan_info, nan_rows, nan_cap, stream);
+        else done = try_project_rows<8>(e, Y, U, S, p, L, N, T, u, w, yl, rho_part, rho_row, nan_info, nan_rows, nan_cap, stream);
     }
     // the tile kernels write one partial sum per 128 steps into the first of its eight slots: clear the others
     if (!done && rho_part) cudaMemsetAsync(rho_part, 0, sizeof(double) * (size_t)N * project_tiles(T), stream);
     if (done) {
     } else if (p % 2 == 0 && aligned && L <= 64 && p >= 8) {
-        if (L <= 8) e = run_project_mma<1>(Y, U, S, p, L, N, T, u, w, yl, rho_part, nan_info, nan_rows, nan_cap, stream);
-        else if (L <= 16) e = run_project_mma<2>(Y, U, S, p, L, N, T, u, w, yl, rho_part, nan_info, nan_rows, nan_cap, stream);
-        else if (L <= 32) e = run_project_mma<4>(Y, U, S, p, L, N, T, u, w, yl, rho_part, nan_info, nan_rows, nan_cap, stream);
-        else e = run_project_mma<8>(Y, U, S, p, L, N, T, u, w, yl, rho_part, nan_info, nan_rows, nan_cap, stream);
+        if (L <= 8) e = run_project_mma<1>(Y, U, S, p, L, N, T, u, w, yl, rho_part, rho_row, nan_info, nan_rows, nan_cap, stream);
+        else if (L <= 16) e = run_project_mma<2>(Y, U, S, p, L, N, T, u, w, yl, rho_part, rho_row, nan_info, nan_rows, nan_cap, stream);
+        else if (L <= 32) e = run_project_mma<4>(Y, U, S, p, L, N, T, u, w, yl, rho_part, rho_row, nan_info, nan_rows, nan_cap, stream);
+        else e = run_project_mma<8>(Y, U, S, p, L, N, T, u, w, yl, rho_part, rho_row, nan_info, nan_rows, nan_cap, stream);
     } else {
         const size_t smem = sizeof(double) * ((size_t)PT * (PC + 1) + (size_t)PC * L + (size_t)PT * (L + 1));
         if (smem > 48 * 1024) cudaFuncSetAttribute(k_project, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         const unsigned grid = (unsigned)(((T + PT - 1) / PT) * N);
-        k_project<<<grid, PT, smem, stream>>>(Y, U, S, p, L, T, u, w, yl, rho_part, nan_info, nan_rows, nan_cap);
+        k_project<<<grid, PT, smem, stream>>>(Y, U, S, p, L, T, u, w, yl, rho_part, rho_row, nan_info, nan_rows, nan_cap);
         e = cudaGetLastError();
     }
     if (e != cudaSuccess) return e;

@@ -70,14 +70,15 @@ __host__ __device__ __forceinline__ int tile_group_stride(int RS) { return SUB *
 // One warp, one (sequence, latent, chunk).  uu[i] = u at global step tf + i (0 beyond T), u_next = u at the first
 // step of the next chunk (0 if none), tf = global index of this lane's first step.
 //   FINAL = false: x_in / b_in are zero (or a unit vector for k_response); returns f_end (lane 31) and beta (lane 0).
-//   FINAL = true : additionally stores X / Xs rows into the shared tiles and returns sum v^2 (per lane).
+//   FINAL = true : additionally stores X / Xs rows into the shared tiles and returns sum v^2 (per lane); vrow (or null) receives
+//                  each step's v^2 at its global step index.
 //   INTERIOR     : every step of the chunk is < T - 1 (no end-of-sequence predicates).
 //   pw           : the latent's scan powers, [2][5][D*D] doubles: M^(SUB 2^k) then G^(SUB 2^k), k = 0..4.
 template <int D, int MODE, bool FINAL, bool INTERIOR>
 __device__ __forceinline__ void chunk_pass(const LC<D>& c, const double* __restrict__ pw, const double (&uu)[SUB], double u_next,
                                            long long tf, long long T, const double (&x_in)[D], const double (&b_in)[D],
                                            int lane, double (&f_end)[D], double (&beta)[D], double& vsq,
-                                           double* tX, double* tXs, int RS, double (&x_last_out)[D]) {
+                                           double* tX, double* tXs, int RS, double (&x_last_out)[D], double* __restrict__ vrow) {
     // ---- forward, local --------------------------------------------------------------------
     double z[D];
 #pragma unroll
@@ -123,6 +124,7 @@ __device__ __forceinline__ void chunk_pass(const LC<D>& c, const double* __restr
         for (int q = 0; q < D; ++q) { x[q] = fma(c.K[q], uu[i], xn[q]); X[i][q] = x[q]; }   // ihgp.h:90
         if (FINAL && (INTERIOR || tf + i < T)) {
             vsq = fma(v[i], v[i], vsq);
+            if (vrow) vrow[tf + i] = v[i] * v[i];
 #pragma unroll
             for (int q = 0; q < D; ++q) tX[i * RS + q] = x[q];
         }
@@ -226,7 +228,7 @@ __global__ void __launch_bounds__(32 * LGMAX, 2) k_scan(const double* __restrict
                                                     double* __restrict__ fsum, double* __restrict__ bsum,
                                                     double* __restrict__ X, double* __restrict__ Xs,
                                                     double* __restrict__ vsq_out, double* __restrict__ xT,
-                                                    const double* __restrict__ u_after, int seq_end) {
+                                                    const double* __restrict__ u_after, int seq_end, double* __restrict__ vstep) {
     extern __shared__ double tile[];
     __shared__ double pws[LGMAX][10 * D * D];       // per latent of the CTA: M^(SUB 2^k), then G^(SUB 2^k), k = 0..4
     const int lane = threadIdx.x & 31, wi = threadIdx.x >> 5;
@@ -258,6 +260,7 @@ __global__ void __launch_bounds__(32 * LGMAX, 2) k_scan(const double* __restrict
     LC<D> cst;
     load_lc<D, MODE>(lc, cst);
     const double* up = u + ((size_t)n * L + (active ? l : l0)) * T;
+    double* const vrow = FINAL && vstep ? vstep + ((size_t)n * L + (active ? l : l0)) * T : nullptr;   // laid out like u
     const long long c_lo = c_base + gi * cpc, c_hi = min(c_base + c_cnt, c_lo + cpc);
 
     for (long long c = c_lo; c < c_hi; ++c) {
@@ -287,8 +290,8 @@ __global__ void __launch_bounds__(32 * LGMAX, 2) k_scan(const double* __restrict
             }
             double* tX = tileX + lane * GS + wi * D;
             double* tXs = tileXs + lane * GS + wi * D;
-            if (t0 + CH < T || !seq_end) chunk_pass<D, MODE, FINAL, true>(cst, pws[wi], uu, u_next, tf, T, x_in, b_in, lane, f_end, beta, vsq, tX, tXs, RS, x_last);
-            else chunk_pass<D, MODE, FINAL, false>(cst, pws[wi], uu, u_next, tf, T, x_in, b_in, lane, f_end, beta, vsq, tX, tXs, RS, x_last);
+            if (t0 + CH < T || !seq_end) chunk_pass<D, MODE, FINAL, true>(cst, pws[wi], uu, u_next, tf, T, x_in, b_in, lane, f_end, beta, vsq, tX, tXs, RS, x_last, vrow);
+            else chunk_pass<D, MODE, FINAL, false>(cst, pws[wi], uu, u_next, tf, T, x_in, b_in, lane, f_end, beta, vsq, tX, tXs, RS, x_last, vrow);
             if (!FINAL) {
                 if (lane == 31) {
 #pragma unroll
@@ -451,7 +454,7 @@ __global__ void __launch_bounds__(32) k_scan_weights(const LatentConsts* __restr
     double x_in[D], b_in[D], f_end[D], beta[D], x_last[D], vsq;
 #pragma unroll
     for (int q = 0; q < D; ++q) { x_in[q] = 0.0; b_in[q] = 0.0; }
-    chunk_pass<D, MODE, false, true>(cst, pw, uu, i == CH ? 1.0 : 0.0, (long long)lane * SUB, 1LL << 60, x_in, b_in, lane, f_end, beta, vsq, nullptr, nullptr, 0, x_last);
+    chunk_pass<D, MODE, false, true>(cst, pw, uu, i == CH ? 1.0 : 0.0, (long long)lane * SUB, 1LL << 60, x_in, b_in, lane, f_end, beta, vsq, nullptr, nullptr, 0, x_last, nullptr);
     double* wl = Wsum + (size_t)l * WS_STRIDE;
     if (i < CH) {
         if (lane == 31) {
@@ -494,7 +497,7 @@ __global__ void __launch_bounds__(32) k_response(const LatentConsts* __restrict_
 #pragma unroll
     for (int q = 0; q < D; ++q) { x_in[q] = q == k ? 1.0 : 0.0; b_in[q] = 0.0; }
     const long long T = kind == 0 ? (1LL << 60) : r_last;
-    chunk_pass<D, MODE, false, false>(cst, pw, uu, 0.0, (long long)lane * SUB, T, x_in, b_in, lane, f_end, beta, vsq, nullptr, nullptr, 0, x_last);
+    chunk_pass<D, MODE, false, false>(cst, pw, uu, 0.0, (long long)lane * SUB, T, x_in, b_in, lane, f_end, beta, vsq, nullptr, nullptr, 0, x_last, nullptr);
     if (lane == 0) {
 #pragma unroll
         for (int q = 0; q < D; ++q) Bx[((size_t)l * 2 + kind) * D * D + q * D + k] = beta[q];
@@ -781,6 +784,33 @@ __global__ void __launch_bounds__(128) k_nll_reduce(const double* __restrict__ p
     nll[n] = acc + (double)T * (nll_step_const(S, p, L, sigma) + 0.5 * logs);   // moihgp.h:652
 }
 
+// Per-step terms of the same sum (MOIHGP::negLogLikelihood(x_{t-1}, y_t), moihgp.h:614-688), one thread per (sequence, step):
+//   nll_steps[n][t] = 1/2 rho_t / sigma + sum_l 1/2 v_{l,t}^2 / S_l + nll_step_const + 1/2 sum_l log S_l
+// rho_t arrives in nll_steps itself (the projection's per-row residual norms) and is replaced in place; vstep[n][l][t] holds v^2
+// (the final scan pass).  The latents are summed in order l = 0 .. L-1: deterministic, no atomics.
+__global__ void __launch_bounds__(256) k_nll_steps(const double* __restrict__ vstep, const LatentConsts* __restrict__ consts,
+                                                  const double* __restrict__ S, double sigma, int p, int L, long long N, long long T,
+                                                  double* __restrict__ nll_steps) {
+    __shared__ double hinvS[64];                                         // 1 / (2 S_l)
+    __shared__ double cst;
+    const int tid = threadIdx.x;
+    const bool inv_sm = L <= 64;
+    if (inv_sm && tid < L) hinvS[tid] = 0.5 / consts[tid].S;
+    if (tid == 0) {
+        double logs = 0.0;
+        for (int l = 0; l < L; ++l) logs += consts[l].logS;
+        cst = nll_step_const(S, p, L, sigma) + 0.5 * logs;
+    }
+    __syncthreads();
+    const long long i = (long long)blockIdx.x * blockDim.x + tid;
+    if (i >= N * T) return;
+    const long long n = i / T, t = i - n * T;
+    const double* vr = vstep + (size_t)n * L * T + t;
+    double vs = 0.0;
+    for (int l = 0; l < L; ++l) vs += vr[(size_t)l * T] * (inv_sm ? hinvS[l] : 0.5 / consts[l].S);
+    nll_steps[i] = 0.5 * nll_steps[i] / sigma + vs + cst;
+}
+
 // ---------------------------------------------------------------------------------------------------------------------
 // k_scan_lanes: the FINAL pass with one THREAD per (latent, sub-chunk of SL = 32 steps) instead of one warp per
 // (latent, chunk).  A CTA owns (sequence, group of LG latents, chunk of CH = 256 steps): thread (s, l) runs sub-chunk s
@@ -805,7 +835,7 @@ __device__ __forceinline__ void lanes_chunk(const LC<D>& c, const double (&PM)[D
                                             unsigned long long* ubar, unsigned uphase,
                                             double (*exch)[LG][D], double (*vred)[LG], double* __restrict__ Xg,
                                             double* __restrict__ Xsg, size_t gstride, bool vec_x, double* __restrict__ vsq_dst,
-                                            double* __restrict__ xT_dst) {
+                                            double* __restrict__ xT_dst, double* __restrict__ vrow) {
     constexpr int NT = NSUBC * LG;
     const int len = INTERIOR ? SL : (int)max(0LL, min((long long)SL, T - ts));
     // ---- inputs: this thread's 32 steps of u (contiguous) and the step after them --------------------------------
@@ -866,6 +896,7 @@ __device__ __forceinline__ void lanes_chunk(const LC<D>& c, const double (&PM)[D
             for (int q = 1; q < D; ++q) hax = fma(c.HA[q], x[q], hax);
             const double v = uu[j] - hax;                                   // ihgp.h:206 (pre-step state)
             vsq = fma(v, v, vsq);
+            if (vrow) vrow[j] = v * v;
             double xn[D];
             mv<D>(c.M, x, xn);
 #pragma unroll
@@ -1008,7 +1039,7 @@ __global__ void __launch_bounds__(NSUBC * LG, (D == 2 ? 384 : 256) / (NSUBC * LG
                                                           const double* __restrict__ xin, const double* __restrict__ bin,
                                                           double* __restrict__ X, double* __restrict__ Xs,
                                                           double* __restrict__ vsq_out, double* __restrict__ xT,
-                                                          const double* __restrict__ u_after, int seq_end) {
+                                                          const double* __restrict__ u_after, int seq_end, double* __restrict__ vstep) {
     extern __shared__ double tile[];                  // the CTA's filtered states: [SL][NT] double2 (D = 2) or [D][SL][NT]
     __shared__ double exch[NSUBC][LG][D];
     __shared__ double vred[NSUBC][LG];
@@ -1047,12 +1078,13 @@ __global__ void __launch_bounds__(NSUBC * LG, (D == 2 ? 384 : 256) / (NSUBC * LG
         double* Xsg = Xs ? Xs + go : nullptr;
         double* vdst = vsq_out + ((size_t)c * N + n) * L + l;
         double* xTd = xT ? xT + ((size_t)n * L + l) * D : nullptr;
+        double* vrow = vstep ? vstep + ((size_t)n * L + l) * T + ts : nullptr;
         // the step after this thread's last one: in the block, or the next block's first (sequence sharded in time)
         const double u_nx = ts + SL < T ? __ldg(up + ts + SL) : (u_after ? __ldg(u_after + (size_t)n * L + l) : 0.0);
         if (c * CH + CH < T || !seq_end)
-            lanes_chunk<D, MODE, LG, true>(cst, PM, PG, up, u_nx, ts, T, s, li, tid, x_chunk, b_chunk, tile, &ubar, (unsigned)((c - c_lo) & 1), exch, vred, Xg, Xsg, gstride, vec_x, vdst, xTd);
+            lanes_chunk<D, MODE, LG, true>(cst, PM, PG, up, u_nx, ts, T, s, li, tid, x_chunk, b_chunk, tile, &ubar, (unsigned)((c - c_lo) & 1), exch, vred, Xg, Xsg, gstride, vec_x, vdst, xTd, vrow);
         else
-            lanes_chunk<D, MODE, LG, false>(cst, PM, PG, up, u_nx, ts, T, s, li, tid, x_chunk, b_chunk, tile, &ubar, (unsigned)((c - c_lo) & 1), exch, vred, Xg, Xsg, gstride, vec_x, vdst, xTd);
+            lanes_chunk<D, MODE, LG, false>(cst, PM, PG, up, u_nx, ts, T, s, li, tid, x_chunk, b_chunk, tile, &ubar, (unsigned)((c - c_lo) & 1), exch, vred, Xg, Xsg, gstride, vec_x, vdst, xTd, vrow);
     }
 }
 
@@ -1070,7 +1102,7 @@ cudaError_t launch_scan_lanes(const ScanArgs& a, long long nC, cudaStream_t st) 
     const long long cpc = chunks_per_group(a.N * nLG, nC, target);
     const long long nG = (nC + cpc - 1) / cpc;
     k_scan_lanes<D, MODE, LG><<<(unsigned)(a.N * nG * nLG), NT, smem, st>>>(a.u, a.consts, a.L, a.N, a.T, nC, cpc, a.xin, a.bin, a.X, a.Xs,
-                                                                            a.vsq, a.xT, a.u_after, a.seq_end);
+                                                                            a.vsq, a.xT, a.u_after, a.seq_end, a.vstep);
     return cudaGetLastError();
 }
 
@@ -1104,7 +1136,7 @@ cudaError_t run_scan(const ScanArgs& a, cudaStream_t st) {
     }
     if ((ph == 0 && nC > 1) || ph == 1 || ph == 2) {
         k_scan<D, MODE, false><<<(unsigned)(a.N * nLG), 32 * lg, 0, st>>>(a.u, a.consts, a.L, a.N, a.T, nC, nLG, nC - 1, 1, 1, nullptr, nullptr,
-                                                                         a.fsum, a.bsum, nullptr, nullptr, nullptr, nullptr, a.u_after, a.seq_end);
+                                                                         a.fsum, a.bsum, nullptr, nullptr, nullptr, nullptr, a.u_after, a.seq_end, nullptr);
         mark(a.mk, "k_scan_summaries");
     }
     if ((ph == 0 && nC > 1) || ph == 2) {
@@ -1147,7 +1179,7 @@ cudaError_t run_scan(const ScanArgs& a, cudaStream_t st) {
     const long long cpc = chunks_per_group(a.N * nLG, nC, target);
     const long long nG = (nC + cpc - 1) / cpc;
     k_scan<D, MODE, true><<<(unsigned)(a.N * nG * nLG), 32 * lg, smem, st>>>(a.u, a.consts, a.L, a.N, a.T, nC, nLG, 0, nC, cpc, a.xin, a.bin,
-                                                                            nullptr, nullptr, a.X, a.Xs, a.vsq, a.xT, a.u_after, a.seq_end);
+                                                                            nullptr, nullptr, a.X, a.Xs, a.vsq, a.xT, a.u_after, a.seq_end, a.vstep);
     mark(a.mk, "k_scan_final");
     return cudaGetLastError();
 }
@@ -1181,6 +1213,12 @@ cudaError_t launch_nll_reduce(const double* rho_part, const double* vsq, const L
 }
 
 size_t nll_partials(long long N) { return (size_t)N * nll_nsplit(N); }
+
+cudaError_t launch_nll_steps(const double* vstep, const LatentConsts* consts, const double* S, double sigma, int p, int L, long long N,
+                             long long T, double* nll_steps, cudaStream_t st) {
+    k_nll_steps<<<(unsigned)((N * T + 255) / 256), 256, 0, st>>>(vstep, consts, S, sigma, p, L, N, T, nll_steps);
+    return cudaGetLastError();
+}
 
 // ---- one long sequence sharded in TIME (moihgp_cuda_fsn_block_*): the two carry exchanges on the device ----------------
 // forward  (DIR 0): gathered[g][n][l][D + 1] = [end state of block g from a zero carry-in | first projected observation of g];

@@ -20,6 +20,8 @@ print("objective:", loss, grad.shape)
 m.bind(Y)
 loss_b, grad_b = m.objective_bound()[:2]
 assert abs(loss_b - loss) <= 1e-12 * abs(loss) and np.allclose(grad_b, grad, rtol=1e-12, atol=0)
+e = m.nll_steps(Y)
+assert e["nll_steps"].shape == (6, 300) and np.allclose(e["nll_steps"].sum(axis=1), r["nll"], rtol=1e-10, atol=0)
 learner = MOIHGPOnlineLearning(0.1, 8, 4, gamma=0.9, windowsize=1)
 for t in range(5):
     yhat = learner.step(rng.standard_normal(8))
