@@ -76,7 +76,8 @@ enum { MOIHGP_SMOOTH_NONE = -1, MOIHGP_SMOOTH_REFERENCE_LITERAL = 0, MOIHGP_SMOO
  * `threading` only selects the reference's loss semantics (moihgp.h:588 vs :601, forced off for L < 2). */
 int moihgp_cuda_create(moihgp_handle** out, int kernel, double dt, size_t num_output, size_t num_latent,
                        int threading, int device);
-/* Limits the reference does not have: 1 <= num_latent <= min(num_output, 64).  Every entry point runs on the handle's device
+/* Limits the reference does not have: 1 <= num_latent <= min(num_output, 256); the streaming learner (moihgp_cuda_online_begin)
+ * takes num_latent <= 64.  Every entry point runs on the handle's device
  * and restores the caller's current CUDA device before it returns. */
 void moihgp_cuda_destroy(moihgp_handle* h);
 /* run every kernel of this handle on `cuda_stream` (a cudaStream_t); NULL = the handle's own (non-blocking) stream.

@@ -382,8 +382,13 @@ public:
 
     // Device-resident streaming learner (moihgp_cuda_online_*: window, moving mean, carried state and proximal term in HBM;
     // one CUDA-graph launch per objective evaluation).  Used by OnlineObjective; false / exception-free probes return false
-    // when the shape does not qualify (the caller then keeps the window on the host).
-    bool onlineBegin(size_t windowsize) { return moihgp_cuda_online_begin(_h, windowsize) == 0; }
+    // when the shape does not qualify (the caller then keeps the window on the host).  A model with more than 64 latents is
+    // refused outright: std::runtime_error with the library's message.
+    bool onlineBegin(size_t windowsize) {
+        const int rc = moihgp_cuda_online_begin(_h, windowsize);
+        if (rc != 0 && _num_latent > 64) detail::check(_h, rc, "MOIHGP::onlineBegin");
+        return rc == 0;
+    }
     void onlinePush(const Vec& y, Vec& ma) {
         pack_y(y, &_yb[0]);
         detail::check(_h, moihgp_cuda_online_push(_h, &_yb[0], NULL, &_yb[_num_output]), "MOIHGP::onlinePush");

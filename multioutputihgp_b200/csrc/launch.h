@@ -40,12 +40,23 @@ cudaError_t launch_setup(int dim, const double* d_igp_params, double dt, int L, 
 // polar.cu  (MOIHGP::update's polar factor on the device, for large p * L)
 size_t polar_smem_bytes(int p, int L);
 cudaError_t launch_polar(const double* A /*[p][L]*/, int p, int L, double* U, int* status /*device int*/, cudaStream_t st);
+// L > 64: the Newton-Schulz iteration over many CTAs (tensor pipe); work: polar_wide_doubles(p, L) doubles.  Waits for the
+// stream; *converged = false (U untouched) asks the caller for the host Jacobi
+size_t polar_wide_doubles(int p, int L);
+cudaError_t launch_polar_wide(const double* A /*[p][L]*/, int p, int L, double* U, double* work, int* status /*device int*/, bool* converged,
+                              int* launched, cudaStream_t st);
+
+// Largest number of latent processes a model may have (moihgp_cuda_create)
+constexpr int MAX_LATENT = 256;
 
 // project.cu
 size_t project_tiles(long long T);     // tiles of 128 time steps per sequence: rho_part is [N][project_tiles(T)]
+// doubles of global scratch k_nan_fix needs at this L: one slice of the missing-output solve per CTA of its grid (0: the
+// solve runs in shared memory)
+size_t ls_global_doubles(int L);
 cudaError_t launch_project(const double* Y, const double* U, const double* S, int p, int L, long long N, long long T,
                            double* u, double* w, double* yl, double* rho_part, double* rho_row /*[N][T] or null*/, int* nan_info /*{flag, count}*/, long long* nan_rows,
-                           long long nan_cap, cudaStream_t stream);
+                           long long nan_cap, double* ls_scratch /*[ls_global_doubles(L)] or null when that is 0*/, cudaStream_t stream);
 cudaError_t launch_backproject(const double* X, const double* U, const double* S, int p, int L, int d, long long N,
                                long long T, double* Yhat, cudaStream_t stream);
 
@@ -202,7 +213,11 @@ struct StepArgs {
     int p, L, dim, threading;
     const double *x, *y, *dx;     // device staging: [L][D], [p] (null = predict only), [L][3][D] (may be null)
     double *xnew, *yhat, *dxnew;  // outputs (yhat/dxnew may be null)
+    double* ls_scratch = nullptr; // [step_global_doubles(L)] global scratch of the missing-output solve where that is > 0, else null
 };
+// doubles of global scratch k_step / k_lik need at this L (0: the missing-output solve runs in shared memory)
+size_t step_global_doubles(int L);
+size_t lik_global_doubles(int L);
 cudaError_t launch_step(const StepArgs& a, cudaStream_t st);
 struct LikArgs {
     const LatentConsts* consts;
@@ -212,6 +227,7 @@ struct LikArgs {
     const double *x, *y, *dx;     // dx null => lik2 (no gradient)
     double* loss;                 // [1]
     double* grad;                 // [num_param] or null
+    double* ls_scratch = nullptr; // [lik_global_doubles(L)] where that is > 0, else null
 };
 cudaError_t launch_lik(const LikArgs& a, cudaStream_t st);
 cudaError_t launch_extract_values(const double* X, double* F, long long n, int d, cudaStream_t st);

@@ -952,8 +952,10 @@ __global__ void __launch_bounds__(256) k_obj_finish(const double* __restrict__ l
             grad[i] = a;
         }
     }
-    // CTA 0: the RSPLIT partials of every per-latent sum in fixed order, then the scalar / per-latent entries
-    __shared__ double lat_sums[65 * 8];
+    // CTA 0: the RSPLIT partials of every per-latent sum in fixed order, then the scalar / per-latent entries.
+    // Dynamic shared memory: lat_sums[(L + 1) * 8], gs_term[L].
+    extern __shared__ double fin_sm[];
+    double* lat_sums = fin_sm;
     if (blockIdx.x == 0) {
         for (int i = tid; i < (L + 1) * 5; i += 256) {
             const int l = i / 5, j = i - l * 5;
@@ -966,7 +968,7 @@ __global__ void __launch_bounds__(256) k_obj_finish(const double* __restrict__ l
     if (blockIdx.x != 0) return;
     // the per-latent entries in parallel (thread l), the two scalars by thread 0 in latent order - the same operations in the
     // same order as a single thread would do them, without 64 latents' worth of divisions queued behind one lane
-    __shared__ double gs_term[64];
+    double* gs_term = lat_sums + (size_t)(L + 1) * 8;
     const double steps = (double)N * (double)T;
     for (int l = tid; l < L; l += 256) {
         const double* q = lat_sums + (size_t)l * 8;
@@ -1204,7 +1206,7 @@ cudaError_t run_objective(const ObjArgs& a, cudaStream_t st) {
     mark(a.mk, "k_gradU");
     double* lat_sums = a.lat_sums;
     k_obj_reduce<<<(a.L + 1) * RSPLIT, 256, 0, st>>>(a.part, a.rho, a.L, a.N, (long long)project_tiles(a.T), nC, lat_sums);
-    k_obj_finish<<<(a.p * a.L + 31) / 32, 256, 0, st>>>(lat_sums, a.gU_part, (int)nsplit, a.S, a.sigma, a.p, a.L, a.N, a.T, a.threading, a.loss, a.grad);
+    k_obj_finish<<<(a.p * a.L + 31) / 32, 256, sizeof(double) * ((size_t)(a.L + 1) * 8 + a.L), st>>>(lat_sums, a.gU_part, (int)nsplit, a.S, a.sigma, a.p, a.L, a.N, a.T, a.threading, a.loss, a.grad);
     mark(a.mk, "k_obj_reduce");
     return cudaGetLastError();
 }

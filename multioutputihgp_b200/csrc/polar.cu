@@ -8,7 +8,9 @@
 // k_polar_ns (below) gets the same factor by the Newton-Schulz iteration and runs first; the Jacobi kernel is its fallback.
 #include <cuda_runtime.h>
 #include <math.h>
+#include <algorithm>
 #include "launch.h"
+#include "ptx.cuh"
 
 namespace moihgp {
 
@@ -243,7 +245,188 @@ __global__ void __launch_bounds__(1024) k_polar_ns(const double* __restrict__ A 
         }
 }
 
+// ---------------------------------------------------------------------------------------------------------------------
+// The Newton-Schulz iteration of k_polar_ns for L > 64, over many CTAs: G = X'X and X <- X (3/2 I - 1/2 G) on the FP64
+// tensor pipe (DMMA m8n8k4), one warp per 8 x 8 output tile, each tile's sum over k in one fixed order (bitwise
+// reproducible); max |G - I| by an integer atomicMax on the bit pattern (exact for non-negative doubles, NaN above every
+// number).  The decisions of k_polar_ns (starting scale, stop tests, hand-over) are taken by one thread of k_nsw_ctl on the
+// device; the host launches the iterations in batches and reads one flag between them.
+struct NsState {
+    int active, do_mul, ok, cur, scaled;
+    double Eprev, scale;
+    unsigned long long Ebits;              // max |G - I| of the last G, as bits
+};
+
+// max that keeps a NaN (fmax would drop it)
+__device__ __forceinline__ double nan_max(double a, double b) { return a != a ? a : (b != b ? b : fmax(a, b)); }
+
+// grid-stride over the warps of the launch: warp w takes tile (w / ntc, w % ntc) of an [ntr x ntc] grid of 8 x 8 tiles
+__device__ __forceinline__ bool next_tile(long long& w, long long nw, int ntr, int ntc, int& t0, int& t1) {
+    if (w >= (long long)ntr * ntc) return false;
+    t0 = (int)(w / ntc) * 8;
+    t1 = (int)(w % ntc) * 8;
+    w += nw;
+    return true;
+}
+
+__global__ void __launch_bounds__(256) k_nsw_start(const double* __restrict__ A, long long n, double* __restrict__ X0, NsState* st) {
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) X0[i] = A[i];
+    if (blockIdx.x == 0 && threadIdx.x == 0) {
+        st->active = 1; st->do_mul = 0; st->ok = 0; st->cur = 0; st->scaled = 0;
+        st->Eprev = 1e300; st->scale = 1.0; st->Ebits = 0ull;
+    }
+}
+
+// G = X'X of X = Xb[cur], and max |G - I| into st->Ebits.  only_scaled: run only if the start was rescaled.
+__global__ void __launch_bounds__(256) k_nsw_gram(const double* __restrict__ X0, const double* __restrict__ X1, int p, int L,
+                                                 double* __restrict__ G, NsState* st, int only_scaled) {
+    if (!st->active || (only_scaled && !st->scaled)) return;
+    const double* X = st->cur ? X1 : X0;
+    const int lane = threadIdx.x & 31, g4 = lane >> 2, q4 = lane & 3;
+    const int nt = (L + 7) / 8;
+    long long w = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const long long nw = ((long long)gridDim.x * blockDim.x) >> 5;
+    int i0, j0;
+    while (next_tile(w, nw, nt, nt, i0, j0)) {
+        double c0 = 0.0, c1 = 0.0;
+        const bool ia = i0 + g4 < L, jb = j0 + g4 < L;
+        for (int r0 = 0; r0 < p; r0 += 4) {
+            const int r = r0 + q4;
+            const double a = (r < p && ia) ? X[(size_t)r * L + i0 + g4] : 0.0;
+            const double b = (r < p && jb) ? X[(size_t)r * L + j0 + g4] : 0.0;
+            dmma884(c0, c1, a, b);
+        }
+        double e = 0.0;
+        const int i = i0 + g4;
+#pragma unroll
+        for (int k = 0; k < 2; ++k) {
+            const int j = j0 + 2 * q4 + k;
+            const double g = k ? c1 : c0;
+            if (i < L && j < L) {
+                G[(size_t)i * L + j] = g;
+                e = nan_max(e, fabs(g - (i == j ? 1.0 : 0.0)));
+            }
+        }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) e = nan_max(e, __shfl_xor_sync(FULL, e, o));
+        if (lane == 0) atomicMax(&st->Ebits, (unsigned long long)__double_as_longlong(e));
+    }
+}
+
+// the starting point of k_polar_ns: X as it is when X'X is close to I, else scaled so that every singular value is <= 1
+// (by the Frobenius norm sqrt(trace G) >= sigma_max; the small singular values then take a few more linear steps)
+__global__ void k_nsw_scale_ctl(const double* __restrict__ G, int L, NsState* st) {
+    const double E = __longlong_as_double((long long)st->Ebits);
+    const int Lp = (L + 1) & ~1;
+    if (!(E * (double)Lp < 0.9)) {
+        double tr = 0.0;
+        for (int i = 0; i < L; ++i) tr += G[(size_t)i * L + i];
+        st->scale = (tr > 0.0 && tr < 1e300) ? 1.0 / sqrt(tr) : 0.0;
+        st->scaled = 1;
+        st->Ebits = 0ull;
+    }
+}
+
+__global__ void __launch_bounds__(256) k_nsw_scale(double* __restrict__ X0, long long n, const NsState* st) {
+    if (!st->scaled) return;
+    const double sc = st->scale;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) X0[i] *= sc;
+}
+
+// one step of k_polar_ns's loop, decided on the last E (the same tests in the same order)
+__global__ void k_nsw_ctl(NsState* st, int it) {
+    st->do_mul = 0;
+    if (!st->active) return;
+    const double E = __longlong_as_double((long long)st->Ebits);
+    if (E < 1e-14) { st->ok = 1; st->active = 0; return; }
+    if (!(E == E) || E > 2.5) { st->active = 0; return; }                  // NaN / outside the convergence radius: hand over
+    st->do_mul = 1;
+    st->cur ^= 1;
+    const bool stop = E < 3e-8 || (it >= 3 && E < 1e-12 && E >= 0.5 * st->Eprev);
+    st->Eprev = E;
+    st->Ebits = 0ull;
+    if (stop) { st->ok = 1; st->active = 0; }
+}
+
+// Xb[cur] = Xb[cur ^ 1] (3/2 I - 1/2 G)
+__global__ void __launch_bounds__(256) k_nsw_mul(double* __restrict__ X0, double* __restrict__ X1, int p, int L, const double* __restrict__ G,
+                                                const NsState* st) {
+    if (!st->do_mul) return;
+    const double* X = st->cur ? X0 : X1;
+    double* Xn = st->cur ? X1 : X0;
+    const int lane = threadIdx.x & 31, g4 = lane >> 2, q4 = lane & 3;
+    const int nr = (p + 7) / 8, nc = (L + 7) / 8;
+    long long w = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const long long nw = ((long long)gridDim.x * blockDim.x) >> 5;
+    int r0, j0;
+    while (next_tile(w, nw, nr, nc, r0, j0)) {
+        double c0 = 0.0, c1 = 0.0;
+        const int r = r0 + g4, j = j0 + g4;
+        for (int k0 = 0; k0 < L; k0 += 4) {
+            const int k = k0 + q4;
+            const double a = (r < p && k < L) ? X[(size_t)r * L + k] : 0.0;
+            const double b = (k < L && j < L) ? (k == j ? 1.5 : 0.0) - 0.5 * G[(size_t)k * L + j] : 0.0;
+            dmma884(c0, c1, a, b);
+        }
+        if (r < p) {
+            const int jc = j0 + 2 * q4;
+            if (jc < L) Xn[(size_t)r * L + jc] = c0;
+            if (jc + 1 < L) Xn[(size_t)r * L + jc + 1] = c1;
+        }
+    }
+}
+
+__global__ void __launch_bounds__(256) k_nsw_finish(const double* __restrict__ X0, const double* __restrict__ X1, long long n,
+                                                   const NsState* st, double* __restrict__ U, int* __restrict__ status) {
+    if (blockIdx.x == 0 && threadIdx.x == 0) status[0] = st->ok ? 0 : 1;
+    if (!st->ok) return;
+    const double* X = st->cur ? X1 : X0;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) U[i] = X[i];
+}
+
 }  // namespace
+
+size_t polar_wide_doubles(int p, int L) { return 2 * (size_t)p * L + (size_t)L * L + (sizeof(NsState) + 7) / 8; }
+
+cudaError_t launch_polar_wide(const double* A, int p, int L, double* U, double* work, int* status, bool* converged, int* launched,
+                              cudaStream_t st) {
+    constexpr int MAX_IT = 60, BATCH = 6;
+    const long long n = (long long)p * L;
+    double* X0 = work;
+    double* X1 = X0 + n;
+    double* G = X1 + n;
+    NsState* s = reinterpret_cast<NsState*>(G + (size_t)L * L);
+    auto grid_of = [](long long warps) { return (unsigned)std::max<long long>(1, std::min<long long>((warps + 7) / 8, 148LL * 8)); };
+    const long long ntl = (L + 7) / 8;
+    const unsigned g_gram = grid_of(ntl * ntl), g_mul = grid_of(((p + 7) / 8) * ntl);
+    const unsigned g_copy = (unsigned)std::min<long long>((n + 255) / 256, 148LL * 8);
+    k_nsw_start<<<g_copy, 256, 0, st>>>(A, n, X0, s);
+    k_nsw_gram<<<g_gram, 256, 0, st>>>(X0, X1, p, L, G, s, 0);
+    k_nsw_scale_ctl<<<1, 1, 0, st>>>(G, L, s);
+    k_nsw_scale<<<g_copy, 256, 0, st>>>(X0, n, s);
+    k_nsw_gram<<<g_gram, 256, 0, st>>>(X0, X1, p, L, G, s, 1);
+    *launched = 6;
+    for (int it0 = 0; it0 < MAX_IT; it0 += BATCH) {
+        for (int it = it0; it < it0 + BATCH && it < MAX_IT; ++it) {
+            k_nsw_ctl<<<1, 1, 0, st>>>(s, it);
+            k_nsw_mul<<<g_mul, 256, 0, st>>>(X0, X1, p, L, G, s);
+            k_nsw_gram<<<g_gram, 256, 0, st>>>(X0, X1, p, L, G, s, 0);
+            *launched += 3;
+        }
+        int active = 0;
+        cudaError_t e = cudaMemcpyAsync(&active, &s->active, sizeof(int), cudaMemcpyDeviceToHost, st);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+        if (e != cudaSuccess) return e;
+        if (!active) break;
+    }
+    k_nsw_finish<<<g_copy, 256, 0, st>>>(X0, X1, n, s, U, status);
+    int stat = 1;
+    cudaError_t e = cudaMemcpyAsync(&stat, status, sizeof(int), cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+    if (e != cudaSuccess) return e;
+    *converged = stat == 0;
+    return cudaGetLastError();
+}
 
 size_t polar_smem_bytes(int p, int L) {
     const size_t Lp = (size_t)((L + 1) & ~1);

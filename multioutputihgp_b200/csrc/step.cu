@@ -19,7 +19,8 @@ namespace {
 
 constexpr int ST = 128;
 
-// Ty for one observation.  Ty[L] (out) and sc[ls_scratch_doubles(L)] in shared memory.
+// Ty for one observation.  Ty[L] (out) in shared memory, sc[ls_scratch_doubles(L)] in shared memory or, where the kernel's
+// shared memory with it would pass 227 KB (k_step: L >= 120, k_lik: L >= 118), in global memory (StepArgs / LikArgs::ls_scratch).
 // Full observation: Ty = (S^-1/2 U') y (moihgp.h:181).  With NaNs: the least-squares projection on the observed rows
 // (ls_project.cuh), over the CTA.
 __device__ void project_one(const double* __restrict__ U, const double* __restrict__ S, const double* __restrict__ y, int p, int L,
@@ -53,8 +54,8 @@ __global__ void __launch_bounds__(ST) k_step(StepArgs a) {
     const int L = a.L, p = a.p, d = a.dim, tid = threadIdx.x;
     double* Ty = sm;                 // [L]
     double* Tyhat = Ty + L;          // [L]
-    double* sc = Tyhat + L;          // [ls_scratch_doubles(L)]
-    int* s_nmiss = (int*)(sc + ls_scratch_doubles(L));
+    double* sc = a.ls_scratch ? a.ls_scratch : Tyhat + L;                   // [ls_scratch_doubles(L)]
+    int* s_nmiss = (int*)(Tyhat + L + (a.ls_scratch ? 0 : ls_scratch_doubles(L)));
     if (a.y) project_one(a.U, a.S, a.y, p, L, Ty, sc, s_nmiss);
     for (int l = tid; l < L; l += ST) {
         const LatentConsts& c = a.consts[l];
@@ -101,8 +102,8 @@ __global__ void __launch_bounds__(ST) k_lik(LikArgs a) {
     double* li = pv + L;             // [L]   per-latent loss
     double* gi = li + L;             // [3L]  per-latent grads
     double* red = gi + 3 * L;        // [ST]
-    double* sc = red + ST;           // [ls_scratch_doubles(L)]
-    int* s_nmiss = (int*)(sc + ls_scratch_doubles(L));
+    double* sc = a.ls_scratch ? a.ls_scratch : red + ST;                    // [ls_scratch_doubles(L)]
+    int* s_nmiss = (int*)(red + ST + (a.ls_scratch ? 0 : ls_scratch_doubles(L)));
     project_one(a.U, a.S, a.y, p, L, Ty, sc, s_nmiss);
     for (int l = tid; l < L; l += ST) {
         double s = 0.0;
@@ -201,13 +202,22 @@ __global__ void __launch_bounds__(128) k_smooth_seq(const double* __restrict__ X
     }
 }
 
-size_t step_smem(int L) { return sizeof(double) * (2 * (size_t)L + ls_scratch_doubles(L)) + sizeof(int); }
-size_t lik_smem(int L) { return sizeof(double) * (7 * (size_t)L + ST + ls_scratch_doubles(L)) + sizeof(int); }
+size_t step_smem(int L, bool global_scratch) {
+    return sizeof(double) * (2 * (size_t)L + (global_scratch ? 0 : ls_scratch_doubles(L))) + sizeof(int);
+}
+size_t lik_smem(int L, bool global_scratch) {
+    return sizeof(double) * (7 * (size_t)L + ST + (global_scratch ? 0 : ls_scratch_doubles(L))) + sizeof(int);
+}
+constexpr size_t SMEM_MAX = 227 * 1024;     // dynamic shared memory of one CTA
 
 }  // namespace
 
+size_t step_global_doubles(int L) { return step_smem(L, false) <= SMEM_MAX ? 0 : (size_t)ls_scratch_doubles(L); }
+size_t lik_global_doubles(int L) { return lik_smem(L, false) <= SMEM_MAX ? 0 : (size_t)ls_scratch_doubles(L); }
+
 cudaError_t launch_step(const StepArgs& a, cudaStream_t st) {
-    const size_t smem = step_smem(a.L);
+    if ((step_global_doubles(a.L) != 0) != (a.ls_scratch != nullptr)) return cudaErrorInvalidValue;
+    const size_t smem = step_smem(a.L, a.ls_scratch != nullptr);
     if (smem > 48 * 1024) cudaFuncSetAttribute(k_step, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     k_step<<<1, ST, smem, st>>>(a);
     return cudaGetLastError();
@@ -300,7 +310,8 @@ cudaError_t launch_smooth_seq(const double* X, const LatentConsts* consts, int L
 }
 
 cudaError_t launch_lik(const LikArgs& a, cudaStream_t st) {
-    const size_t smem = lik_smem(a.L);
+    if ((lik_global_doubles(a.L) != 0) != (a.ls_scratch != nullptr)) return cudaErrorInvalidValue;
+    const size_t smem = lik_smem(a.L, a.ls_scratch != nullptr);
     if (smem > 48 * 1024) cudaFuncSetAttribute(k_lik, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     k_lik<<<1, ST, smem, st>>>(a);
     return cudaGetLastError();

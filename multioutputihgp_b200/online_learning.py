@@ -46,6 +46,8 @@ class MOIHGPOnlineLearning:
         self.ma = None
         self.dma = np.zeros((num_output,), dtype=np.float64)
         self._resident = self._seq.online_begin(self.windowsize)
+        if not self._resident and num_latent > 64:
+            raise ValueError("MOIHGPOnlineLearning: " + self._seq._lib.moihgp_cuda_last_error(self._seq._h).decode())
         if self._resident:
             self._seq.online_set_proximal(None)           # the proximal term stays here (hess_inv solve, as the reference's)
 
