@@ -191,6 +191,21 @@ int moihgp_cuda_sample_posterior(moihgp_handle* h, const double* Y, size_t N, si
                                  unsigned long long seed, double* Xs_mean, double* Xsamp, double* Fsamp, double* Ysamp);
 /* the sampler's factors LF, LC of latent l (lower-triangular, d x d row-major; either may be NULL) */
 int moihgp_cuda_sampler_consts(moihgp_handle* h, size_t l, double* LF, double* LC);
+/* The sampler on one contiguous BLOCK of a longer sequence sharded in time (DESIGN 4.8, 6).  DEVICE buffers, asynchronous on
+ * the handle's stream, capturable into a CUDA graph.  The block holds steps t0 .. t0 + T - 1 of the sequence (the Philox
+ * counter is the global step, so the draws are those of the whole-sequence call); seq_end = 1 on the block that ends it.
+ * Xs_mean [N][T][L][d] is the block's RTS mean: phase 3 of moihgp_cuda_fsn_block_async with smoother_mode = 1.  Two phases:
+ *   1  dev_out [S][N][L][d] = e at the block's first step from a zero e_end (from LF z on the block that ends the sequence).
+ *      Xs_mean may be NULL.
+ *      -> caller: all-gather dev_out of every block into gathered [G][S N][L][d], then this block's
+ *         e_end = moihgp_cuda_fsn_carry_dev(h, 1, 1, gathered, G, block_lengths, rank, S * N, NULL, e_end, NULL)
+ *         (the backward exchange of the RTS smoother: the layout [S][N][L][d] is [S N][L][d])
+ *   2  e_end [S][N][L][d] (NULL on the block that ends the sequence): Xsamp, Fsamp, Ysamp of the block, laid out as in
+ *      moihgp_cuda_sample_posterior_dev with T steps; any may be NULL, not all three.
+ * t0 + T <= 2^32 and S N < 2^32.  moihgp_cuda_set_path selects the variant as for the whole sequence. */
+int moihgp_cuda_sample_block_async(moihgp_handle* h, int phase, const double* Xs_mean, size_t N, size_t T, unsigned long long t0, int seq_end,
+                                   size_t S, unsigned long long seed, const double* e_end, double* Xsamp, double* Fsamp, double* Ysamp,
+                                   double* dev_out);
 
 /* RegressionObjective::operator() / OnlineObjective::operator() window loop over N sequences
  * (moihgp_regression.h:42-50, moihgp_online.h:61-70): loss = sum_n sum_t negLogLikelihood(x, y, dx, grad)

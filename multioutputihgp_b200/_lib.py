@@ -147,6 +147,9 @@ def load():
     for name in ("moihgp_cuda_nll_steps", "moihgp_cuda_nll_steps_dev"):
         getattr(lib, name).restype = ctypes.c_int
         getattr(lib, name).argtypes = [vp, vp, sz, sz, vp, vp, vp, vp]
+    lib.moihgp_cuda_sample_block_async.restype = ctypes.c_int
+    lib.moihgp_cuda_sample_block_async.argtypes = [vp, ctypes.c_int, vp, sz, sz, ctypes.c_uint64, ctypes.c_int, sz, ctypes.c_uint64, vp, vp, vp,
+                                                   vp, vp]
     lib.moihgp_cuda_sampler_consts.restype = ctypes.c_int
     lib.moihgp_cuda_sampler_consts.argtypes = [vp, sz, vp, vp]
     lib.moihgp_cuda_bind_data.restype = ctypes.c_int
@@ -164,5 +167,6 @@ CUDA_NAMES = ["create", "destroy", "set_stream", "sync", "last_error", "launch_c
               "num_igp_param", "update", "get_params", "get_U", "latent_consts", "latent_iters", "smoother_consts",
               "filter_smoother_nll", "filter_smoother_nll_values", "filter_smoother_nll_dev", "objective", "objective_dev", "bind_data", "objective_bound", "objective_begin_dev", "objective_finish_dev", "block_transition", "fsn_block_dev", "fsn_block_async", "fsn_carry_dev", "smoother_power", "smooth", "smooth_dev", "objective_begin_async", "carry_in_dev", "nan_status", "online_begin", "online_push", "online_set_proximal",
               "online_objective", "online_get_state", "sample_posterior", "sample_posterior_dev", "sampler_consts",
+              "sample_block_async",
               "nll_steps", "nll_steps_dev"]
 ALL_SYMBOLS = ["gp%s_%s" % (xx, n) for xx in ("32", "52") for n in LEGACY_NAMES] + ["moihgp_cuda_" + n for n in CUDA_NAMES]

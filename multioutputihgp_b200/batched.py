@@ -415,6 +415,23 @@ class MOIHGPSequences(object):
         self.set_stream(_torch_stream(Y.device))
         self._check(self._lib.moihgp_cuda_sample_posterior_dev(self._h, ptr[0], N, T, ptr[1], S, int(seed) & (2**64 - 1), *ptr[2:]))
 
+    def sample_block_async(self, phase, Xs_mean, num_samples, seed, t0, seq_end, e_end=None, Xsamp=None, Fsamp=None, Ysamp=None, out=None):
+        """One phase (1, 2) of the sampler on one block of a sequence sharded in time (torch CUDA tensors, asynchronous on
+        torch's current stream).  Xs_mean [N,T,L,d] is the block's RTS mean (fsn_block_async phase 3, smoother_mode 1), t0 the
+        global index of its first step.  Phase 1 writes e at the block's first step from a zero e_end to ``out`` [S,N,L,d];
+        phase 2 writes X [S,N,T,L,d], F [S,N,T,L] and / or Ysamp [S,N,T,p] from ``e_end`` [S,N,L,d] (None on the block that
+        ends the sequence).  Between the phases: fsn_carry_device(1, gathered [G,S*N,L,d], ..., smoother_mode=1)."""
+        where = "sample_block_async"
+        if getattr(Xs_mean, "ndim", None) != 4:
+            _refuse(where, "Xs_mean", "a [N,T,L,d] tensor", "shape %s" % (getattr(Xs_mean, "shape", type(Xs_mean).__name__),))
+        N, T = int(Xs_mean.shape[0]), int(Xs_mean.shape[1])
+        S, L, d, p = int(num_samples), self.num_latent, self.igp_dim, self.num_output
+        ptr = _dev(where, Xs_mean=(Xs_mean, N * T * L * d), e_end=(e_end, S * N * L * d), Xsamp=(Xsamp, S * N * T * L * d),
+                   Fsamp=(Fsamp, S * N * T * L), Ysamp=(Ysamp, S * N * T * p), out=(out, S * N * L * d))
+        self.set_stream(_torch_stream(Xs_mean.device))
+        self._check(self._lib.moihgp_cuda_sample_block_async(self._h, int(phase), ptr[0], N, T, int(t0), 1 if seq_end else 0, S,
+                                                             int(seed) & (2**64 - 1), *ptr[1:]))
+
     def sampler_consts(self, l):
         """(LF, LC) of latent l, [d,d] lower-triangular: LF LF' = PF, LC LC' = PF - G PPc G' (the sampler's noise factors)."""
         d = self.igp_dim

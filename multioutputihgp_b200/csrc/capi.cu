@@ -976,6 +976,40 @@ int moihgp_cuda_sample_posterior_dev(moihgp_handle* h, const double* Y, size_t N
     return 0;
 }
 
+int moihgp_cuda_sample_block_async(moihgp_handle* h, int phase, const double* Xs_mean, size_t N, size_t T, unsigned long long t0, int seq_end,
+                                   size_t S, unsigned long long seed, const double* e_end, double* Xsamp, double* Fsamp, double* Ysamp,
+                                   double* dev_out) {
+    if (!h) return -2;
+    if (phase < 1 || phase > 2) return fail(h, "sample_block: phase must be 1 or 2");
+    if (N == 0 || T == 0) return fail(h, "N and T must be positive");
+    if (S == 0) return fail(h, "sample_block: the number of samples S must be positive");
+    const unsigned long long lim = 1ull << 32;           // the Philox counter holds t0 + t, n and s in 32-bit words
+    if (t0 > lim || T > lim - t0) return fail(h, "sample_block: t0 + T must not exceed 2^32");
+    if (N >= lim || S >= lim || S * N >= lim) return fail(h, "sample_block: S * N must be below 2^32");
+    if (phase == 1 && !dev_out) return fail(h, "sample_block: phase 1 needs dev_out [S][N][L][d]");
+    if (phase == 2 && !(Xsamp || Fsamp || Ysamp)) return fail(h, "sample_block: no output requested (Xsamp, Fsamp and Ysamp are all NULL)");
+    if (phase == 2 && !Xs_mean) return fail(h, "sample_block: phase 2 needs Xs_mean [N][T][L][d]");
+    if (phase == 2 && !seq_end && !e_end) return fail(h, "sample_block: phase 2 of a block that does not end the sequence needs e_end");
+    DeviceGuard guard(h->device);
+    const int L = h->L, D = h->dim;
+    const long long chains = (long long)(S * N * L);
+    const bool chunked = sample_chunked((long long)T, chains, h->path);
+    SampleArgs a;
+    a.consts = h->d_consts; a.S = (long long)S; a.N = (long long)N; a.T = (long long)T; a.L = L; a.seed = seed;
+    a.Xs = Xs_mean; a.Xsamp = phase == 2 ? Xsamp : nullptr; a.F = phase == 2 ? Fsamp : nullptr; a.carry = nullptr;
+    a.mk = h->profiling ? &h->marker : nullptr;
+    if (phase == 2 && Ysamp && !Fsamp && ws_get(h, "sF", S * N * T * L, &a.F)) return -1;
+    if (chunked && ws_get(h, "scarry", sample_carry_doubles(D, (long long)T, chains), &a.carry)) return -1;
+    CK(launch_sample_block(D, phase, a, chunked, t0, seq_end, e_end, dev_out, h->stream));
+    h->launches += sample_block_launch_count(phase, chunked);
+    if (phase == 2 && Ysamp) {
+        CK(launch_backproject(a.F, h->d_U, h->d_S, h->p, L, 1, (long long)(S * N), (long long)T, Ysamp, h->stream));
+        h->launches += 1;
+        mark(a.mk, "k_backproject");
+    }
+    return 0;
+}
+
 int moihgp_cuda_sample_posterior(moihgp_handle* h, const double* Y, size_t N, size_t T, const double* x0, size_t S,
                                  unsigned long long seed, double* Xs_mean, double* Xsamp, double* Fsamp, double* Ysamp) {
     if (!h || !Y) return -2;

@@ -204,6 +204,11 @@ long long sample_chunk_len(long long T, long long chains);
 size_t sample_carry_doubles(int dim, long long T, long long chains);
 int sample_launch_count(bool chunked);
 cudaError_t launch_sample(int dim, const SampleArgs& a, bool chunked, cudaStream_t st);
+// one block of a sequence sharded in time: phase 1 leaves e at the block's first step from a zero e_end in e_start
+// [S N L][D]; phase 2 writes the paths from e_end (null on the block that ends the sequence).  t0: the block's first step
+int sample_block_launch_count(int phase, bool chunked);
+cudaError_t launch_sample_block(int dim, int phase, const SampleArgs& a, bool chunked, unsigned long long t0, int seq_end, const double* e_end,
+                                double* e_start, cudaStream_t st);
 
 // step.cu  (one observation per call: the legacy gpXX_* entry points)
 struct StepArgs {

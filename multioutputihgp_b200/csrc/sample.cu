@@ -16,6 +16,7 @@
 //   time-chunked k_sample<D, 1> runs every chunk of time backwards from a zero carry and keeps only its start value;
 //                k_sample_carry chains the chunk starts from the end of the sequence with G^len (binary powering on the
 //                powG[1] tables); k_sample<D, 2> runs every chunk again from its true carry and writes the outputs.
+//   k_sample_block: the same kernels on one block of a sequence sharded in time over several devices (DESIGN 4.8).
 #include <cuda_runtime.h>
 #include <curand_philox4x32_x.h>
 #include "launch.h"
@@ -60,11 +61,21 @@ __device__ __forceinline__ void step(const double* M, const double* Lo, const do
     for (int i = 0; i < D; ++i) e[i] = en[i];
 }
 
+// One block of a sequence sharded in time (moihgp_cuda_sample_block_async): t0 is the global index of its first step (the
+// Philox counter is t0 + t), seq_end says whether it ends the sequence, e_end [S N L][D] is e at the first step after it
+// (null: zero, the phase-1 start).  The whole sequence is {0, 1, null}.
+struct SampleBlock {
+    unsigned long long t0 = 0;
+    int seq_end = 1;
+    const double* e_end = nullptr;
+};
+
 // PHASE 0: one pass over the whole sequence, outputs written.  PHASE 1: chunk from a zero carry, start value -> carry.
 // PHASE 2: chunk from its true carry (carry[c + 1]), outputs written.  Thread index = chunk * chains + chain,
 // chain = (s N + n) L + l, so that the lanes of a warp write neighbouring latents of one state row.
-template <int D, int PHASE>
-__global__ void __launch_bounds__(kThreads) k_sample(const SampleArgs a, long long chunk_len, long long nC) {
+// BLOCK: the call covers one block of the sequence (b); false compiles the whole-sequence kernels, which ignore b.
+template <int D, int PHASE, bool BLOCK>
+__device__ __forceinline__ void sample_chunk(const SampleArgs& a, long long chunk_len, long long nC, const SampleBlock& b) {
     const long long chains = a.S * a.N * a.L;
     const long long id = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (id >= chains * nC) return;
@@ -98,15 +109,19 @@ __global__ void __launch_bounds__(kThreads) k_sample(const SampleArgs a, long lo
             fo[t * a.L] = xs[t * stride] + e[0];
         }
     };
+    const unsigned t0 = BLOCK ? (unsigned)b.t0 : 0u;             // t0 + t < 2^32 (moihgp_cuda_sample_block_async)
     long long t = t_hi - 1;
-    if (t_hi == a.T) {                                           // the end of the sequence: e = LF z
-        normals<D>(key, (unsigned)s, (unsigned)n, (unsigned)l, (unsigned)t, z);
+    if (t_hi == a.T && (!BLOCK || b.seq_end)) {                  // the end of the sequence: e = LF z
+        normals<D>(key, (unsigned)s, (unsigned)n, (unsigned)l, t0 + (unsigned)t, z);
 #pragma unroll
         for (int i = 0; i < D; ++i) e[i] = 0.0;
         step<D>(G, LF, z, e);
         emit(t);
         --t;
-    } else if (PHASE == 1) {
+    } else if (BLOCK && t_hi == a.T && b.e_end) {                // the block's last step: e_end from the next block
+#pragma unroll
+        for (int i = 0; i < D; ++i) e[i] = b.e_end[chain * D + i];
+    } else if (PHASE == 1 || (BLOCK && t_hi == a.T)) {
 #pragma unroll
         for (int i = 0; i < D; ++i) e[i] = 0.0;
     } else {
@@ -116,7 +131,7 @@ __global__ void __launch_bounds__(kThreads) k_sample(const SampleArgs a, long lo
     }
 #pragma unroll 2
     for (; t >= t_lo; --t) {
-        normals<D>(key, (unsigned)s, (unsigned)n, (unsigned)l, (unsigned)t, z);
+        normals<D>(key, (unsigned)s, (unsigned)n, (unsigned)l, t0 + (unsigned)t, z);
         step<D>(G, LC, z, e);
         emit(t);
     }
@@ -125,6 +140,16 @@ __global__ void __launch_bounds__(kThreads) k_sample(const SampleArgs a, long lo
 #pragma unroll
         for (int i = 0; i < D; ++i) co[i] = e[i];
     }
+}
+
+template <int D, int PHASE>
+__global__ void __launch_bounds__(kThreads) k_sample(const SampleArgs a, long long chunk_len, long long nC) {
+    sample_chunk<D, PHASE, false>(a, chunk_len, nC, SampleBlock{});
+}
+
+template <int D, int PHASE>
+__global__ void __launch_bounds__(kThreads) k_sample_block(const SampleArgs a, long long chunk_len, long long nC, const SampleBlock b) {
+    sample_chunk<D, PHASE, true>(a, chunk_len, nC, b);
 }
 
 // carry[c][chain] <- e at the start of chunk c:  E(nC-1) = carry(nC-1),  E(c) = carry(c) + G^chunk_len E(c+1).
@@ -186,6 +211,38 @@ cudaError_t run_sample(const SampleArgs& a, bool chunked, cudaStream_t st) {
     return cudaGetLastError();
 }
 
+// One block of a sharded sequence.  Phase 1: e at the block's first step from a zero e_end -> e_start [S N L][D] (one pass:
+// a walk with no stores; chunked: the chain's chunk-0 value).  Phase 2: the paths, the last chunk starting from b.e_end
+// (LF z on the block that ends the sequence).
+template <int D>
+cudaError_t run_sample_block(int phase, SampleArgs a, bool chunked, SampleBlock b, double* e_start, cudaStream_t st) {
+    const long long chains = a.S * a.N * a.L;
+    if (phase == 1) b.e_end = nullptr;
+    if (!chunked) {
+        if (phase == 1) {
+            a.carry = e_start;
+            k_sample_block<D, 1><<<blocks(chains), kThreads, 0, st>>>(a, a.T, 1, b);
+        } else {
+            k_sample_block<D, 0><<<blocks(chains), kThreads, 0, st>>>(a, a.T, 1, b);
+        }
+        mark(a.mk, "k_sample_block");
+        return cudaGetLastError();
+    }
+    const long long cl = sample_chunk_len(a.T, chains), nC = (a.T + cl - 1) / cl;
+    k_sample_block<D, 1><<<blocks(chains * nC), kThreads, 0, st>>>(a, cl, nC, b);
+    mark(a.mk, "k_sample_block_chunks");
+    k_sample_carry<D><<<blocks(chains), kThreads, 0, st>>>(a, cl, nC);
+    mark(a.mk, "k_sample_carry");
+    if (phase == 1) {
+        const cudaError_t e = cudaMemcpyAsync(e_start, a.carry, sizeof(double) * chains * D, cudaMemcpyDeviceToDevice, st);
+        if (e != cudaSuccess) return e;
+    } else {
+        k_sample_block<D, 2><<<blocks(chains * nC), kThreads, 0, st>>>(a, cl, nC, b);
+        mark(a.mk, "k_sample_block_final");
+    }
+    return cudaGetLastError();
+}
+
 }  // namespace
 
 // One pass as soon as the chains alone give every SM eight warps: with fewer, the one-pass loop cannot hide its fp64
@@ -212,6 +269,15 @@ int sample_launch_count(bool chunked) { return chunked ? 3 : 1; }
 
 cudaError_t launch_sample(int dim, const SampleArgs& a, bool chunked, cudaStream_t st) {
     return dim == 3 ? run_sample<3>(a, chunked, st) : run_sample<2>(a, chunked, st);
+}
+
+int sample_block_launch_count(int phase, bool chunked) { return chunked ? (phase == 1 ? 2 : 3) : 1; }
+
+cudaError_t launch_sample_block(int dim, int phase, const SampleArgs& a, bool chunked, unsigned long long t0, int seq_end, const double* e_end,
+                                double* e_start, cudaStream_t st) {
+    SampleBlock b;
+    b.t0 = t0; b.seq_end = seq_end ? 1 : 0; b.e_end = e_end;
+    return dim == 3 ? run_sample_block<3>(phase, a, chunked, b, e_start, st) : run_sample_block<2>(phase, a, chunked, b, e_start, st);
 }
 
 }  // namespace moihgp

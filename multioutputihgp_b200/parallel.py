@@ -412,3 +412,56 @@ class TimeShardedFilterSmoother(object):
         if multi:
             dist.all_reduce(nll_dev, op=dist.ReduceOp.SUM, group=self.group)
         return nll_dev.cpu().numpy()
+
+
+class TimeShardedPosteriorSampler(object):
+    """Posterior sample paths of ONE long sequence (or N of them) whose contiguous time blocks live on different ranks
+    (DESIGN 4.8, 6): the RTS mean by ``TimeShardedFilterSmoother`` (smoother_mode 1), then the sampler's noise process, whose
+    backward exchange is the RTS smoother's with N -> S N: every rank runs its block from a zero carry (sampler phase 1),
+    all-gathers the S N L d start values, forms its carry from the right with ``fsn_carry_device(1, ..., smoother_mode=1)``
+    and draws its block (phase 2).  The draws equal those of the whole-sequence call with the same seed: the random numbers
+    are indexed by the global step.  ``model`` provides the ``TimeShardedFilterSmoother`` interface and ``sample_block_async``
+    (``MOIHGPSequences``); every block but the last holds a multiple of 256 steps (``time_block_bounds_aligned``)."""
+
+    def __init__(self, model, block_lengths, group=None, device=None):
+        import torch
+        self.model, self.group = model, group
+        self.block_lengths = [int(b) for b in block_lengths]
+        self.dev = device if device is not None else torch.device("cuda", torch.cuda.current_device())
+        self.mean = TimeShardedFilterSmoother(model, self.block_lengths, 1, group=group, device=self.dev)
+
+    def _buffers(self, N, n, S):
+        import torch
+        if getattr(self, "_shape", None) != (N, n, S):
+            L, d, G = self.model.num_latent, self.model.igp_dim, len(self.block_lengths)
+            f64 = dict(dtype=torch.float64, device=self.dev)
+            self._X, self._Xs = torch.zeros((N, n, L, d), **f64), torch.zeros((N, n, L, d), **f64)
+            self._e1, self._eg, self._eend = (torch.zeros(s, **f64) for s in ((S * N, L, d), (G, S * N, L, d), (S * N, L, d)))
+            self._shape = (N, n, S)
+        return self
+
+    def enqueue(self, Y_block, num_samples, seed, Xsamp=None, Fsamp=None, Ysamp=None, x0=None, Xs_mean=None):
+        """Queue the whole exchange on torch's current stream with NO host round trip: the time-sharded RTS pass into
+        ``Xs_mean`` [N,n,L,d] (a workspace when None) -> sampler phase 1 -> all-gather -> backward carry kernel -> sampler
+        phase 2 into Xsamp [S,N,n,L,d], Fsamp [S,N,n,L], Ysamp [S,N,n,p] (this rank's block; at least one).  x0 [N,L,d]: the
+        state before the first step of the WHOLE sequence or None.  Returns the tensor holding the RTS mean."""
+        dist = _dist()
+        m = self.model
+        N, n, S = int(Y_block.shape[0]), int(Y_block.shape[1]), int(num_samples)
+        multi = dist.is_available() and dist.is_initialized() and dist.get_world_size(self.group) > 1
+        world = dist.get_world_size(self.group) if multi else 1
+        rank = dist.get_rank(self.group) if multi else 0
+        last = rank == world - 1
+        b = self._buffers(N, n, S)
+        Xs = Xs_mean if Xs_mean is not None else b._Xs
+        self.mean.enqueue(Y_block, b._X, Xs, x0=x0)
+        outs = dict(Xsamp=Xsamp, Fsamp=Fsamp, Ysamp=Ysamp)
+        if not multi:
+            m.sample_block_async(2, Xs, S, seed, 0, True, **outs)
+            return Xs
+        t0 = sum(self.block_lengths[:rank])
+        m.sample_block_async(1, Xs, S, seed, t0, last, out=b._e1)
+        self.mean._all_gather(b._eg, b._e1)
+        m.fsn_carry_device(1, b._eg, self.block_lengths, rank, b._eend, smoother_mode=1)
+        m.sample_block_async(2, Xs, S, seed, t0, last, e_end=None if last else b._eend, **outs)
+        return Xs
