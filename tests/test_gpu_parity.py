@@ -1014,7 +1014,8 @@ def test_objective_kernels_agree(cuda_lib, kernel, p, L, N, T):
 @pytest.mark.parametrize("kernel", ["Matern32", "Matern52"])
 def test_block_transition_matches_the_host_powering(cuda_lib, kernel):
     """moihgp_cuda_block_transition (binary powering on the library's power tables) against parallel.block_transition
-    (numpy, from AKHA and dAKHA alone) and against the brute-force sum for a short block."""
+    (numpy, from AKHA and dAKHA alone) and against the brute-force sum for a short block; with slowly forgetting latents,
+    block_transition and smoother_power against mpmath at n = 256 ... 10^6."""
     from multioutputihgp_b200 import MOIHGPSequences
     from multioutputihgp_b200.parallel import block_transition, stack_consts
     from oracle.gen_golden import make_params
@@ -1034,6 +1035,27 @@ def test_block_transition_matches_the_host_powering(cuda_lib, kernel):
         for k in range(3):
             brute = sum(np.linalg.matrix_power(M, 4 - i) @ dAK[l, k] @ np.linalg.matrix_power(M, i) for i in range(5))
             assert rel_err(E5[l, k], brute) < 1e-12
+    # On the table above every power from n = 256 on is below rounding.  With slowly forgetting latents M^n, E_k(n) and the
+    # RTS gain's G^n stay of order one and larger at these spans: compare them with mpmath, every latent on its own scale.
+    from test_gpu_long_memory import CH, GROUP, OBJ_GROUP, SLOW, SUPER, _Powers, _f64, _mp, assert_regime, per_step_err
+    L = 5
+    m = MOIHGPSequences(0.1, p, L, kernel, True)
+    m.update(make_params(rng, p, L, kernel, SLOW))
+    consts = [m.latent_consts(l) for l in range(L)]
+    Grts = [m.smoother_consts(l, 1)[0] for l in range(L)]
+    assert_regime(kernel, consts, Grts)
+    d = m.igp_dim
+    for n in (CH, GROUP, OBJ_GROUP, SUPER, 10 ** 6):
+        P, E = m.block_transition(n)
+        Gn = m.smoother_power(n, 1)
+        for l in range(L):
+            c = consts[l]
+            same = lambda a, b: per_step_err(a.reshape(1, -1), b.reshape(1, -1)) < TOL     # the whole matrix on its own scale
+            assert same(P[l], _f64(_Powers(c["AKHA"]).apply(n, _mp(np.eye(d))))), (n, l)
+            assert same(Gn[l], _f64(_Powers(Grts[l]).apply(n, _mp(np.eye(d))))), (n, l)
+            for k in range(3):
+                Z = np.block([[c["AKHA"], c["dAKHA%d" % k]], [np.zeros((d, d)), c["AKHA"]]])
+                assert same(E[l, k], _f64(_Powers(Z).apply(n, _mp(np.eye(2 * d))))[:d, d:]), (n, l, k)
 
 
 @pytest.mark.gpu
