@@ -257,7 +257,8 @@ int moihgp_cuda_objective_finish_dev(moihgp_handle* h, const double* Y, size_t N
  *   begin_async : like begin, the end state goes to DEVICE memory zend_dev[N][L][4][d] (NULL on the last block)
  *   carry_in_dev: ends_dev[G][N][L][4][d] = every block's end state (all-gathered); block `rank`'s true carry-in
  *                 z_in(g+1) = T(n_g) z_in(g) + ends_g, chained over g < rank from (x0, dx0) (device, NULL = zeros), is
- *                 written to xin_dev[N][L][d], dxin_dev[N][L][3][d] - pass them to finish_dev.  block_lengths: G host values. */
+ *                 written to xin_dev[N][L][d], dxin_dev[N][L][3][d] - pass them to finish_dev.  block_lengths: G host values,
+ *                 at most 64 blocks. */
 int moihgp_cuda_objective_begin_async(moihgp_handle* h, const double* Y, size_t N, size_t T, double* zend_dev);
 int moihgp_cuda_carry_in_dev(moihgp_handle* h, const double* ends_dev, size_t G, const long long* block_lengths, size_t rank, size_t N,
                              const double* x0_dev, const double* dx0_dev, double* xin_dev, double* dxin_dev);
@@ -292,7 +293,8 @@ int moihgp_cuda_fsn_block_dev(moihgp_handle* h, int phase, const double* Y, size
  *                    block's first projected observation (untouched on the last block);
  *                    direction 1 (after phase 2): gathered_dev[G][N][L][d] -> out_dev[N][L][d] = this block's b_end
  *                    (untouched on the last block).  The arithmetic of moihgp_cuda_block_transition /
- *                    moihgp_cuda_smoother_power in a one-thread-per-(sequence, latent) kernel.  block_lengths: G host values. */
+ *                    moihgp_cuda_smoother_power in the one-thread-per-(sequence, latent) kernel of carry_in_dev.
+ *                    block_lengths: G host values, G <= 64 as for carry_in_dev. */
 int moihgp_cuda_fsn_block_async(moihgp_handle* h, int phase, const double* Y, size_t N, size_t T, int seq_end, int smoother_mode,
                                 const double* x0, const double* u_after, const double* b_end, double* X, double* Xs, double* nll,
                                 double* xT, double* dev_out);

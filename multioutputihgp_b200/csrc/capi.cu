@@ -718,37 +718,31 @@ static int fsn_block_impl(moihgp_handle* h, int phase, const double* Y, size_t N
     if (phase == 3 && Xs && !X) return fail(h, "Xs needs X");
     DeviceGuard guard(h->device);
     const int L = h->L, D = h->dim;
-    double *xe, *bo;
-    if (ws_get(h, "blk_xe", N * L * D, &xe) || ws_get(h, "blk_bo", N * L * D, &bo)) return -1;
+    // phases 1 and 2 leave their output in dev_out, or in a workspace that host_out is copied from
+    double *xe, *out = dev_out;
+    if (ws_get(h, "blk_xe", N * L * D, &xe) || (phase < 3 && !out && ws_get(h, "blk_out", N * L * (D + 1), &out))) return -1;
     ScanArgs a{};
     a.N = (long long)N; a.T = (long long)T; a.x0 = x0;
     a.X = phase == 3 ? X : nullptr; a.Xs = phase == 3 ? Xs : nullptr; a.xT = phase == 3 ? xT : nullptr;
     a.phase = phase; a.seq_end = seq_end ? 1 : 0; a.u_after = seq_end ? nullptr : u_after; a.b_end = phase == 3 ? b_end : nullptr;
-    a.x_end = phase == 1 ? xe : nullptr; a.b_out = phase == 2 ? bo : nullptr;
+    a.x_end = phase == 1 ? xe : nullptr; a.b_out = phase == 2 ? out : nullptr;
     if (const int rc = scan_pass(h, Y, mode, nll, a)) return rc;
-    const double* u = a.u;
-    if (phase == 1 && host_out) {
+    if (phase == 1) {
         // [N][L][D + 1]: the block's end state from x0, then its first projected observation (the previous block's u_after)
-        std::vector<double> hx(N * L * D), hu(N * L);
-        CK(cudaMemcpyAsync(hx.data(), xe, sizeof(double) * N * L * D, cudaMemcpyDeviceToHost, h->stream));
-        CK(cudaMemcpy2DAsync(hu.data(), sizeof(double), u, sizeof(double) * T, sizeof(double), N * L, cudaMemcpyDeviceToHost, h->stream));
-        CK(cudaStreamSynchronize(h->stream));
-        for (size_t i = 0; i < N * L; ++i) {
-            for (int q = 0; q < D; ++q) host_out[i * (D + 1) + q] = hx[i * D + q];
-            host_out[i * (D + 1) + D] = hu[i];
-        }
+        CK(cudaMemcpy2DAsync(out, sizeof(double) * (D + 1), xe, sizeof(double) * D, sizeof(double) * D, N * L, cudaMemcpyDeviceToDevice, h->stream));
+        CK(cudaMemcpy2DAsync(out + D, sizeof(double) * (D + 1), a.u, sizeof(double) * T, sizeof(double), N * L, cudaMemcpyDeviceToDevice, h->stream));
     }
-    if (phase == 2 && host_out) {
-        CK(cudaMemcpyAsync(host_out, bo, sizeof(double) * N * L * D, cudaMemcpyDeviceToHost, h->stream));
+    if (phase < 3 && host_out) {
+        CK(cudaMemcpyAsync(host_out, out, sizeof(double) * N * L * (phase == 1 ? D + 1 : D), cudaMemcpyDeviceToHost, h->stream));
         CK(cudaStreamSynchronize(h->stream));
     }
-    // the same values left in DEVICE memory, asynchronously on the handle's stream (no host round trip: the caller's
-    // all-gather - NCCL on the same stream - follows directly)
-    if (phase == 1 && dev_out) {
-        CK(cudaMemcpy2DAsync(dev_out, sizeof(double) * (D + 1), xe, sizeof(double) * D, sizeof(double) * D, N * L, cudaMemcpyDeviceToDevice, h->stream));
-        CK(cudaMemcpy2DAsync(dev_out + D, sizeof(double) * (D + 1), u, sizeof(double) * T, sizeof(double), N * L, cudaMemcpyDeviceToDevice, h->stream));
-    }
-    if (phase == 2 && dev_out) CK(cudaMemcpyAsync(dev_out, bo, sizeof(double) * N * L * D, cudaMemcpyDeviceToDevice, h->stream));
+    return 0;
+}
+
+// The carry kernel of the time-sharded passes takes the block lengths by value (launch_block_carry)
+static int check_time_blocks(moihgp_handle* h, size_t G, size_t rank) {
+    if (G == 0 || G > (size_t)MAX_TIME_BLOCKS || rank >= G)
+        return fail(h, "need 1 <= G <= " + std::to_string(MAX_TIME_BLOCKS) + " time blocks and rank < G");
     return 0;
 }
 
@@ -769,10 +763,10 @@ int moihgp_cuda_fsn_carry_dev(moihgp_handle* h, int direction, int mode, const d
     if (!h || !gathered_dev || !block_lengths || !out_dev) return -2;
     if (direction < 0 || direction > 1) return fail(h, "direction must be 0 (forward) or 1 (backward)");
     if (mode < 0 || mode > 1) return fail(h, "smoother_mode must be 0 or 1");
-    if (G == 0 || G > 64 || rank >= G) return fail(h, "need 1 <= G <= 64 blocks and rank < G");
+    if (const int rc = check_time_blocks(h, G, rank)) return rc;
     DeviceGuard guard(h->device);
-    CK(launch_fsn_carry(h->dim, direction, mode, h->d_consts, h->L, (long long)N, (int)rank, (int)G, block_lengths, gathered_dev, x0_dev, out_dev,
-                        u_after_dev, h->stream));
+    CK(launch_block_carry(h->dim, direction, mode, h->d_consts, h->L, (long long)N, (int)rank, (int)G, block_lengths, gathered_dev, x0_dev,
+                          nullptr, out_dev, nullptr, u_after_dev, h->stream));
     h->launches += 1;
     return 0;
 }
@@ -1102,9 +1096,10 @@ int moihgp_cuda_objective_begin_async(moihgp_handle* h, const double* Y, size_t 
 int moihgp_cuda_carry_in_dev(moihgp_handle* h, const double* ends_dev, size_t G, const long long* block_lengths, size_t rank, size_t N,
                              const double* x0_dev, const double* dx0_dev, double* xin_dev, double* dxin_dev) {
     if (!h || !xin_dev || !dxin_dev || (rank > 0 && (!ends_dev || !block_lengths))) return -2;
-    if (rank >= G || G > 64) return fail(h, "carry_in: need rank < G <= 64 blocks");
+    if (const int rc = check_time_blocks(h, G, rank)) return rc;
     DeviceGuard guard(h->device);
-    CK(launch_block_carry(h->dim, h->d_consts, h->L, (long long)N, (int)rank, block_lengths, ends_dev, x0_dev, dx0_dev, xin_dev, dxin_dev, h->stream));
+    CK(launch_block_carry(h->dim, 0, 0, h->d_consts, h->L, (long long)N, (int)rank, (int)G, block_lengths, ends_dev, x0_dev, dx0_dev, xin_dev,
+                          dxin_dev, nullptr, h->stream));
     h->launches += 1;
     return 0;
 }

@@ -122,6 +122,15 @@ cudaError_t launch_nll_steps(const double* vstep, const LatentConsts* consts, co
                              long long T, double* nll_steps, cudaStream_t st);
 cudaError_t launch_nll_reduce(const double* rho_part, const double* vsq, const LatentConsts* consts, const double* S, double sigma,
                               int p, int L, long long N, long long T, double* part, double* nll, cudaStream_t st);
+// One long sequence sharded in time over at most MAX_TIME_BLOCKS blocks (the block lengths travel by value in the launch
+// parameters; the entry points check G): the carry of block `rank` from every block's output from a zero carry, gathered
+// [G][N][L][W].  dxout == null: the filter + smoother exchanges, direction 0 -> x_in (out) and u_after from
+// [x_end | u_first] records (W = D + 1), direction 1 -> b_end (out) from the blocks' first backward values (W = D, powers of
+// G[mode]); dxout != null: the objective's carry-in (direction 0) from the end states [x; dx_0..2] (W = 4 D) -> out, dxout.
+constexpr int MAX_TIME_BLOCKS = 64;
+cudaError_t launch_block_carry(int dim, int direction, int mode, const LatentConsts* consts, int L, long long N, int rank, int G,
+                               const long long* block_lengths, const double* gathered, const double* x0, const double* dx0, double* out,
+                               double* dxout, double* u_after, cudaStream_t st);
 
 // chain.cu  (many-chains path: thread per (sequence, latent), sequential in time)
 struct ChainArgs {
@@ -170,14 +179,6 @@ size_t obj_chunks(long long T);
 size_t obj_gu_splits(long long N, long long T);
 int obj_launch_count(long long T, int L);
 cudaError_t launch_objective(int dim, const ObjArgs& a, cudaStream_t st);
-// carry-in of time block `rank` from the gathered block ends (device arithmetic of moihgp_cuda_block_transition)
-cudaError_t launch_block_carry(int dim, const LatentConsts* consts, int L, long long N, int rank, const long long* block_lengths,
-                               const double* ends /*[G][N][L][4][D]*/, const double* x0, const double* dx0, double* xin, double* dxin,
-                               cudaStream_t st);
-// the two carry exchanges of the time-sharded filter + smoother pass on the device (scan.cu)
-cudaError_t launch_fsn_carry(int dim, int direction, int mode, const LatentConsts* consts, int L, long long N, int rank, int G,
-                             const long long* block_lengths, const double* gathered, const double* x0, double* out, double* u_after,
-                             cudaStream_t st);
 size_t obj_small_smem(int p, int L, long long T);
 cudaError_t launch_objective_small(int dim, const double* Y, const double* U, const double* S, double sigma, const LatentConsts* consts,
                                    int p, int L, long long T, int threading, const double* x0, const double* dx0, double* out, double* xT,

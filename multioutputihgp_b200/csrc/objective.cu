@@ -1254,76 +1254,4 @@ cudaError_t launch_objective(int dim, const ObjArgs& a, cudaStream_t st) {
     return dim == 2 ? run_objective<2>(a, st) : run_objective<3>(a, st);
 }
 
-// ---- one long sequence sharded in TIME over several devices: the carry-in of a block from the gathered block ends ----
-// ends[g][n][l][4][D] = end state [x; dx_0; dx_1; dx_2] of block g from a ZERO carry-in (k_obj_block_end).  Block `rank`
-// starts from  z_in(g+1) = T(n_g) z_in(g) + ends_g  chained over g < rank, with T(n): x -> M^n x, dx_k -> M^n dx_k + E_k(n) x,
-// M = AKHA, E_k(n) = sum_i M^(n-1-i) dAKHA_k M^i (block_transition, as moihgp_cuda_block_transition) - on the device, so
-// that begin -> all-gather -> finish needs no host round trip.  One thread per (sequence, latent).
-struct BlockLens { long long n[64]; };
-
-template <int D>
-__global__ void __launch_bounds__(128) k_block_carry(const LatentConsts* __restrict__ consts, int L, long long N, int rank, BlockLens lens,
-                                                    const double* __restrict__ ends, const double* __restrict__ x0,
-                                                    const double* __restrict__ dx0, double* __restrict__ xin, double* __restrict__ dxin) {
-    const long long id = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (id >= N * L) return;
-    const int l = (int)(id % L);
-    const LatentConsts& c = consts[l];
-    double x[D], dx[3][D];
-#pragma unroll
-    for (int q = 0; q < D; ++q) {
-        x[q] = x0 ? x0[id * D + q] : 0.0;
-#pragma unroll
-        for (int k = 0; k < 3; ++k) dx[k][q] = dx0 ? dx0[(id * 3 + k) * D + q] : 0.0;
-    }
-    double P[D * D], E[3][D * D];
-    long long have = -1;
-    for (int g = 0; g < rank; ++g) {
-        const long long n = lens.n[g];
-        if (n != have) {
-            block_transition<D>(c, n, P, E);
-            have = n;
-        }
-        const double* e = ends + ((size_t)g * N * L + id) * 4 * D;
-        double xn[D], dxn[3][D];
-#pragma unroll
-        for (int i = 0; i < D; ++i) {
-            double s = 0.0;
-#pragma unroll
-            for (int q = 0; q < D; ++q) s += P[i * D + q] * x[q];
-            xn[i] = s + e[i];
-#pragma unroll
-            for (int k = 0; k < 3; ++k) {
-                double a = 0.0, b = 0.0;
-#pragma unroll
-                for (int q = 0; q < D; ++q) { a += P[i * D + q] * dx[k][q]; b += E[k][i * D + q] * x[q]; }
-                dxn[k][i] = a + b + e[(1 + k) * D + i];
-            }
-        }
-#pragma unroll
-        for (int i = 0; i < D; ++i) {
-            x[i] = xn[i];
-#pragma unroll
-            for (int k = 0; k < 3; ++k) dx[k][i] = dxn[k][i];
-        }
-    }
-#pragma unroll
-    for (int q = 0; q < D; ++q) {
-        xin[id * D + q] = x[q];
-#pragma unroll
-        for (int k = 0; k < 3; ++k) dxin[(id * 3 + k) * D + q] = dx[k][q];
-    }
-}
-
-cudaError_t launch_block_carry(int dim, const LatentConsts* consts, int L, long long N, int rank, const long long* block_lengths,
-                               const double* ends, const double* x0, const double* dx0, double* xin, double* dxin, cudaStream_t st) {
-    if (rank < 0 || rank > 64) return cudaErrorInvalidValue;
-    BlockLens lens;
-    for (int g = 0; g < 64; ++g) lens.n[g] = g < rank ? block_lengths[g] : 0;
-    const unsigned grid = (unsigned)((N * L + 127) / 128);
-    if (dim == 3) k_block_carry<3><<<grid, 128, 0, st>>>(consts, L, N, rank, lens, ends, x0, dx0, xin, dxin);
-    else k_block_carry<2><<<grid, 128, 0, st>>>(consts, L, N, rank, lens, ends, x0, dx0, xin, dxin);
-    return cudaGetLastError();
-}
-
 }  // namespace moihgp

@@ -1220,87 +1220,100 @@ cudaError_t launch_nll_steps(const double* vstep, const LatentConsts* consts, co
     return cudaGetLastError();
 }
 
-// ---- one long sequence sharded in TIME (moihgp_cuda_fsn_block_*): the two carry exchanges on the device ----------------
-// forward  (DIR 0): gathered[g][n][l][D + 1] = [end state of block g from a zero carry-in | first projected observation of g];
-//                   x_in(g+1) = AKHA^n_g x_in(g) + x_end_g chained over g < rank from x0 -> out[n][l][D];
-//                   u_after[n][l] = first observation of block rank + 1 (untouched on the last block)
-// backward (DIR 1): gathered[g][n][l][D] = backward value at block g's first step from a ZERO b_end;
-//                   b_start(G-1) = gathered[G-1], b_start(g) = gathered[g] + G^n_g b_start(g+1); out = b_start(rank + 1)
-//                   (untouched on the last block, whose b_end is not used)
-// Powers by binary powering on the latent's 2^k tables (mat_pow).  One thread per (sequence, latent) - the arithmetic of
-// parallel.forward_carry_in / backward_carry_in.
-struct FsnBlockLens { long long n[64]; };
+// ---- one long sequence sharded in TIME over several devices: the carry of a block across the blocks before or after it ----
+// gathered[g][n][l][W] holds what block g computed from a ZERO carry; one thread per (sequence, latent) chains the blocks
+// with their transitions, taken by binary powering on the latent's 2^k tables, so that the exchanges stay on the device:
+// forward  (dir 0, K = 0): gathered = [end state of block g | first projected observation of g], W = D + 1;
+//                          x_in(g+1) = AKHA^n_g x_in(g) + x_end_g chained over g < rank from x0 -> out[n][l][D];
+//                          u_after[n][l] = first observation of block rank + 1 (untouched on the last block)
+//                          (moihgp_cuda_fsn_carry_dev, parallel.forward_carry_in)
+// backward (dir 1, K = 0): gathered = backward value at block g's first step from a ZERO b_end, W = D;
+//                          b_start(G-1) = gathered[G-1], b_start(g) = gathered[g] + G^n_g b_start(g+1); out = b_start(rank + 1)
+//                          (untouched on the last block, whose b_end is not used) (parallel.backward_carry_in)
+// objective (dir 0, K = 3): gathered = end state [x; dx_0; dx_1; dx_2] of block g (k_obj_block_end), W = 4 D;
+//                          z_in(g+1) = T(n_g) z_in(g) + ends_g chained over g < rank from (x0, dx0), with
+//                          T(n): x -> M^n x, dx_k -> M^n dx_k + E_k(n) x (block_transition) -> out, dxout[n][l][3][D]
+//                          (moihgp_cuda_carry_in_dev, parallel.carry_in_from_block_ends)
+struct BlockLens { long long n[MAX_TIME_BLOCKS]; };
 
-template <int D>
-__global__ void __launch_bounds__(128) k_fsn_carry(const LatentConsts* __restrict__ consts, int L, long long N, int rank, int G, int dir, int mode,
-                                                  FsnBlockLens lens, const double* __restrict__ gathered, const double* __restrict__ x0,
-                                                  double* __restrict__ out, double* __restrict__ u_after) {
+template <int D, int K>
+__global__ void __launch_bounds__(128) k_block_carry(const LatentConsts* __restrict__ consts, int L, long long N, int rank, int G, int dir,
+                                                    int mode, BlockLens lens, const double* __restrict__ gathered,
+                                                    const double* __restrict__ x0, const double* __restrict__ dx0,
+                                                    double* __restrict__ out, double* __restrict__ dxout, double* __restrict__ u_after) {
+    static_assert(K == 0 || K == 3, "no derivative chains, or the objective's three");
+    constexpr int KD = K > 0 ? K : 1;
     const long long id = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (id >= N * L) return;
+    if (dir == 1 && rank >= G - 1) return;
     const LatentConsts& c = consts[id % L];
-    const double (*tab)[9] = dir == 0 ? c.powM : c.powG[mode];  // M = AKHA (forward) or G[mode] (backward)
-    double P[D * D];
-    long long have = -1;
-    auto power = [&](long long n) {                       // P = M^n
-        if (n == have) return;
-        mat_pow<D>(tab, n, P);
-        have = n;
-    };
-    double v[D];
+    const double (*tab)[9] = dir == 0 ? c.powM : c.powG[mode];   // M = AKHA (forward) or G[mode] (backward)
+    const int W = K > 0 ? 4 * D : (dir == 0 ? D + 1 : D);
+    double x[D], dx[KD][D];
     if (dir == 0) {
-        const int W = D + 1;
 #pragma unroll
-        for (int q = 0; q < D; ++q) v[q] = x0 ? x0[id * D + q] : 0.0;
-        for (int g = 0; g < rank; ++g) {
-            power(lens.n[g]);
-            const double* e = gathered + ((size_t)g * N * L + id) * W;
-            double vn[D];
+        for (int q = 0; q < D; ++q) {
+            x[q] = x0 ? x0[id * D + q] : 0.0;
 #pragma unroll
-            for (int i = 0; i < D; ++i) {
-                double a = 0.0;
-#pragma unroll
-                for (int q = 0; q < D; ++q) a += P[i * D + q] * v[q];
-                vn[i] = a + e[i];
-            }
-#pragma unroll
-            for (int i = 0; i < D; ++i) v[i] = vn[i];
+            for (int k = 0; k < K; ++k) dx[k][q] = dx0 ? dx0[(id * K + k) * D + q] : 0.0;
         }
-#pragma unroll
-        for (int q = 0; q < D; ++q) out[id * D + q] = v[q];
-        if (u_after && rank + 1 < G) u_after[id] = gathered[((size_t)(rank + 1) * N * L + id) * W + D];
     } else {
-        if (rank >= G - 1) return;
-        const double* e = gathered + ((size_t)(G - 1) * N * L + id) * D;
+        const double* e = gathered + ((size_t)(G - 1) * N * L + id) * W;   // the last block has b_end = 0
 #pragma unroll
-        for (int q = 0; q < D; ++q) v[q] = e[q];
-        for (int g = G - 2; g > rank; --g) {
-            power(lens.n[g]);
-            e = gathered + ((size_t)g * N * L + id) * D;
-            double vn[D];
+        for (int q = 0; q < D; ++q) x[q] = e[q];
+    }
+    double P[D * D], E[KD][D * D];
+    long long have = -1;
+    const int steps = dir == 0 ? rank : G - 2 - rank;
+    for (int j = 0; j < steps; ++j) {
+        const int g = dir == 0 ? j : G - 2 - j;
+        const long long n = lens.n[g];
+        if (n != have) {
+            if constexpr (K > 0) block_transition<D>(c, n, P, E);
+            else mat_pow<D>(tab, n, P);
+            have = n;
+        }
+        const double* e = gathered + ((size_t)g * N * L + id) * W;
+        double xn[D], dxn[KD][D];
 #pragma unroll
-            for (int i = 0; i < D; ++i) {
-                double a = 0.0;
+        for (int i = 0; i < D; ++i) {
+            double s = 0.0;
 #pragma unroll
-                for (int q = 0; q < D; ++q) a += P[i * D + q] * v[q];
-                vn[i] = e[i] + a;
+            for (int q = 0; q < D; ++q) s += P[i * D + q] * x[q];
+            xn[i] = s + e[i];
+#pragma unroll
+            for (int k = 0; k < K; ++k) {
+                double a = 0.0, b = 0.0;
+#pragma unroll
+                for (int q = 0; q < D; ++q) { a += P[i * D + q] * dx[k][q]; b += E[k][i * D + q] * x[q]; }
+                dxn[k][i] = a + b + e[(1 + k) * D + i];
             }
-#pragma unroll
-            for (int i = 0; i < D; ++i) v[i] = vn[i];
         }
 #pragma unroll
-        for (int q = 0; q < D; ++q) out[id * D + q] = v[q];
+        for (int i = 0; i < D; ++i) {
+            x[i] = xn[i];
+#pragma unroll
+            for (int k = 0; k < K; ++k) dx[k][i] = dxn[k][i];
+        }
     }
+#pragma unroll
+    for (int q = 0; q < D; ++q) {
+        out[id * D + q] = x[q];
+#pragma unroll
+        for (int k = 0; k < K; ++k) dxout[(id * K + k) * D + q] = dx[k][q];
+    }
+    if (dir == 0 && u_after && rank + 1 < G) u_after[id] = gathered[((size_t)(rank + 1) * N * L + id) * W + D];
 }
 
-cudaError_t launch_fsn_carry(int dim, int direction, int mode, const LatentConsts* consts, int L, long long N, int rank, int G,
-                             const long long* block_lengths, const double* gathered, const double* x0, double* out, double* u_after,
-                             cudaStream_t st) {
-    if (G < 1 || G > 64 || rank < 0 || rank >= G) return cudaErrorInvalidValue;
-    FsnBlockLens lens;
-    for (int g = 0; g < 64; ++g) lens.n[g] = g < G ? block_lengths[g] : 0;
+cudaError_t launch_block_carry(int dim, int direction, int mode, const LatentConsts* consts, int L, long long N, int rank, int G,
+                               const long long* block_lengths, const double* gathered, const double* x0, const double* dx0, double* out,
+                               double* dxout, double* u_after, cudaStream_t st) {
+    BlockLens lens{};
+    for (int g = 0; g < G && block_lengths; ++g) lens.n[g] = block_lengths[g];
     const unsigned grid = (unsigned)((N * L + 127) / 128);
-    if (dim == 3) k_fsn_carry<3><<<grid, 128, 0, st>>>(consts, L, N, rank, G, direction, mode, lens, gathered, x0, out, u_after);
-    else k_fsn_carry<2><<<grid, 128, 0, st>>>(consts, L, N, rank, G, direction, mode, lens, gathered, x0, out, u_after);
+    auto run = [&](auto kernel) { kernel<<<grid, 128, 0, st>>>(consts, L, N, rank, G, direction, mode, lens, gathered, x0, dx0, out, dxout, u_after); };
+    if (dim == 3) dxout ? run(k_block_carry<3, 3>) : run(k_block_carry<3, 0>);
+    else dxout ? run(k_block_carry<2, 3>) : run(k_block_carry<2, 0>);
     return cudaGetLastError();
 }
 

@@ -100,12 +100,23 @@ __host__ __device__ __forceinline__ void block_transition(const LatentConsts& c,
             HD_UNROLL
             for (int i = 0; i < D * D; ++i) P[i] = t1[i];
         }
+        // E(2b) = E(b) M^b + M^b E(b), the sum formed entry by entry (the sums of mat_mul, in its order): one temporary
+        // instead of two, so that the device carry (k_block_carry) fits in registers at D = 3
         HD_UNROLL
-        for (int k = 0; k < 3; ++k) {                               // E(2b) = E(b) M^b + M^b E(b)
-            mat_mul<D>(Eb[k], Pb, t1);
-            mat_mul<D>(Pb, Eb[k], t2);
+        for (int k = 0; k < 3; ++k) {
             HD_UNROLL
-            for (int i = 0; i < D * D; ++i) Eb[k][i] = t1[i] + t2[i];
+            for (int i = 0; i < D; ++i)
+                HD_UNROLL
+                for (int j = 0; j < D; ++j) {
+                    double s1 = 0.0, s2 = 0.0;
+                    HD_UNROLL
+                    for (int q = 0; q < D; ++q) s1 += Eb[k][i * D + q] * Pb[q * D + j];
+                    HD_UNROLL
+                    for (int q = 0; q < D; ++q) s2 += Pb[i * D + q] * Eb[k][q * D + j];
+                    t1[i * D + j] = s1 + s2;
+                }
+            HD_UNROLL
+            for (int i = 0; i < D * D; ++i) Eb[k][i] = t1[i];
         }
     }
 }

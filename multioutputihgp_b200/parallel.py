@@ -27,6 +27,23 @@ def _dist():
     return dist
 
 
+def _ranks(group):
+    """(multi, world, rank) of this process in ``group``: (False, 1, 0) without a process group of more than one rank."""
+    dist = _dist()
+    if not (dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1):
+        return False, 1, 0
+    return True, dist.get_world_size(group), dist.get_rank(group)
+
+
+def _all_gather_into(out, inp, group):
+    """out[G, ...] <- every rank's inp, on the current stream (NCCL); gloo (ranks sharing a GPU, CPU tests) takes the list form"""
+    dist = _dist()
+    if dist.get_backend(group) == "gloo":
+        dist.all_gather(list(out.unbind(0)), inp, group=group)
+    else:
+        dist.all_gather_into_tensor(out, inp, group=group)
+
+
 class ShardedObjective(object):
     """loss, grad = sum over ALL ranks' sequences of the objective; call with this rank's shard.
 
@@ -47,7 +64,7 @@ class ShardedObjective(object):
             buf[0] = loss
             buf[1:] = grad
         dist = _dist()
-        if dist.is_available() and dist.is_initialized() and dist.get_world_size(self.group) > 1:
+        if _ranks(self.group)[0]:
             t = torch.from_numpy(buf)
             if self.device is not None:
                 t = t.to(self.device)
@@ -71,7 +88,7 @@ class ShardedDeviceObjective(object):
         self.buf.zero_()
         if Y_local_device is not None and Y_local_device.shape[0] > 0:
             self.model.objective_device(Y_local_device, self.buf[0:1], self.buf[2:])
-        if dist.is_available() and dist.is_initialized() and dist.get_world_size(self.group) > 1:
+        if _ranks(self.group)[0]:
             dist.all_reduce(self.buf, op=dist.ReduceOp.SUM, group=self.group)
         host = self.buf.cpu().numpy()
         return float(host[0]), host[2:].copy()
@@ -84,7 +101,7 @@ def sharded_nll(local_nll, group=None, device=None):
     if device is not None:
         t = t.to(device)
     dist = _dist()
-    if dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:
+    if _ranks(group)[0]:
         dist.all_reduce(t, op=dist.ReduceOp.SUM, group=group)
     return float(t.item())
 
@@ -192,9 +209,7 @@ class TimeShardedObjective(object):
     def __call__(self, Y_block, x0=None, dx0=None):
         import torch
         dist = _dist()
-        multi = dist.is_available() and dist.is_initialized() and dist.get_world_size(self.group) > 1
-        world = dist.get_world_size(self.group) if multi else 1
-        rank = dist.get_rank(self.group) if multi else 0
+        multi, world, rank = _ranks(self.group)
         consts, L, d = self._current()
         x0 = np.zeros((L, d)) if x0 is None else np.asarray(x0, dtype=np.float64).reshape(L, d)
         dx0 = np.zeros((L, 3, d)) if dx0 is None else np.asarray(dx0, dtype=np.float64).reshape(L, 3, d)
@@ -260,16 +275,11 @@ class TimeShardedDeviceObjective(object):
         x0 / dx0: carried-in state of the WHOLE sequence (torch CUDA tensors or None = zeros)."""
         dist = _dist()
         m = self.model
-        multi = dist.is_available() and dist.is_initialized() and dist.get_world_size(self.group) > 1
-        world = dist.get_world_size(self.group) if multi else 1
-        rank = dist.get_rank(self.group) if multi else 0
+        multi, world, rank = _ranks(self.group)
         last = rank == world - 1
         m.objective_begin_async(Y_block_dev, None if last else self.zend)
         if multi:
-            if dist.get_backend(self.group) == "gloo":       # gloo (ranks sharing a GPU, CPU tests) takes the list form
-                dist.all_gather(list(self.ends.unbind(0)), self.zend, group=self.group)
-            else:
-                dist.all_gather_into_tensor(self.ends, self.zend, group=self.group)
+            _all_gather_into(self.ends, self.zend, self.group)
         m.carry_in_device(self.ends, self.block_lengths, rank, self.xin, self.dxin, x0=x0, dx0=dx0)
         m.objective_finish_device(Y_block_dev, self.buf[0:1], self.buf[2:], x0=self.xin, dx0=self.dxin)
         if multi:
@@ -310,30 +320,15 @@ def backward_carry_in(smoother_power, block_lengths, starts_b, rank):
 class TimeShardedFilterSmoother(object):
     """Fused filter + smoother + NLL of ONE long sequence (or N of them) whose contiguous time blocks live on different
     ranks: forward carry exchange, then the mirror-image backward exchange, two all-gathers of O(L d) doubles and one
-    all-reduce of the NLL.  ``model`` provides ``fsn_block(phase, ...)``, ``block_transition(n)``, ``smoother_power(n, mode)``
-    (``MOIHGPSequences``); every block but the last holds a multiple of 256 steps (``time_block_bounds_aligned``)."""
+    all-reduce of the NLL, all queued on the device.  ``model`` provides ``fsn_block_async(phase, ...)`` and
+    ``fsn_carry_device(direction, ...)`` (``MOIHGPSequences``); every block but the last holds a multiple of 256 steps
+    (``time_block_bounds_aligned``)."""
 
     def __init__(self, model, block_lengths, smoother_mode=1, group=None, device=None):
         import torch
         self.model, self.group, self.mode = model, group, int(smoother_mode)
         self.block_lengths = [int(b) for b in block_lengths]
         self.dev = device if device is not None else torch.device("cuda", torch.cuda.current_device())
-
-    def _gather(self, arr, world):
-        import torch
-        dist = _dist()
-        t = torch.from_numpy(np.ascontiguousarray(arr)).to(self.dev)
-        out = [torch.empty_like(t) for _ in range(world)]
-        dist.all_gather(out, t, group=self.group)
-        return [o.cpu().numpy() for o in out]
-
-    def _all_gather(self, out, inp):
-        """out[G, ...] <- every rank's inp, on the current stream (NCCL); gloo (CPU tests) takes the list form"""
-        dist = _dist()
-        if dist.get_backend(self.group) == "gloo":
-            dist.all_gather(list(out.unbind(0)), inp, group=self.group)
-        else:
-            dist.all_gather_into_tensor(out, inp, group=self.group)
 
     def _buffers(self, N):
         import torch
@@ -355,9 +350,7 @@ class TimeShardedFilterSmoother(object):
         dist = _dist()
         m = self.model
         N = Y_block.shape[0]
-        multi = dist.is_available() and dist.is_initialized() and dist.get_world_size(self.group) > 1
-        world = dist.get_world_size(self.group) if multi else 1
-        rank = dist.get_rank(self.group) if multi else 0
+        multi, world, rank = _ranks(self.group)
         last = rank == world - 1
         b = self._buffers(N)
         nll_dev = nll if nll is not None else b._nll
@@ -367,11 +360,11 @@ class TimeShardedFilterSmoother(object):
             m.fsn_block_async(3, Y_block, True, self.mode, x0=x0, X=X, Xs=Xs, nll=nll_dev, xT=xT)
             return nll_dev
         m.fsn_block_async(1, Y_block, last, self.mode, out=b._p1)
-        self._all_gather(b._g1, b._p1)
+        _all_gather_into(b._g1, b._p1, self.group)
         m.fsn_carry_device(0, b._g1, self.block_lengths, rank, b._xin, self.mode, x0=x0, u_after=b._uaf)
         u_after = None if last else b._uaf
         m.fsn_block_async(2, Y_block, last, self.mode, x0=b._xin, u_after=u_after, out=b._p2)
-        self._all_gather(b._g2, b._p2)
+        _all_gather_into(b._g2, b._p2, self.group)
         m.fsn_carry_device(1, b._g2, self.block_lengths, rank, b._bend, self.mode)
         m.fsn_block_async(3, Y_block, last, self.mode, x0=b._xin, u_after=u_after, b_end=None if last else b._bend, X=X, Xs=Xs,
                           nll=nll_dev, xT=xT)
@@ -379,39 +372,14 @@ class TimeShardedFilterSmoother(object):
         return nll_dev
 
     def __call__(self, Y_block, X, Xs, x0=None, nll=None, xT=None):
-        """Y_block [N,n,p], X / Xs [N,n,L,d] (this rank's block, tensors on the device); returns nll [N] of the whole
-        sequence (numpy).  x0 [N,L,d] is the state before the first step of the WHOLE sequence."""
+        """``enqueue`` and a synchronise.  Y_block [N,n,p], X / Xs [N,n,L,d] (this rank's block, tensors on the device); x0
+        [N,L,d] (NumPy or None) is the state before the first step of the WHOLE sequence; returns its nll [N] (NumPy)."""
         import torch
-        dist = _dist()
-        m = self.model
-        N = Y_block.shape[0]
-        L, d = m.num_latent, m.igp_dim
-        multi = dist.is_available() and dist.is_initialized() and dist.get_world_size(self.group) > 1
-        world = dist.get_world_size(self.group) if multi else 1
-        rank = dist.get_rank(self.group) if multi else 0
-        last = rank == world - 1
-        x0 = np.zeros((N, L, d)) if x0 is None else np.asarray(x0, dtype=np.float64).reshape(N, L, d)
-        to_dev = lambda a: torch.from_numpy(np.ascontiguousarray(a)).to(self.dev)
-        x_end, u_first = m.fsn_block(1, Y_block, last, self.mode)
-        x_in, u_after = x0, None
-        if multi:
-            got = self._gather(np.concatenate([x_end.ravel(), u_first.ravel()]), world)
-            ends = [g_[:N * L * d].reshape(N, L, d) for g_ in got]
-            x_in = forward_carry_in(m.block_transition, self.block_lengths, ends, x0, rank)
-            if not last:
-                u_after = to_dev(got[rank + 1][N * L * d:].reshape(N, L))
-        x_in_dev = to_dev(x_in)
-        b0 = m.fsn_block(2, Y_block, last, self.mode, x0=x_in_dev, u_after=u_after)
-        b_end = None
-        if multi:
-            starts = [g_.reshape(N, L, d) for g_ in self._gather(b0.ravel(), world)]
-            be = backward_carry_in(lambda n_: m.smoother_power(n_, self.mode), self.block_lengths, starts, rank)
-            b_end = None if be is None else to_dev(be)
-        nll_dev = nll if nll is not None else torch.zeros(N, dtype=torch.float64, device=self.dev)
-        m.fsn_block(3, Y_block, last, self.mode, x0=x_in_dev, u_after=u_after, b_end=b_end, X=X, Xs=Xs, nll=nll_dev, xT=xT)
-        if multi:
-            dist.all_reduce(nll_dev, op=dist.ReduceOp.SUM, group=self.group)
-        return nll_dev.cpu().numpy()
+        N, L, d = Y_block.shape[0], self.model.num_latent, self.model.igp_dim
+        if x0 is not None:
+            x0 = torch.from_numpy(np.ascontiguousarray(np.asarray(x0, dtype=np.float64).reshape(N, L, d))).to(self.dev)
+        # a copy: on a CPU device .cpu() would hand out the buffer the next call overwrites
+        return self.enqueue(Y_block, X, Xs, x0=x0, nll=nll, xT=xT).cpu().numpy().copy()
 
 
 class TimeShardedPosteriorSampler(object):
@@ -445,12 +413,9 @@ class TimeShardedPosteriorSampler(object):
         ``Xs_mean`` [N,n,L,d] (a workspace when None) -> sampler phase 1 -> all-gather -> backward carry kernel -> sampler
         phase 2 into Xsamp [S,N,n,L,d], Fsamp [S,N,n,L], Ysamp [S,N,n,p] (this rank's block; at least one).  x0 [N,L,d]: the
         state before the first step of the WHOLE sequence or None.  Returns the tensor holding the RTS mean."""
-        dist = _dist()
         m = self.model
         N, n, S = int(Y_block.shape[0]), int(Y_block.shape[1]), int(num_samples)
-        multi = dist.is_available() and dist.is_initialized() and dist.get_world_size(self.group) > 1
-        world = dist.get_world_size(self.group) if multi else 1
-        rank = dist.get_rank(self.group) if multi else 0
+        multi, world, rank = _ranks(self.group)
         last = rank == world - 1
         b = self._buffers(N, n, S)
         Xs = Xs_mean if Xs_mean is not None else b._Xs
@@ -461,7 +426,7 @@ class TimeShardedPosteriorSampler(object):
             return Xs
         t0 = sum(self.block_lengths[:rank])
         m.sample_block_async(1, Xs, S, seed, t0, last, out=b._e1)
-        self.mean._all_gather(b._eg, b._e1)
+        _all_gather_into(b._eg, b._e1, self.group)
         m.fsn_carry_device(1, b._eg, self.block_lengths, rank, b._eend, smoother_mode=1)
         m.sample_block_async(2, Xs, S, seed, t0, last, e_end=None if last else b._eend, **outs)
         return Xs

@@ -20,7 +20,7 @@ import torch.distributed as dist
 
 from bench import model_params, DT
 from multioutputihgp_b200 import MOIHGPSequences
-from multioutputihgp_b200.parallel import TimeShardedPosteriorSampler, time_block_bounds_aligned
+from multioutputihgp_b200.parallel import TimeShardedPosteriorSampler, _all_gather_into, time_block_bounds_aligned
 from test_gpu_sampling import normals
 
 rank, world, local = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1)), int(os.environ.get("LOCAL_RANK", 0))
@@ -78,7 +78,7 @@ def steps_timed(sampler, outs):
     Xs = b._Xs
     steps = [("mean", lambda: sampler.mean.enqueue(Yb, b._X, Xs)),
              ("phase1", lambda: m.sample_block_async(1, Xs, S, seed, t0, last, out=b._e1)),
-             ("all_gather", lambda: sampler.mean._all_gather(b._eg, b._e1)),
+             ("all_gather", lambda: _all_gather_into(b._eg, b._e1, sampler.group)),
              ("carry", lambda: m.fsn_carry_device(1, b._eg, lengths, rank, b._eend, smoother_mode=1)),
              ("phase2", lambda: m.sample_block_async(2, Xs, S, seed, t0, last, e_end=None if last else b._eend, **outs))]
     rec = {k: [] for k, _ in steps}

@@ -44,11 +44,11 @@ fs(Yb, X, Xs)                                         # warm-up
 torch.cuda.synchronize(dev)
 dist.barrier()
 tic = time.perf_counter()
-nll_host = fs(Yb, X, Xs)                              # exchanges through the host thread (the round-1 protocol)
+nll_call = fs(Yb, X, Xs)                              # __call__ = enqueue + synchronise
 torch.cuda.synchronize(dev)
 dist.barrier()
-t_host = time.perf_counter() - tic
-Xh, Xsh = X.clone(), Xs.clone()
+t_call = time.perf_counter() - tic
+Xc, Xsc = X.clone(), Xs.clone()
 X.zero_(); Xs.zero_()
 for _ in range(2):                                    # device-side exchange: nothing leaves the stream (warm-up, then timed)
     torch.cuda.synchronize(dev)
@@ -59,7 +59,7 @@ for _ in range(2):                                    # device-side exchange: no
     dist.barrier()
     t_shard = time.perf_counter() - tic
 nll = nll.cpu().numpy()
-assert torch.equal(X, Xh) and float((Xs - Xsh).abs().max()) <= 1e-12 * float(Xsh.abs().max()) and abs(nll[0] - nll_host[0]) <= 1e-12 * abs(nll_host[0])
+assert torch.equal(X, Xc) and torch.equal(Xs, Xsc) and np.array_equal(nll, nll_call)
 # every rank checks its own block against the whole-sequence pass computed on rank 0
 if rank == 0:
     Yd = torch.from_numpy(Y).to(dev)[None].contiguous()
@@ -78,8 +78,8 @@ if rank == 0:
     e_s = float((Xs - Xsw[:, t0_b:t1_b]).abs().max()) / scale_s
     e_n = abs(float(nll[0]) - float(nllw[0])) / abs(float(nllw[0]))
     # the other ranks' blocks: gather their first / last rows through the host is overkill - compare the block borders
-    print("time-sharded filter+smoother+NLL: world=%d p=%d L=%d T=%d  rank-0 block rel.err X %.2e Xs %.2e, nll %.2e | wall: sharded %.2f ms (exchange through the host %.2f ms), one GPU %.2f ms"
-          % (world, p, L, T, e_x, e_s, e_n, 1e3 * t_shard, 1e3 * t_host, 1e3 * t_one))
+    print("time-sharded filter+smoother+NLL: world=%d p=%d L=%d T=%d  rank-0 block rel.err X %.2e Xs %.2e, nll %.2e | wall: sharded %.2f ms (__call__ = enqueue + sync %.2f ms), one GPU %.2f ms"
+          % (world, p, L, T, e_x, e_s, e_n, 1e3 * t_shard, 1e3 * t_call, 1e3 * t_one))
     assert e_x < 1e-9 and e_s < 1e-9 and e_n < 1e-9
     ref_tail = (Xw[:, -1].cpu().numpy(), Xsw[:, -1].cpu().numpy(), Xsw[:, bounds[-1][0]].cpu().numpy())
     tail = torch.from_numpy(np.concatenate([a.ravel() for a in ref_tail])).to(dev)
